@@ -16,6 +16,10 @@ only for the timing barrier and the max-over-ranks reduction.
              algorithmic bytes 28*W*N over its CUDA-event time, against MEASURED_PEAKS.json hbm_gbs
   cpu_baseline : the CPU oracle (the only CPU implementation of this path that exists here: upstream's Rust crates
              are not vendored / buildable) on a bounded sample, scaled linearly in cycles to po2=20
+
+--dump-outputs DIR writes the seals of the last timed step of `value` (one per context in flight, the arrays
+prove_resident returns) as DIR/seal_rank<R>_ctx<I>.npy, u32 words stored exactly as float64.  Blinding is then
+derived from the seeds, so the same arguments give the same seals on every run and build.
 """
 import argparse
 import json
@@ -27,12 +31,14 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the bench writes nothing into it
 
 METRIC = "po2=20 segments/sec (synthetic rv32im-shaped segment, W=256); camt53 proof seconds measured on a 37-segment proof (camt53.proof_seconds)"
 UNIT = "segments/s"
 WIDTHS = (16, 192, 48)
 CAMT53_SEGMENTS = 37  # /root/reference/docs/runtime.md:50 (segment_count of the test camt53 proof)
 TRACE_SEED = 0x48595046
+DUMP_LIMIT = 64 * 10**6  # bytes --dump-outputs may write over all ranks
 
 
 def measured_hbm_peak():
@@ -227,7 +233,11 @@ def main():
     ap.add_argument("--ir-scale", action="store_true", help="run tools/ir_scale_probe.py live (51 k-step data-defined circuit; ~1 min) instead of quoting profiles/r2_ir_scale.json")
     ap.add_argument("--inflight", type=int, default=0, help="prover contexts (segments in flight) per GPU; 0 = auto: 8 (measured best on one B200: 20.0 / 19.7 "
                     "segments/s resident / e2e against 19.9 / 19.1 with 4), fewer when the ranks' pinned trace buffers would take more than a quarter of the host's free memory, never below 4")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the seals of the last timed step as DIR/seal_rank<R>_ctx<I>.npy (float64, at most 64 MB in all; "
+                    "blinding derived from the seeds so that runs compare seal for seal)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
     if args.warmup < 3:
@@ -292,7 +302,13 @@ def main():
         F = max(1, min(F, int(0.8 * free_dev / (7.4e9 * 2.0 ** (po2 - 20)))))
     # F prover contexts per GPU, each driven by its own host thread (ctypes releases the GIL): while one segment sits
     # in its serial Fiat-Shamir tail or copies its trace, the other keeps the SMs busy.  A step = F segments per GPU.
-    ctxs = [pkg.Context(device=local_rank, max_po2=po2, circuit=WIDTHS) for _ in range(F)]
+    deterministic = bool(args.dump_outputs) or os.environ.get("HFB200_DETERMINISTIC_BLINDING", "0") == "1"
+    ctxs = [pkg.Context(device=local_rank, max_po2=po2, circuit=WIDTHS, deterministic=deterministic) for _ in range(F)]
+    if args.dump_outputs:
+        dump_bytes = world * F * ctxs[0].seal_words(po2) * 8
+        if dump_bytes > DUMP_LIMIT:
+            raise SystemExit("bench.py: --dump-outputs would write %.1f MB (more than %d MB); use fewer --inflight contexts" % (dump_bytes / 1e6, DUMP_LIMIT // 10**6))
+        os.makedirs(args.dump_outputs, exist_ok=True)
     # per-(rank, context) segment: seed = f(global seed, rank, slot) -> every context proves a different segment
     gl = [c.witgen_synth(po2, TRACE_SEED + 1000003 * rank + 7919 * i, 1 + rank) for i, c in enumerate(ctxs)]
     ctx, g = ctxs[0], gl[0]
@@ -514,7 +530,7 @@ def main():
                            "cache": "inputs (1 GiB trace, 4 GiB LDE) are larger than L2; no flush needed", "seal_words": seal_words,
                            "camt53_segments": CAMT53_SEGMENTS,
                            "camt53_proof_seconds": (camt53 or {}).get("proof_seconds"), "camt53_proof_seconds_is": "MEASURED: wall clock of one 37-segment proof with host trace buffers (camt53 object); null when --no-camt53 / --no-e2e",
-                           "blinding": "library default: a fresh 256-bit key from OS entropy per segment, ChaCha20-expanded on the device (the seeds passed are only mixed in)" if os.environ.get("HFB200_DETERMINISTIC_BLINDING", "0") != "1" else "deterministic test mode (HFB200_DETERMINISTIC_BLINDING=1)",
+                           "blinding": "library default: a fresh 256-bit key from OS entropy per segment, ChaCha20-expanded on the device (the seeds passed are only mixed in)" if not deterministic else "deterministic test mode (HFB200_DETERMINISTIC_BLINDING=1 or --dump-outputs)",
                            "host_syncs_per_segment": stage.get("host_syncs", 0.0) / args.steps},
                 "stages_ms_per_segment": {k: v / args.steps for k, v in stage.items() if k.startswith("ms_")},
                 "stages_note": "CUDA events on the library stream, one context in flight (kernel durations undisturbed); value/e2e use %d contexts in flight" % F,
@@ -522,6 +538,9 @@ def main():
                 "gpu_launches": launches_all, "clocks": clocks}
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
+    if args.dump_outputs:
+        for slot, s in enumerate(seals):
+            np.save(os.path.join(args.dump_outputs, "seal_rank%d_ctx%d.npy" % (rank, slot)), s.astype(np.float64))
     for c in ctxs:
         c.close()
     if dist is not None:
