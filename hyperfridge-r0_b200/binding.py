@@ -256,6 +256,7 @@ class Context:
         seal = np.empty(cap, np.uint32)
         got = C.c_size_t()
         self._check(self.lib.hfb200_prove_segment(self._h, po2, _ptr(globals_), _ptr(code), _ptr(data), blind_seed, _ptr(seal), cap, C.byref(got)))
+        self._po2 = po2  # the proved trace is now the resident one (prove_resident, read_group)
         return seal[:got.value]
 
     def segment_begin(self, po2, globals_, code, data, blind_seed):
@@ -388,6 +389,7 @@ class Context:
         code = _u32(code)
         out = np.empty(8, np.uint32)
         self._check(self.lib.hfb200_control_root(self._h, po2, _ptr(code), _ptr(out)))
+        self._po2 = po2  # the context now holds columns of this size
         return out
 
     def ir_jit_active(self):

@@ -199,7 +199,7 @@ const char* hfb200_read_group(hfb200_ctx* ctx, uint32_t group, uint32_t* out, si
     API_CATCH
 }
 
-size_t hfb200_seal_words(const hfb200_ctx* ctx, uint32_t po2) { return ctx ? ctx->p.seal_words(po2) : 0; }
+size_t hfb200_seal_words(const hfb200_ctx* ctx, uint32_t po2) { return ctx && po2 >= MIN_PO2 && po2 <= MAX_PO2 ? ctx->p.seal_words(po2) : 0; }
 
 const char* hfb200_checkpoint(hfb200_ctx* ctx, const char* name, uint32_t* out, size_t cap, size_t* n_words) {
     API_TRY
@@ -351,10 +351,10 @@ const char* hfb200_pool_prove(hfb200_pool* pool, hfb200_segment_job* jobs, size_
     // argument checks up front: a mis-shaped job must not reach cudaMemcpyAsync
     for (size_t i = 0; i < n_jobs; i++) {
         hfb200_segment_job& j = jobs[i];
+        if (!j.globals || !j.data || !j.seal_out) { j.error = dup_err("job has a NULL globals / data / seal_out pointer"); continue; }
+        if (j.po2 < MIN_PO2 || j.po2 > pool->max_po2) { j.error = dup_err("job po2 " + std::to_string(j.po2) + " outside [12, " + std::to_string(pool->max_po2) + "]"); continue; }
         const size_t need = hfb200_seal_words(pool->slots.empty() ? nullptr : pool->slots[0].ctx, j.po2);
-        if (!j.globals || !j.data || !j.seal_out) j.error = dup_err("job has a NULL globals / data / seal_out pointer");
-        else if (j.po2 < 12 || j.po2 > pool->max_po2) j.error = dup_err("job po2 " + std::to_string(j.po2) + " outside [12, " + std::to_string(pool->max_po2) + "]");
-        else if (need && j.seal_cap < need) { j.seal_words = need; j.error = dup_err("seal buffer too small: need " + std::to_string(need) + " words"); }
+        if (need && j.seal_cap < need) { j.seal_words = need; j.error = dup_err("seal buffer too small: need " + std::to_string(need) + " words"); }
     }
     std::mutex mu;
     std::condition_variable cv;

@@ -29,6 +29,7 @@ struct StageRange {
 };
 
 static constexpr uint32_t QUERIES = 50, INV_RATE = 4, FRI_FOLD = 16, FRI_MIN_DEGREE = 256, CHECK_SIZE = 16;
+static constexpr uint32_t MIN_PO2 = 12, MAX_PO2 = 22;  // segment sizes a context can be created for (max_po2) and can prove
 
 struct MerkleShape {
     uint32_t rows, layers, top_layer, top_size;
@@ -141,7 +142,7 @@ struct Prover {
 
     void init(int device, uint32_t max_po2_, uint32_t wc, uint32_t wd, uint32_t wa, const IrTap* taps = nullptr, size_t n_taps = 0,
               const IrStep* steps = nullptr, size_t n_steps = 0, uint32_t ret = 0, uint32_t n_mix_ir = 0, const uint8_t* info16 = nullptr) {
-        if (max_po2_ < 12 || max_po2_ > 22) throw Err("max_po2 must be in [12, 22]");
+        if (max_po2_ < MIN_PO2 || max_po2_ > MAX_PO2) throw Err("max_po2 must be in [12, 22]");
         max_po2 = max_po2_;
         set_circuit_info(circuit_info, taps != nullptr, info16);
 #ifndef HFB200_EMU
@@ -180,10 +181,16 @@ struct Prover {
         if (const char* env = std::getenv("HFB200_HBM_PEAK_GBS")) metrics_peak_gbs = std::atof(env);
         stage_cap = (size_t)4 << 20;
         if (gen.active) stage_cap += (size_t)gen.n_mixpow * sizeof(E4);
+        // the device transcript's landing area, sized once for the largest segment (seal_words grows with po2): a CUDA graph of
+        // transcript mode 2 records its device->host copies into this buffer, so it must stay put until destroy()
+        out_cap = (seal_words(max_po2) + CP_WORDS) * 4;
 #ifndef HFB200_EMU
         CUDA_CHECK(cudaHostAlloc((void**)&stage_h, stage_cap, cudaHostAllocDefault));
+        CUDA_CHECK(cudaHostAlloc((void**)&out_h, out_cap, cudaHostAllocDefault));
 #else
         stage_h = (uint8_t*)std::malloc(stage_cap);
+        out_h = (uint8_t*)std::malloc(out_cap);
+        if (!stage_h || !out_h) throw Err("emu: out of memory");
 #endif
     }
     // asynchronous upload of a small host array: staged in pinned memory when it fits (no sync needed), else copy + sync
@@ -846,21 +853,8 @@ struct Prover {
     bool device_transcript() const { return transcript_setting() >= 1 && !gen.active; }
     bool graph_replay() const { return transcript_setting() >= 2 && !gen.active && !debug_checkpoints; }
     uint64_t graph_launches = 0;  // segments issued as one cudaGraphLaunch
-    uint8_t* out_h = nullptr;     // pinned landing area of the seal and the checkpoint words (device-transcript path)
+    uint8_t* out_h = nullptr;     // pinned landing area of the seal and the checkpoint words (device-transcript path), allocated in init
     size_t out_cap = 0;
-    void ensure_out(size_t bytes) {
-        if (bytes <= out_cap) return;
-#ifndef HFB200_EMU
-        if (out_h) cudaFreeHost(out_h);
-        out_h = nullptr; out_cap = 0;
-        CUDA_CHECK(cudaHostAlloc((void**)&out_h, bytes, cudaHostAllocDefault));
-#else
-        std::free(out_h);
-        out_h = (uint8_t*)std::malloc(bytes);
-        if (!out_h) throw Err("emu: out of memory");
-#endif
-        out_cap = bytes;
-    }
 #ifndef HFB200_EMU
     struct GraphEntry { int state = 0; cudaGraphExec_t exec = nullptr; };  // 0: never run, 1: warmed up, 2: instantiated
     std::map<uint64_t, GraphEntry> graphs;                                // key = po2 * 2 + use_control
@@ -878,7 +872,7 @@ struct Prover {
         const size_t words = seal_words(po2);
         if (n_mix > 4096) throw Err("internal: accum mix larger than the checkpoint buffer");
         const size_t cp_words = CP_ACCUM_MIX + n_mix;
-        ensure_out((words + cp_words) * 4);
+        if ((words + cp_words) * 4 > out_cap) throw Err("internal: seal larger than the landing buffer sized for max_po2");
         uint32_t* seal_pin = reinterpret_cast<uint32_t*>(out_h);
         uint32_t* cp_pin = seal_pin + words;
         HostRng r0;

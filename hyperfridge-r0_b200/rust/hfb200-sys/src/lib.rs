@@ -101,6 +101,7 @@ extern "C" {
     pub fn hfb200_ir_jit_active(ctx: *const hfb200_ctx, compile_ms: *mut f32) -> c_int;
     pub fn hfb200_destroy(ctx: *mut hfb200_ctx);
     pub fn hfb200_free_error(msg: *const c_char);
+    /// Seal length in words for `po2`; 0 for po2 outside [12, 22].
     pub fn hfb200_seal_words(ctx: *const hfb200_ctx, po2: u32) -> usize;
     pub fn hfb200_prove_segment(
         ctx: *mut hfb200_ctx, po2: u32, globals: *const u32, code: *const u32, data: *const u32, blind_seed: u64,

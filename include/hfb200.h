@@ -135,7 +135,8 @@ const char* hfb200_prove_resident(hfb200_ctx* ctx, uint64_t blind_seed, uint32_t
 /* Copies resident columns back (group: 0 accum, 1 code, 2 data), for parity tests of witgen/step_accum. */
 const char* hfb200_read_group(hfb200_ctx* ctx, uint32_t group, uint32_t* out, size_t cap_words);
 
-/* Seal length in words for (circuit, po2) -- what upstream's Vec<u32> seal would hold. */
+/* Seal length in words for (circuit, po2) -- what upstream's Vec<u32> seal would hold.  Defined for 12 <= po2 <= 22, the sizes
+ * hfb200_init accepts as max_po2, whatever this context's own max_po2; returns 0 for any other po2 and for ctx == NULL. */
 size_t hfb200_seal_words(const hfb200_ctx* ctx, uint32_t po2);
 
 /* ---- transcript checkpoints of the last proved segment (parity tests) ------------------------ */
