@@ -319,8 +319,9 @@ struct GenericCircuitHost {
     std::vector<BcIns> prog;   // the whole constraint polynomial as ONE program (verifier, reference for the chunks)
     uint32_t n_fp_slots = 0, n_mix_slots = 0, ret_slot = 0, n_mixpow = 0;
     // The same polynomial cut along its top-level AndEqz / AndCond chain into CHUNKS of ~400 steps: the sum
-    // tot = sum_k mix^e_k * term_k splits anywhere, so every chunk is a self-contained program (its Gets re-issued, its chain head
-    // starting at the exponent the prefix reached) that adds its partial sum into the check buffer.  At rv32im scale (tens of
+    // tot = sum_k mix^e_k * term_k splits between any two elements whose chunk does not read one of them as a value (make_chunks),
+    // so every chunk is a self-contained program (its Gets re-issued, its chain head starting at the exponent the prefix reached)
+    // that adds its partial sum into the check buffer.  At rv32im scale (tens of
     // thousands of steps, a thousand taps) one straight-line kernel does not compile in useful time and keeps ~1000 values
     // live; chunks compile in parallel in seconds and keep the live set small (upstream splits its generated eval_check the same way).
     struct Chunk { std::vector<BcIns> prog; uint32_t n_fp_slots = 0, n_mix_slots = 0, ret_slot = 0; BcIns* d_prog = nullptr; };
@@ -505,10 +506,19 @@ struct GenericCircuitHost {
             chunks.push_back(std::move(c));
             return;
         }
+        // Inside a chunk an element of the top-level chain carries a PARTIAL sum (it starts from the chunk's synthetic head), so
+        // a step that reads it other than as its chain predecessor (an AndCond inner, the start of another chain) must not sit
+        // in the same chunk: it would see the partial sum where the program means the full one.  Such a consumer starts a new
+        // chunk instead, where `mark` recomputes the element it reads from the real head.  The first chunk starts at the real
+        // head (exponent 0), so its partial sums are the full ones.
+        std::vector<uint32_t> chain_pos(n, 0xFFFFFFFFu);
+        for (size_t q = 0; q < chain.size(); q++) chain_pos[mix_of[chain[q]]] = (uint32_t)q;
         std::vector<uint32_t> stamp(n, 0);
         std::vector<uint32_t> stack;
-        // marks the steps element `var` needs (its own step, its fp operands, its inner chain) -- not its chain predecessor
-        auto mark = [&](uint32_t var, uint32_t id) {
+        // marks the steps element `var` needs (its own step, its fp operands, its inner chain) -- not its chain predecessor.
+        // `reads_from`: set when those steps read a chain element at position >= `lo` other than as a chain predecessor.
+        bool reads_from = false;
+        auto mark = [&](uint32_t var, uint32_t id, size_t lo) {
             size_t added = 0;
             stack.clear();
             const uint32_t self = mix_of[var];
@@ -518,6 +528,7 @@ struct GenericCircuitHost {
             if (e.op == IR_AND_COND) stack.push_back(mix_of[e.c]);
             while (!stack.empty()) {
                 const uint32_t i = stack.back(); stack.pop_back();
+                if (chain_pos[i] != 0xFFFFFFFFu && chain_pos[i] >= lo) reads_from = true;
                 if (stamp[i] == id) continue;
                 stamp[i] = id; added++;
                 const IrStep& s = st[i];
@@ -535,16 +546,18 @@ struct GenericCircuitHost {
         while (k < chain.size()) {
             id++;
             const size_t k0 = k;
+            const size_t lo = k0 > 1 ? k0 : chain.size();  // chain elements a consumer in this chunk may not read
             size_t count = 0;
             while (k < chain.size()) {
                 // tentative: does element k still fit?  (marking is idempotent within the id, so an overshoot only costs the re-mark below)
-                const size_t add = mark(chain[k], id);
-                if (k > k0 && count + add > limit) { break; }
+                reads_from = false;
+                const size_t add = mark(chain[k], id, lo);
+                if (k > k0 && (reads_from || count + add > limit)) { break; }
                 count += add; k++;
             }
             if (k < chain.size()) {  // the element that did not fit was marked with this id: redo the group cleanly
                 id++;
-                for (size_t q = k0; q < k; q++) mark(chain[q], id);
+                for (size_t q = k0; q < k; q++) mark(chain[q], id, chain.size());
             }
             // sub-list: synthetic head TRUE, then the marked steps in their original order, operands renumbered
             std::vector<IrStep> sub;
