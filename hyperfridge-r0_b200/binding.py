@@ -25,6 +25,8 @@ EXPORTS = [
     "hfb200_pool_create", "hfb200_pool_create_ir", "hfb200_pool_load_control", "hfb200_pool_prove", "hfb200_pool_destroy",
     "hfb200_set_blinding", "hfb200_pool_set_blinding", "hfb200_pool_stats", "hfb200_pool_inject_fault",
     "hfb200_set_transcript", "hfb200_graph_launches", "hfb200_digest_bytes", "hfb200_digest_pair", "hfb200_claim_encode", "hfb200_claim_decode", "hfb200_claim_next_state", "hfb200_verify_claims",
+    "hfb200_segment_begin_dev", "hfb200_segment_finish_dev", "hfb200_segment_accum_scan", "hfb200_segment_accum_blind", "hfb200_device_count",
+    "hfb200_pool_set_accum",
 ]
 
 BLIND_OS_ENTROPY, BLIND_DETERMINISTIC = 0, 1
@@ -88,6 +90,36 @@ class Claim(C.Structure):
 
 
 EXIT_HALTED, EXIT_SYSTEM_SPLIT = 0, 1
+DEV_INPUTS = 1
+SCAN_PRODUCT, SCAN_SUM = 0, 1
+
+
+class SegmentDev(C.Structure):
+    """hfb200_segment_dev: the segment in flight between segment_begin_dev and segment_finish_dev.  `code`, `data`, `globals`,
+    `mix` and `accum` are device addresses (host addresses in the emulator); `stream` is the context's cudaStream_t."""
+    _fields_ = [("po2", C.c_uint32), ("zk_rows", C.c_uint32), ("w_code", C.c_uint32), ("w_data", C.c_uint32), ("w_accum", C.c_uint32),
+                ("n_mix", C.c_uint32), ("device", C.c_int), ("stream", C.c_void_p), ("code", C.c_void_p), ("data", C.c_void_p),
+                ("globals", C.c_void_p), ("mix", C.c_void_p), ("accum", C.c_void_p), ("mix_host", C.POINTER(C.c_uint32)),
+                ("globals_host", C.POINTER(C.c_uint32)), ("blind_seed", C.c_uint64)]
+
+    @property
+    def rows(self):
+        return 1 << self.po2
+
+    def mix_array(self):
+        return np.ctypeslib.as_array(self.mix_host, shape=(self.n_mix,)).copy()
+
+    def globals_array(self):
+        return np.ctypeslib.as_array(self.globals_host, shape=(N_GLOBAL,)).copy()
+
+    def host_view(self, name):
+        """numpy view of a column group -- only where device addresses ARE host addresses (the host emulator)."""
+        w = {"code": self.w_code, "data": self.w_data, "accum": self.w_accum}[name]
+        return np.ctypeslib.as_array(C.cast(getattr(self, name), C.POINTER(C.c_uint32)), shape=(w * self.rows,)).reshape(w, self.rows)
+
+
+# int (*hfb200_accum_fn)(void* user, hfb200_ctx* ctx, const hfb200_segment_dev* seg, size_t job)
+ACCUM_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.POINTER(SegmentDev), C.c_size_t)
 
 
 class PoolStats(C.Structure):
@@ -158,6 +190,12 @@ def load_library(path=None):
         "hfb200_claim_next_state": (err, [vp, u32, u32, vp]),
         "hfb200_verify_segments": (err, [C.POINTER(CircuitDesc), C.POINTER(CircuitIR), C.POINTER(vp), C.POINTER(sz), sz, vp, vp, C.c_uint, C.POINTER(sz)]),
         "hfb200_verify_claims": (err, [C.POINTER(vp), C.POINTER(sz), sz, vp, C.c_char_p, sz]),
+        "hfb200_segment_begin_dev": (err, [vp, u32, vp, vp, vp, u64, u32, C.POINTER(SegmentDev)]),
+        "hfb200_segment_finish_dev": (err, [vp, vp, sz, C.POINTER(sz)]),
+        "hfb200_segment_accum_scan": (err, [vp, C.c_int, u32, u32, sz]),
+        "hfb200_segment_accum_blind": (err, [vp]),
+        "hfb200_device_count": (err, [C.POINTER(C.c_int)]),
+        "hfb200_pool_set_accum": (err, [vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -275,6 +313,37 @@ class Context:
         seal = np.empty(cap, np.uint32)
         got = C.c_size_t()
         self._check(self.lib.hfb200_segment_finish(self._h, _ptr(accum), _ptr(seal), cap, C.byref(got)))
+        return seal[:got.value]
+
+    def segment_begin_dev(self, po2, globals_, code, data, blind_seed, device_inputs=False):
+        """hfb200_segment_begin_dev.  Host numpy arrays by default; device_inputs=True takes device addresses (ints, e.g.
+        torch_tensor.data_ptr()) of columns on this context's device, copied device to device.  Returns the SegmentDev."""
+        globals_ = _u32(globals_)
+        if device_inputs:
+            code_p, data_p = code, data
+        else:
+            code = _u32(code) if code is not None else None
+            data = _u32(data) if data is not None else None
+            code_p, data_p = _ptr(code), _ptr(data)
+        seg = SegmentDev()
+        self._check(self.lib.hfb200_segment_begin_dev(self._h, po2, _ptr(globals_), code_p, data_p, blind_seed,
+                                                      DEV_INPUTS if device_inputs else 0, C.byref(seg)))
+        self._po2 = po2
+        return seg
+
+    def segment_accum_scan(self, kind, first_chain, n_chains, rows):
+        """In-place inclusive scan (SCAN_PRODUCT / SCAN_SUM) of the Fp4 chains in accum columns 4c..4c+3 over rows [0, rows)."""
+        self._check(self.lib.hfb200_segment_accum_scan(self._h, int(kind), first_chain, n_chains, rows))
+
+    def segment_accum_blind(self):
+        self._check(self.lib.hfb200_segment_accum_blind(self._h))
+
+    def segment_finish_dev(self):
+        """Completes the segment from the accum columns as they stand in device memory."""
+        cap = self.seal_words(self._po2)
+        seal = np.empty(cap, np.uint32)
+        got = C.c_size_t()
+        self._check(self.lib.hfb200_segment_finish_dev(self._h, _ptr(seal), cap, C.byref(got)))
         return seal[:got.value]
 
     def witgen_synth(self, po2, trace_seed, blind_seed):
@@ -413,6 +482,27 @@ class Context:
         ms = C.c_float()
         self._check(self.lib.hfb200_mark_elapsed(self._h, slot_a, other._h, slot_b, C.byref(ms)))
         return ms.value
+
+
+def device_count(lib=None):
+    """Number of CUDA devices (hfb200_device_count); 0 without a device or a driver."""
+    lib = lib or load_library()
+    n = C.c_int()
+    _raise_err(lib, lib.hfb200_device_count(C.byref(n)))
+    return n.value
+
+
+class SegmentHandle:
+    """What a Python accum callback of Pool.set_accum may call on the context it is given."""
+
+    def __init__(self, lib, ctx):
+        self.lib, self._h = lib, ctx
+
+    def accum_scan(self, kind, first_chain, n_chains, rows):
+        _raise_err(self.lib, self.lib.hfb200_segment_accum_scan(self._h, int(kind), first_chain, n_chains, rows))
+
+    def accum_blind(self):
+        _raise_err(self.lib, self.lib.hfb200_segment_accum_blind(self._h))
 
 
 def verify_segment(seal, code_root, circuit=(16, 192, 48), ir=None, lib=None):
@@ -580,6 +670,33 @@ class Pool:
             self.lib.hfb200_free_error(e)
             raise Hfb200Error(msg)
 
+    def set_accum(self, fn, user=None):
+        """The caller's step_accum for every job (hfb200_pool_set_accum); None removes it.
+        `fn` is either the address (int) of a C function `int fn(void* user, hfb200_ctx*, const hfb200_segment_dev*, size_t job)`
+        -- `user` is then passed through as a pointer (int or None) -- or a Python callable fn(ctx, seg, job) with ctx a
+        SegmentHandle (accum_scan / accum_blind) and seg the SegmentDev.  A Python callback runs on the worker threads, one at a
+        time under the GIL; an exception fails that job only and its text appears in the job's error."""
+        self._accum_errors = {}
+        if fn is None:
+            self._accum_cb = None
+            self._raise(self.lib.hfb200_pool_set_accum(self._h, None, None))
+            return
+        if isinstance(fn, int):
+            self._accum_cb = None
+            self._raise(self.lib.hfb200_pool_set_accum(self._h, fn, user))
+            return
+        lib, errors = self.lib, self._accum_errors
+
+        def trampoline(_user, ctx, seg, job):
+            try:
+                fn(SegmentHandle(lib, ctx), seg.contents, int(job))
+                return 0
+            except BaseException as e:  # noqa: B036 -- nothing may unwind into the C worker thread
+                errors[int(job)] = "%s: %s" % (type(e).__name__, e)
+                return 1
+        self._accum_cb = ACCUM_FN(trampoline)  # kept alive as long as the pool may call it
+        self._raise(self.lib.hfb200_pool_set_accum(self._h, C.cast(self._accum_cb, C.c_void_p).value, None))
+
     def close(self):
         if self._h:
             self.lib.hfb200_pool_destroy(self._h)
@@ -624,12 +741,16 @@ class Pool:
             arr[i].po2, arr[i].blind_seed = po2, seed
             arr[i].globals, arr[i].code, arr[i].data = g.ctypes.data, (code.ctypes.data if code is not None else None), data.ctypes.data
             arr[i].seal_out, arr[i].seal_cap = seals[i].ctypes.data, seal_cap
+        accum_errors = getattr(self, "_accum_errors", {})
+        accum_errors.clear()
         e = self.lib.hfb200_pool_prove(self._h, arr, n)
         errs = [None] * n
         for i in range(n):
             if arr[i].error:
                 errs[i] = C.cast(arr[i].error, C.c_char_p).value.decode(errors="replace")
                 self.lib.hfb200_free_error(arr[i].error)
+                if i in accum_errors:  # the Python accum callback's own exception
+                    errs[i] += ": " + accum_errors[i]
         self.last_attempts = [arr[i].attempts for i in range(n)]
         out = ([seals[i][:arr[i].seal_words] if errs[i] is None else seals[i][:0] for i in range(n)], [arr[i].device for i in range(n)],
                [arr[i].ms for i in range(n)])
@@ -637,6 +758,10 @@ class Pool:
             if e:
                 self.lib.hfb200_free_error(e)
             return out + (errs,)
+        if e and accum_errors:
+            self.lib.hfb200_free_error(e)  # the library's message lacks the callback's text: report the job's own
+            i = next(k for k in range(n) if errs[k] is not None)
+            raise Hfb200Error("job %d: %s" % (i, errs[i]))
         self._raise(e)
         first = [m for m in errs if m is not None]
         if first:

@@ -92,11 +92,17 @@ struct GenDerivedKernel {
 };
 
 // ---- step_accum: Fp4 running products (three-phase scan) -----------------------------------------------
-// In-place inclusive scan (Fp4 product) of buf0[0..n) in shared memory; buf1 is scratch. Result in the returned buffer.
-HD E4* block_scan_e4(const KCtx& cx, E4* buf0, E4* buf1, uint32_t n) {
+// The two scans of hfb200_segment_accum_scan: running products (grand products, Hal::prefix_products) and running sums (LogUp).
+enum : int { SCAN_PRODUCT = 0, SCAN_SUM = 1 };
+HD E4 scan_op(int kind, const E4& a, const E4& b) { return kind == SCAN_SUM ? e4_add(a, b) : e4_mul(a, b); }
+HD E4 scan_identity(int kind) { return kind == SCAN_SUM ? e4_zero() : e4_one(); }
+
+// In-place inclusive scan (Fp4 product, or sum for kind = SCAN_SUM) of buf0[0..n) in shared memory; buf1 is scratch. Result in
+// the returned buffer.
+HD E4* block_scan_e4(const KCtx& cx, E4* buf0, E4* buf1, uint32_t n, int kind = SCAN_PRODUCT) {
     E4 *src = buf0, *dst = buf1;
     for (uint32_t d = 1; d < n; d <<= 1) {
-        for (uint32_t i = cx.tid; i < n; i += cx.nt) dst[i] = i >= d ? e4_mul(src[i - d], src[i]) : src[i];
+        for (uint32_t i = cx.tid; i < n; i += cx.nt) dst[i] = i >= d ? scan_op(kind, src[i - d], src[i]) : src[i];
         cx.sync();
         E4* t = src; src = dst; dst = t;
     }
@@ -150,17 +156,84 @@ struct AccumKernel {
         }
     }
 };
-// Exclusive scan of the per-block products of one chain (grid.y = chain, one block): partial[i] <- prod_{j<i}.
+// Exclusive scan of the per-block products of one chain (grid.y = chain, one block): partial[i] <- prod_{j<i} (sum for SCAN_SUM).
 struct AccumOffsetsKernel {
     static constexpr bool kBarrier = true;
-    HD static void run(const KCtx& cx, uint32_t* sm, E4* partial, uint32_t nblk) {
+    HD static void run(const KCtx& cx, uint32_t* sm, E4* partial, uint32_t nblk, int kind = SCAN_PRODUCT) {
         E4* buf0 = reinterpret_cast<E4*>(sm);
         E4* buf1 = buf0 + nblk;
         E4* p = partial + (uint64_t)cx.by * nblk;
         for (uint32_t i = cx.tid; i < nblk; i += cx.nt) buf0[i] = p[i];
         cx.sync();
-        E4* sc = block_scan_e4(cx, buf0, buf1, nblk);
-        for (uint32_t i = cx.tid; i < nblk; i += cx.nt) p[i] = i == 0 ? e4_one() : sc[i - 1];
+        E4* sc = block_scan_e4(cx, buf0, buf1, nblk, kind);
+        for (uint32_t i = cx.tid; i < nblk; i += cx.nt) p[i] = i == 0 ? scan_identity(kind) : sc[i - 1];
+    }
+};
+
+// ---- hfb200_segment_accum_scan: the same two-pass scan over terms the CALLER wrote into the accum columns --------------------
+// Chain c = first_chain + grid.y lives in columns 4c..4c+3; rows [0, rows) are scanned in place, ACC_RPB rows per block.  The
+// block's rows are staged in shared memory with coalesced loads (one E4 of padding every ACC_PER elements, so that the
+// per-thread runs of ACC_PER consecutive rows sit in different banks), reduced per thread, scanned across the block, and (mode 1)
+// written back with coalesced stores.  mode 0: block totals to partial[chain * nblk + blk]; mode 1: apply the exclusive offsets
+// AccumOffsetsKernel left there.
+static constexpr uint32_t SCAN_TILE = ACC_RPB + ACC_RPB / ACC_PER;  // padded tile, E4 elements
+HD uint32_t scan_slot(uint32_t i) { return i + i / ACC_PER; }
+struct AccumScanKernel {
+    static constexpr bool kBarrier = true;
+    HD static void run(const KCtx& cx, uint32_t* sm, uint32_t* accum, uint64_t n, uint64_t rows, uint32_t first_chain, int kind, E4* partial, int mode) {
+        const uint32_t chain = first_chain + cx.by, blk = cx.bx, nblk = cx.gx;
+        uint32_t* col = accum + (uint64_t)4 * chain * n;
+        E4* tile = reinterpret_cast<E4*>(sm);
+        E4* buf0 = tile + SCAN_TILE;
+        E4* buf1 = buf0 + ACC_ITEMS;
+        const uint64_t row0 = (uint64_t)blk * ACC_RPB;
+        const uint32_t cnt = (uint32_t)(rows - row0 < ACC_RPB ? rows - row0 : ACC_RPB);
+        for (uint32_t i = cx.tid; i < cnt; i += cx.nt) {
+            const uint64_t r = row0 + i;
+            tile[scan_slot(i)] = e4(col[r], col[n + r], col[2 * n + r], col[3 * n + r]);
+        }
+        cx.sync();
+        for (uint32_t it = cx.tid; it < ACC_ITEMS; it += cx.nt) {
+            E4 pr = scan_identity(kind);
+            for (uint32_t j = 0; j < ACC_PER; j++) {
+                const uint32_t i = it * ACC_PER + j;
+                if (i < cnt) pr = scan_op(kind, pr, tile[scan_slot(i)]);
+            }
+            buf0[it] = pr;
+        }
+        cx.sync();
+        E4* sc = block_scan_e4(cx, buf0, buf1, ACC_ITEMS, kind);
+        if (mode == 0) {
+            if (cx.tid == 0) partial[(uint64_t)cx.by * nblk + blk] = sc[ACC_ITEMS - 1];
+            return;
+        }
+        const E4 off = partial[(uint64_t)cx.by * nblk + blk];
+        for (uint32_t it = cx.tid; it < ACC_ITEMS; it += cx.nt) {
+            E4 pr = it == 0 ? off : scan_op(kind, off, sc[it - 1]);
+            for (uint32_t j = 0; j < ACC_PER; j++) {
+                const uint32_t i = it * ACC_PER + j;
+                if (i >= cnt) break;
+                pr = scan_op(kind, pr, tile[scan_slot(i)]);
+                tile[scan_slot(i)] = pr;
+            }
+        }
+        cx.sync();
+        for (uint32_t i = cx.tid; i < cnt; i += cx.nt) {
+            const uint64_t r = row0 + i;
+            const E4 v = tile[scan_slot(i)];
+            col[r] = v.c[0]; col[n + r] = v.c[1]; col[2 * n + r] = v.c[2]; col[3 * n + r] = v.c[3];
+        }
+    }
+};
+// hfb200_segment_accum_blind: the last zk rows of every accum column, exactly the values AccumKernel mode 1 writes there.
+struct AccumBlindKernel {
+    static constexpr bool kBarrier = false;
+    HD static void run(const KCtx& cx, uint32_t*, uint32_t* accum, uint32_t w_accum, uint32_t po2, uint32_t zk, BlindKey blind) {
+        const uint64_t n = 1ull << po2;
+        const uint64_t t = (uint64_t)cx.bx * cx.nt + cx.tid;
+        if (t >= (uint64_t)w_accum * zk) return;
+        const uint32_t c = (uint32_t)(t / zk), r = (uint32_t)(n - zk + t % zk);
+        accum[(uint64_t)c * n + r] = blind_value(blind, GROUP_ACCUM, c, r);
     }
 };
 

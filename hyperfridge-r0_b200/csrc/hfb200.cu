@@ -171,6 +171,60 @@ const char* hfb200_segment_finish(hfb200_ctx* ctx, const uint32_t* accum_or_null
     API_CATCH_QUIESCE(ctx)
 }
 
+const char* hfb200_segment_begin_dev(hfb200_ctx* ctx, uint32_t po2, const uint32_t* globals, const uint32_t* code, const uint32_t* data,
+                                     uint64_t blind_seed, uint32_t flags, hfb200_segment_dev* out) {
+    API_TRY
+    if (!ctx || !globals || !out) throw Err("hfb200_segment_begin_dev: NULL argument");
+    if (flags & ~(uint32_t)HFB200_DEV_INPUTS) throw Err("hfb200_segment_begin_dev: unknown flags");
+    Prover& p = ctx->p;
+    p.begin_dev(po2, globals, code, data, blind_seed, (flags & HFB200_DEV_INPUTS) != 0);
+    hfb200_segment_dev s{};
+    s.po2 = p.po2; s.zk_rows = ZK_CYCLES;
+    s.w_code = p.cir.cd.w_code; s.w_data = p.cir.cd.w_data; s.w_accum = p.cir.cd.w_accum; s.n_mix = (uint32_t)p.mix.size();
+    s.device = p.device_id;
+    s.stream = (void*)p.dev.stream;
+    s.code = p.tr[GROUP_CODE]; s.data = p.tr[GROUP_DATA]; s.globals = p.d_globals; s.mix = p.d_mix; s.accum = p.tr[GROUP_ACCUM];
+    s.mix_host = p.mix.data(); s.globals_host = p.globals;
+    s.blind_seed = blind_seed;
+    *out = s;
+    API_CATCH_QUIESCE(ctx)
+}
+const char* hfb200_segment_finish_dev(hfb200_ctx* ctx, uint32_t* seal_out, size_t seal_cap, size_t* seal_words) {
+    API_TRY
+    if (!ctx) throw Err("hfb200_segment_finish_dev: NULL ctx");
+    ctx->p.finish(nullptr, ctx->seal, true);
+    if (const char* e = emit_seal(ctx, seal_out, seal_cap, seal_words)) return e;
+    API_CATCH_QUIESCE(ctx)
+}
+// argument errors leave the segment in flight (nothing was queued); the caller may still finish or abandon it
+const char* hfb200_segment_accum_scan(hfb200_ctx* ctx, int kind, uint32_t first_chain, uint32_t n_chains, size_t rows) {
+    API_TRY
+    if (!ctx) throw Err("hfb200_segment_accum_scan: NULL ctx");
+    ctx->p.accum_scan(kind, first_chain, n_chains, rows);
+    API_CATCH
+}
+const char* hfb200_segment_accum_blind(hfb200_ctx* ctx) {
+    API_TRY
+    if (!ctx) throw Err("hfb200_segment_accum_blind: NULL ctx");
+    ctx->p.accum_blind();
+    API_CATCH
+}
+const char* hfb200_device_count(int* out) {
+    API_TRY
+    if (!out) throw Err("hfb200_device_count: out is NULL");
+    *out = 0;
+#ifndef HFB200_EMU
+    int n = 0;
+    const cudaError_t e = cudaGetDeviceCount(&n);
+    if (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver) { cudaGetLastError(); return nullptr; }  // a count of zero
+    CUDA_CHECK(e);
+    *out = n;
+#else
+    *out = 1;
+#endif
+    API_CATCH
+}
+
 const char* hfb200_witgen_synth(hfb200_ctx* ctx, uint32_t po2, uint64_t trace_seed, uint64_t blind_seed, uint32_t* globals_out) {
     API_TRY
     if (!ctx || !globals_out) throw Err("hfb200_witgen_synth: NULL argument");
@@ -247,6 +301,9 @@ struct hfb200_pool {
     bool is_ir = false;
     std::vector<IrTap> ir_taps; std::vector<IrStep> ir_steps; uint32_t ir_ret = 0, ir_n_mix = 0; uint8_t ir_info[16] = {0};
     int blind_mode = BLIND_OS_ENTROPY;
+    // the caller's step_accum (hfb200_pool_set_accum): jobs then run begin_dev -> accum_fn -> finish_dev
+    hfb200_accum_fn accum_fn = nullptr;
+    void* accum_user = nullptr;
     // test hook (hfb200_pool_inject_fault): worker `w` reports a CUDA error instead of proving its n-th job from now
     std::mutex inject_mu;
     std::map<size_t, std::pair<uint64_t, int>> inject;  // worker -> (jobs to let pass, kind)
@@ -284,6 +341,28 @@ static void pool_fill(hfb200_pool* pool, const int* devices, int n_devices, int 
         }
 }
 static bool is_device_fault(const char* msg) { return msg && std::strncmp(msg, "CUDA error", 10) == 0; }
+// One job through the device seam: begin_dev (the job's host inputs), the caller's step_accum on this worker thread, finish_dev.
+// A nonzero return of the callback fails the job (never retried) and abandons the segment: the stream is drained so that the
+// context is usable for the next job.  If draining it reports a CUDA error, the callback met a device fault: the worker takes
+// the device-fault path (context re-created, job re-queued).
+static const char* prove_job_with_accum(hfb200_pool* pool, hfb200_ctx* ctx, hfb200_segment_job& j, size_t idx) {
+    hfb200_segment_dev seg;
+    if (const char* e = hfb200_segment_begin_dev(ctx, j.po2, j.globals, j.code, j.data, j.blind_seed, 0, &seg)) return e;
+    const int rc = pool->accum_fn(pool->accum_user, ctx, &seg, idx);
+    if (rc != 0) {
+#ifndef HFB200_EMU
+        cudaSetDevice(ctx->p.device_id);
+        const cudaError_t e = cudaStreamSynchronize(ctx->p.dev.stream);
+        ctx->p.quiesce();
+        if (e != cudaSuccess)
+            return dup_err(std::string("CUDA error ") + cudaGetErrorName(e) + " after the accum callback: " + cudaGetErrorString(e));
+#else
+        ctx->p.quiesce();
+#endif
+        return dup_err("accum callback returned " + std::to_string(rc));
+    }
+    return hfb200_segment_finish_dev(ctx, j.seal_out, j.seal_cap, &j.seal_words);
+}
 static const char* control_root_impl(hfb200_ctx* ctx, uint32_t po2, const uint32_t* code, uint32_t* root_out, uint64_t gen);
 extern "C" {
 
@@ -407,7 +486,8 @@ const char* hfb200_pool_prove(hfb200_pool* pool, hfb200_segment_job* jobs, size_
                     err = control_root_impl(sl.ctx, j.po2, it->second.code, root, it->second.gen);
                 }
             }
-            if (!err) err = hfb200_prove_segment(sl.ctx, j.po2, j.globals, j.code, j.data, j.blind_seed, j.seal_out, j.seal_cap, &j.seal_words);
+            if (!err && pool->accum_fn) err = prove_job_with_accum(pool, sl.ctx, j, idx);
+            else if (!err) err = hfb200_prove_segment(sl.ctx, j.po2, j.globals, j.code, j.data, j.blind_seed, j.seal_out, j.seal_cap, &j.seal_words);
             j.device = sl.device;
             j.ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
             bool requeue = false, retire = false;
@@ -460,6 +540,14 @@ const char* hfb200_pool_load_control(hfb200_pool* pool, uint32_t po2, const uint
     // every load gets a new generation: a worker whose resident control group came from an earlier load (even of the same
     // pointer: the caller may have rewritten the columns) re-commits it before its next code == NULL job
     if (code) pool->control[po2] = hfb200_pool::Control{code, pool->next_gen++}; else pool->control.erase(po2);
+    API_CATCH
+}
+
+const char* hfb200_pool_set_accum(hfb200_pool* pool, hfb200_accum_fn fn, void* user) {
+    API_TRY
+    if (!pool) throw Err("hfb200_pool_set_accum: NULL pool");
+    pool->accum_fn = fn;
+    pool->accum_user = fn ? user : nullptr;
     API_CATCH
 }
 

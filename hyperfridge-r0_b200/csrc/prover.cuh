@@ -363,7 +363,20 @@ struct Prover {
     // checks the arguments, resets the per-segment state and queues the host->device copies of the trace (data columns in
     // H2D_CHUNKS slices on the copy stream).  Returns whether the data copy is chunked / the cached control group is used.
     struct Staged { bool chunked, use_control; };
-    Staged stage_inputs(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind) {
+    // HFB200_DEV_INPUTS: the caller's columns must be device memory of this context's device (a host pointer would make the
+    // device-to-device copy fault or read another GPU's memory).  The emulator has no device memory to tell apart.
+    void check_device_ptr(const void* ptr, const char* what) const {
+#ifndef HFB200_EMU
+        cudaPointerAttributes a{};
+        const cudaError_t e = cudaPointerGetAttributes(&a, ptr);
+        if (e != cudaSuccess) cudaGetLastError();  // not a pointer the driver knows: clear the error, refuse below
+        if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != device_id)
+            throw Err(std::string("HFB200_DEV_INPUTS: ") + what + " is not device memory of device " + std::to_string(device_id));
+#else
+        (void)ptr; (void)what;
+#endif
+    }
+    Staged stage_inputs(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind, bool dev_inputs = false) {
         t_begin = std::chrono::steady_clock::now();
         bind();
         layout(p);
@@ -379,12 +392,18 @@ struct Prover {
         for (uint32_t i = 0; i < N_GLOBAL; i++) if (globals_h[i] >= P) throw Err("globals: non-canonical field element");
         if (data_h && !code_h && !control_cached) throw Err("code is NULL and no control group is resident for this po2 (hfb200_control_root)");
         if (!data_h && !have_trace) throw Err("no trace: pass code/data (code may be NULL after hfb200_control_root) or call hfb200_witgen_synth first");
+        if (dev_inputs && code_h) check_device_ptr(code_h, "code");
+        if (dev_inputs && data_h) check_device_ptr(data_h, "data");
         std::memcpy(globals, globals_h, sizeof globals);
         mark(0);
         bool chunked = false;
-        if (code_h) { dev.h2d(tr[GROUP_CODE], code_h, (size_t)cir.cd.w_code * N * 4); }
+        if (code_h) {
+            if (dev_inputs) dev.d2d(tr[GROUP_CODE], code_h, (size_t)cir.cd.w_code * N * 4);
+            else dev.h2d(tr[GROUP_CODE], code_h, (size_t)cir.cd.w_code * N * 4);
+        }
+        if (dev_inputs && data_h) dev.d2d(tr[GROUP_DATA], data_h, (size_t)cir.cd.w_data * N * 4);  // in stream order: no chunking needed
 #ifndef HFB200_EMU
-        if (data_h && cir.cd.w_data >= (uint32_t)H2D_CHUNKS) {
+        else if (data_h && cir.cd.w_data >= (uint32_t)H2D_CHUNKS) {
             // the copy stream may not overwrite the data columns before everything already queued on the main
             // stream (a previous segment's readers) has finished
             CUDA_CHECK(cudaEventRecord(copy_gate, dev.stream));
@@ -404,7 +423,7 @@ struct Prover {
             chunked = true;
         } else
 #endif
-        if (data_h) { dev.h2d(tr[GROUP_DATA], data_h, (size_t)cir.cd.w_data * N * 4); }
+        if (data_h && !dev_inputs) { dev.h2d(tr[GROUP_DATA], data_h, (size_t)cir.cd.w_data * N * 4); }
         const bool use_control = !code_h && data_h && control_cached;
         if (code_h) { control_cached = false; control_gen = 0; }  // the resident control columns change
         if (data_h) have_trace = true;
@@ -428,8 +447,8 @@ struct Prover {
     }
 
     // ---- SegmentProver::prove, phase 1: header + CODE + DATA commits, returns the accum mix ----
-    void begin(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind) {
-        const Staged sg = stage_inputs(p, globals_h, code_h, data_h, blind);
+    void begin(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind, bool dev_inputs = false) {
+        const Staged sg = stage_inputs(p, globals_h, code_h, data_h, blind, dev_inputs);
         const bool chunked = sg.chunked, use_control = sg.use_control;
         const size_t N = (size_t)1 << po2;
         mark(1);
@@ -462,6 +481,44 @@ struct Prover {
         for (auto& m : mix) m = rng.random_elem();
         cp_add("accum_mix", mix.data(), mix.size());
         begun = true;
+    }
+
+    // ---- the device seam of the two-phase form (hfb200_segment_begin_dev .. _finish_dev) ----
+    uint32_t* d_globals = nullptr;  // per segment, from the arena: valid until the segment is finished
+    // begin, then the mix and the globals in device memory for the caller's step_accum
+    void begin_dev(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind, bool dev_inputs) {
+        begin(p, globals_h, code_h, data_h, blind, dev_inputs);
+        d_globals = arena.take<uint32_t>(N_GLOBAL);
+        h2d_small(d_globals, globals, N_GLOBAL * 4);
+        h2d_small(d_mix, mix.data(), mix.size() * 4);
+    }
+    // in-place inclusive scan (product or sum) of the Fp4 chains in accum columns 4c..4c+3, rows [0, rows)
+    void accum_scan(int kind, uint32_t first_chain, uint32_t n_chains, uint64_t rows) {
+        if (!begun) throw Err("hfb200_segment_accum_scan: no segment in flight");
+        if (kind != SCAN_PRODUCT && kind != SCAN_SUM) throw Err("hfb200_segment_accum_scan: kind must be HFB200_SCAN_PRODUCT (0) or HFB200_SCAN_SUM (1)");
+        const uint32_t chains = cir.cd.w_accum / 4;
+        if ((uint64_t)first_chain + n_chains > chains)
+            throw Err("hfb200_segment_accum_scan: chains [" + std::to_string(first_chain) + ", " + std::to_string((uint64_t)first_chain + n_chains) +
+                      ") beyond w_accum / 4 = " + std::to_string(chains));
+        const uint64_t N = 1ull << po2;
+        if (rows > N) throw Err("hfb200_segment_accum_scan: rows " + std::to_string(rows) + " > N = " + std::to_string(N));
+        if (n_chains == 0 || rows == 0) return;
+        bind();
+        const uint32_t nblk = (uint32_t)((rows + ACC_RPB - 1) / ACC_RPB);
+        const size_t save = arena.off;
+        E4* partial = arena.take<E4>((size_t)n_chains * nblk);
+        const size_t sm = (SCAN_TILE + 2 * ACC_ITEMS) * sizeof(E4);
+        dev.launch<AccumScanKernel, 256, 1>(nblk, n_chains, 256, sm, tr[GROUP_ACCUM], N, rows, first_chain, kind, partial, 0);
+        dev.launch<AccumOffsetsKernel, 256, 1>(1, n_chains, 256, 2 * (size_t)nblk * sizeof(E4), partial, nblk, kind);
+        dev.launch<AccumScanKernel, 256, 1>(nblk, n_chains, 256, sm, tr[GROUP_ACCUM], N, rows, first_chain, kind, partial, 1);
+        arena.off = save;  // stream order makes reuse by later kernels safe
+    }
+    // the ZK_CYCLES blinding rows of every accum column, from this segment's key
+    void accum_blind() {
+        if (!begun) throw Err("hfb200_segment_accum_blind: no segment in flight");
+        bind();
+        const uint64_t total = (uint64_t)cir.cd.w_accum * ZK_CYCLES;
+        dev.launch<AccumBlindKernel, 256, 1>((unsigned)((total + 255) / 256), 1, 256, 0, tr[GROUP_ACCUM], cir.cd.w_accum, po2, ZK_CYCLES, blind_key);
     }
 
     // key_dev != NULL: the blinding key is read from device memory (graph replay); the by-value copy is then a placeholder
@@ -520,20 +577,27 @@ struct Prover {
     }
 
     // ---- phase 2: ACCUM commit, check polynomial, DEEP, FRI, queries ----
-    void finish(const uint32_t* accum_h, std::vector<uint32_t>& seal_out) {
-        if (!begun) throw Err("segment_finish without segment_begin");
+    // dev_accum: hfb200_segment_finish_dev -- the accum columns are already in device memory (the caller's step_accum); ms_accum
+    // is then the stream time from the end of the DATA commit (begin's event 5) to this call
+    void finish(const uint32_t* accum_h, std::vector<uint32_t>& seal_out, bool dev_accum = false) {
+        if (!begun) throw Err(dev_accum ? "hfb200_segment_finish_dev: no segment in flight" : "segment_finish without segment_begin");
         begun = false;
         bind();
         const size_t N = (size_t)1 << po2, D = 4 * N;
         const CircuitDev& cd = cir.cd;
         const uint32_t W = cir.n_regs(), T = cir.n_taps;
 
-        mark(5);
-        h2d_small(d_mix, mix.data(), mix.size() * 4);
-        if (accum_h) dev.h2d(tr[GROUP_ACCUM], accum_h, (size_t)cd.w_accum * N * 4);
-        else if (gen.active) throw Err("data-defined circuit: step_accum is the caller's (pass the accum columns to hfb200_segment_finish)");
-        else step_accum();
-        mark(6);
+        if (dev_accum) {
+            mark(6);
+            h2d_small(d_mix, mix.data(), mix.size() * 4);  // after begin (host) the mix is not on the device yet
+        } else {
+            mark(5);
+            h2d_small(d_mix, mix.data(), mix.size() * 4);
+            if (accum_h) dev.h2d(tr[GROUP_ACCUM], accum_h, (size_t)cd.w_accum * N * 4);
+            else if (gen.active) throw Err("data-defined circuit: step_accum is the caller's (pass the accum columns to hfb200_segment_finish)");
+            else step_accum();
+            mark(6);
+        }
         { StageRange r("hfb200:commit_accum"); commit_group(GROUP_ACCUM, "accum_root", 6, 7, 8); }  // ends with a stream sync: events 5..8 are complete
         stage_ms[3] = between(5, 6);
         stage_ms[1] += between(6, 7);

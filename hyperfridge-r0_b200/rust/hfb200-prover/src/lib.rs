@@ -179,8 +179,10 @@ impl B200Prover {
 
     fn prove_session(&self, ctx: &VerifierContext, session: &Session) -> Result<ProveInfo> {
         // Segments are independent (SURVEY.md section 8e): one worker thread and one context per GPU, segments handed out
-        // from a shared index; no collective, only the seals return.  (With witness generation on the host the pool of
-        // include/hfb200.h -- hfb200_pool_prove -- cannot be used directly: its jobs are one-shot and step_accum is upstream's.)
+        // from a shared index; no collective, only the seals return.  (The pool of include/hfb200.h -- hfb200_pool_prove with
+        // hfb200_pool_set_accum -- carries upstream's step_accum once it runs on the device: a callback that launches
+        // rv32im-sys's accum kernel on seg.stream.  That kernel is not part of this crate, so segments go through the host
+        // two-phase path of B200SegmentProver here.)
         let n = session.segments.len();
         let next = std::sync::atomic::AtomicUsize::new(0);
         let seals: Vec<std::sync::Mutex<Option<Result<Seal>>>> = (0..n).map(|_| std::sync::Mutex::new(None)).collect();
@@ -259,18 +261,12 @@ pub fn b200_prover() -> Rc<dyn Prover> {
 }
 
 fn visible_gpus() -> i32 {
-    // the library has no device-count entry on purpose (plain C ABI, no CUDA types): probe by initialising
-    let mut n = 0;
-    loop {
-        let mut ctx = std::ptr::null_mut();
-        let desc = sys::hfb200_circuit_desc { w_code: 16, w_data: 16, w_accum: 8, flags: 0 };
-        let e = unsafe { sys::hfb200_init(n, 12, &desc, &mut ctx) };
-        if !e.is_null() {
-            unsafe { sys::hfb200_free_error(e) };
-            break;
-        }
-        unsafe { sys::hfb200_destroy(ctx) };
-        n += 1;
+    // a count is a query: no device or no driver is 0 GPUs, not an error (the prover then fails when it creates a context)
+    let mut n: std::os::raw::c_int = 0;
+    let e = unsafe { sys::hfb200_device_count(&mut n) };
+    if !e.is_null() {
+        unsafe { sys::hfb200_free_error(e) };
+        return 1;
     }
     n.max(1)
 }

@@ -1,7 +1,7 @@
 //! Raw bindings of `include/hfb200.h`.  Error convention is the one of upstream's sys crates
 //! (`risc0_sys::ffi_wrap`): NULL = success, otherwise a malloc'd C string released with `hfb200_free_error`.
 #![allow(non_camel_case_types)]
-use std::os::raw::{c_char, c_int, c_uint};
+use std::os::raw::{c_char, c_int, c_uint, c_void};
 
 #[repr(C)]
 pub struct hfb200_ctx {
@@ -82,6 +82,37 @@ pub const HFB200_EXIT_SYSTEM_SPLIT: u32 = 1;
 pub const HFB200_BLIND_OS_ENTROPY: c_int = 0;
 pub const HFB200_BLIND_DETERMINISTIC: c_int = 1;
 
+/// The segment in flight between `hfb200_segment_begin_dev` and `hfb200_segment_finish_dev`: device pointers of the committed
+/// columns, the mix and the writable accum columns (valid until the segment is finished), and the context's stream.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct hfb200_segment_dev {
+    pub po2: u32,
+    /// the last `zk_rows` rows of DATA and ACCUM are blinding rows
+    pub zk_rows: u32,
+    pub w_code: u32,
+    pub w_data: u32,
+    pub w_accum: u32,
+    pub n_mix: u32,
+    pub device: c_int,
+    /// the context's `cudaStream_t` (null in the host emulator)
+    pub stream: *mut c_void,
+    pub code: *const u32,
+    pub data: *const u32,
+    pub globals: *const u32,
+    pub mix: *const u32,
+    pub accum: *mut u32,
+    pub mix_host: *const u32,
+    pub globals_host: *const u32,
+    pub blind_seed: u64,
+}
+pub const HFB200_DEV_INPUTS: u32 = 1;
+pub const HFB200_SCAN_PRODUCT: c_int = 0;
+pub const HFB200_SCAN_SUM: c_int = 1;
+/// The caller's step_accum for every job of a pool (`hfb200_pool_set_accum`); nonzero fails the job.
+pub type hfb200_accum_fn =
+    Option<unsafe extern "C" fn(user: *mut c_void, ctx: *mut hfb200_ctx, seg: *const hfb200_segment_dev, job: usize) -> c_int>;
+
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
 pub struct hfb200_pool_stats_t {
@@ -112,6 +143,22 @@ extern "C" {
         mix_out: *mut u32, mix_cap: usize, mix_words: *mut usize,
     ) -> *const c_char;
     pub fn hfb200_segment_finish(ctx: *mut hfb200_ctx, accum_or_null: *const u32, seal_out: *mut u32, seal_cap: usize, seal_words: *mut usize) -> *const c_char;
+    /// `hfb200_segment_begin`, then `out` describes the segment in device memory; flags: `HFB200_DEV_INPUTS` (code / data are
+    /// device pointers on the context's device).
+    pub fn hfb200_segment_begin_dev(
+        ctx: *mut hfb200_ctx, po2: u32, globals: *const u32, code: *const u32, data: *const u32, blind_seed: u64, flags: u32,
+        out: *mut hfb200_segment_dev,
+    ) -> *const c_char;
+    /// Commits the accum columns as they stand in device memory and completes the seal.
+    pub fn hfb200_segment_finish_dev(ctx: *mut hfb200_ctx, seal_out: *mut u32, seal_cap: usize, seal_words: *mut usize) -> *const c_char;
+    /// `Hal::prefix_products` (kind `HFB200_SCAN_PRODUCT`) or running sums (`HFB200_SCAN_SUM`) of the Fp4 chains in accum columns
+    /// 4c..4c+3, rows [0, rows), in place on the context's stream.
+    pub fn hfb200_segment_accum_scan(ctx: *mut hfb200_ctx, kind: c_int, first_chain: u32, n_chains: u32, rows: usize) -> *const c_char;
+    /// The accum group's blinding rows from the segment's blinding key.
+    pub fn hfb200_segment_accum_blind(ctx: *mut hfb200_ctx) -> *const c_char;
+    /// Number of CUDA devices; 0 (and success) without a device or a driver.
+    pub fn hfb200_device_count(out: *mut c_int) -> *const c_char;
+    pub fn hfb200_pool_set_accum(pool: *mut hfb200_pool, f: hfb200_accum_fn, user: *mut c_void) -> *const c_char;
     pub fn hfb200_pool_create(
         devices: *const c_int, n_devices: c_int, contexts_per_device: c_int, max_po2: u32, circuit: *const hfb200_circuit_desc,
         out: *mut *mut hfb200_pool,

@@ -46,7 +46,9 @@ typedef struct {
  *           CONST a = canonical value | GET a = tap index | GET_GLOBAL a = 0 (globals) / 1 (mix), b = offset |
  *           ADD/SUB/MUL a, b = fp vars | TRUE | AND_EQZ a = mix var, b = fp var | AND_COND a = mix var, b = fp cond, c = inner mix var
  * Limits: <= 4 taps per register, <= 4 distinct back values, <= 8 distinct tap sets.  For a data-defined circuit the
- * witness and the accum columns are the caller's (two-phase API); hfb200_witgen_synth / finish(NULL) are refused. */
+ * witness and the accum columns are the caller's: two-phase API, either on the host (hfb200_segment_begin / _finish with
+ * the columns) or on the device (hfb200_segment_begin_dev / _finish_dev, or a pool with hfb200_pool_set_accum);
+ * hfb200_witgen_synth / finish(NULL) are refused. */
 typedef struct { uint32_t group, offset, back; } hfb200_tap;
 typedef struct { uint32_t op, a, b, c; } hfb200_poly_step;
 enum { HFB200_OP_CONST = 0, HFB200_OP_GET = 1, HFB200_OP_GET_GLOBAL = 2, HFB200_OP_ADD = 3, HFB200_OP_SUB = 4, HFB200_OP_MUL = 5,
@@ -127,6 +129,48 @@ const char* hfb200_segment_begin(hfb200_ctx* ctx, uint32_t po2, const uint32_t* 
                                  const uint32_t* data, uint64_t blind_seed, uint32_t* mix_out, size_t mix_cap, size_t* mix_words);
 const char* hfb200_segment_finish(hfb200_ctx* ctx, const uint32_t* accum_or_null, uint32_t* seal_out, size_t seal_cap, size_t* seal_words);
 
+/* Two-phase form on DEVICE memory (upstream's GPU path keeps witgen and step_accum on the device).  begin_dev is
+ * hfb200_segment_begin plus a description of the segment in flight: the committed columns, the mix and the writable accum
+ * columns, all in the context's device memory.  The caller's step_accum writes the accum columns in place, on `stream` or on
+ * its own streams; finish_dev then commits them as they stand.  Every pointer stays valid until the segment is finished. */
+typedef struct {
+    uint32_t po2;            /* N = 2^po2 rows                                                                          */
+    uint32_t zk_rows;        /* the last zk_rows rows of DATA and ACCUM are blinding rows (upstream ZK_CYCLES)           */
+    uint32_t w_code, w_data, w_accum, n_mix;
+    int device;              /* CUDA ordinal of the context                                                            */
+    void* stream;            /* the context's cudaStream_t (NULL in the host emulator)                                  */
+    const uint32_t* code;    /* device u32[w_code][N]: committed control columns                                        */
+    const uint32_t* data;    /* device u32[w_data][N]: committed witness columns                                        */
+    const uint32_t* globals; /* device [32]                                                                             */
+    const uint32_t* mix;     /* device [n_mix]: the accum mix drawn after the DATA commit                               */
+    uint32_t* accum;         /* device u32[w_accum][N]: the caller writes these                                         */
+    const uint32_t* mix_host;     /* host copies, owned by the context                                                  */
+    const uint32_t* globals_host;
+    uint64_t blind_seed;
+} hfb200_segment_dev;
+/* flags of hfb200_segment_begin_dev: `code` / `data` are device pointers on the context's device, copied device to device on
+ * the context's stream (the copy follows the stream's earlier work; anything writing them on other streams must be complete).
+ * A pointer that is not device memory of that device is refused before anything is queued. */
+enum { HFB200_DEV_INPUTS = 1 };
+/* `code == NULL` reuses the resident control group as in hfb200_segment_begin; `data` may be NULL after hfb200_witgen_synth. */
+const char* hfb200_segment_begin_dev(hfb200_ctx* ctx, uint32_t po2, const uint32_t* globals, const uint32_t* code, const uint32_t* data,
+                                     uint64_t blind_seed, uint32_t flags, hfb200_segment_dev* out);
+/* Completes the segment begun by either begin, from the accum columns as they stand in device memory (no upload, no built-in
+ * step_accum).  The caller's accum work must be enqueued on `stream`, or complete on the caller's own streams, before the
+ * call.  hfb200_last_stats then reports as ms_accum the device time on the stream from the end of the DATA commit to this
+ * call: the caller's kernels AND any idle time of the stream in between. */
+const char* hfb200_segment_finish_dev(hfb200_ctx* ctx, uint32_t* seal_out, size_t seal_cap, size_t* seal_words);
+/* Device form of risc0-zkp `Hal::prefix_products` (and of the running sums of LogUp-style arguments): an in-place inclusive scan
+ * of the Fp4 chains stored in accum columns 4c..4c+3, c in [first_chain, first_chain + n_chains), over rows [0, rows), on the
+ * context's stream.  Valid between a begin and its finish. */
+enum { HFB200_SCAN_PRODUCT = 0, HFB200_SCAN_SUM = 1 };
+const char* hfb200_segment_accum_scan(hfb200_ctx* ctx, int kind, uint32_t first_chain, uint32_t n_chains, size_t rows);
+/* Writes the zk_rows blinding rows of every accum column from the segment's blinding key (the rows the built-in step_accum
+ * writes; the key itself never leaves the library).  On the context's stream; valid between a begin and its finish. */
+const char* hfb200_segment_accum_blind(hfb200_ctx* ctx);
+/* Number of CUDA devices.  No device or no driver is a count of 0 (NULL returned), not an error. */
+const char* hfb200_device_count(int* out);
+
 /* Witness stand-in on the device (replaces preflight + WitnessGenerator for the synthetic circuit):
  * fills the context's resident code/data columns; globals_out receives the 32 global words. */
 const char* hfb200_witgen_synth(hfb200_ctx* ctx, uint32_t po2, uint64_t trace_seed, uint64_t blind_seed, uint32_t* globals_out);
@@ -198,7 +242,8 @@ typedef struct {
     float ms_h2d;          /* host->device trace copies (0 for resident)                                  */
     float ms_ntt_main;     /* iNTT+zk_shift and expand+NTT (LDE) of code+data+accum columns               */
     float ms_hash_main;    /* Poseidon2 leaf hashing + tree folds of code+data+accum                      */
-    float ms_accum;        /* step_accum                                                                  */
+    float ms_accum;        /* step_accum (after hfb200_segment_finish_dev: stream time from the DATA commit to the call,  */
+                           /* the caller's accum kernels and any idle time together)                                      */
     float ms_check;        /* eval_check + check-group commit                                             */
     float ms_deep;         /* DEEP evaluations + quotient                                                 */
     float ms_fri;          /* FRI rounds + query openings                                                 */
@@ -217,7 +262,8 @@ uint64_t hfb200_total_launches(const hfb200_ctx* ctx);
 /* ---- multi-GPU: a pool of contexts fed from one queue of independent segments --------------------------------- */
 /* Replaces the segment loop of upstream's `ProverImpl::prove_session` (sequential there).  One worker thread per
  * (device, slot); whole segments are handed out longest-first (by po2); no collective, only seals return.  Seals depend
- * on (trace, blind_seed) only, so the result is identical for any number of devices. */
+ * on (trace, blind_seed) only, so the result is identical for any number of devices.  A pool proves data-defined circuits
+ * once it has an accum callback (hfb200_pool_set_accum); without one their jobs are refused (step_accum is the caller's). */
 typedef struct hfb200_pool hfb200_pool;
 typedef struct {
     uint32_t po2;
@@ -264,6 +310,14 @@ const char* hfb200_pool_inject_fault(hfb200_pool* pool, size_t worker, uint64_t 
  * per load (each call starts a new generation, so a reload -- same pointer or not -- is re-committed by every worker before its
  * next code == NULL job) and reuses it; seals are identical to the ones produced with the columns passed per job. */
 const char* hfb200_pool_load_control(hfb200_pool* pool, uint32_t po2, const uint32_t* code);
+/* The caller's step_accum for every job of the pool (both kinds of pool; on a built-in pool it replaces the built-in one).  Each
+ * job then runs hfb200_segment_begin_dev (host inputs, as jobs carry them), fn on the worker thread (the context's device is
+ * current; `job` = index into the jobs array), hfb200_segment_finish_dev.  Callbacks run concurrently, one per worker, and may
+ * call only hfb200_segment_accum_scan / _accum_blind on the `ctx` they are given (plus their own kernels on seg->stream).  A
+ * nonzero return fails that job only ("accum callback returned <rc>"), is not retried, and leaves the context usable; a CUDA
+ * error takes the device-fault path above.  fn = NULL removes the callback. */
+typedef int (*hfb200_accum_fn)(void* user, hfb200_ctx* ctx, const hfb200_segment_dev* seg, size_t job);
+const char* hfb200_pool_set_accum(hfb200_pool* pool, hfb200_accum_fn fn, void* user);
 void hfb200_pool_destroy(hfb200_pool* pool);
 
 /* ---- HAL-level operators (second seam: risc0-zkp `Hal` methods), host buffers in/out ----------- */
