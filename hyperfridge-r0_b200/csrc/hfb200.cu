@@ -623,7 +623,7 @@ const char* hfb200_op_poseidon2(hfb200_ctx* ctx, uint32_t* states, size_t n) {
     Dev& d = ctx->p.dev;
     DevBuf b(d, n * 24);
     d.h2d(b.p, states, n * 24 * 4);
-    d.launch<PermuteKernel, 128, 1>((unsigned)((n + 127) / 128), 1, 128, 0, b.p, (uint32_t)n);
+    ctx->p.merkle.permute(b.p, (uint32_t)n);
     d.d2h(states, b.p, n * 24 * 4);
     d.sync();
     API_CATCH

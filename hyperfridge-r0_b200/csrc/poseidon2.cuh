@@ -13,7 +13,66 @@ namespace hf {
 struct P2Consts {
     uint32_t rc_first[96], rc_partial[21], rc_last[96], diag[24];  // Montgomery form
     uint32_t diag_std[24], diag_shoup[24];  // canonical d_i and floor(d_i * 2^32 / p): constant multiplier in Shoup form
+    int32_t tri_c[21];  // partial rounds in tensor form: c_k = (M_I^k)[0][0] * 2^32 mod p, balanced in (-p/2, p/2], k = 1..20
 };
+
+// ---- the 21 partial rounds as two linear maps ----------------------------------------------------------------------------
+// Partial round r (r = 0..20) on state v_r: cell 0 becomes sbox(v_r[0] + rc_r), then v_{r+1} = M_I (v_r + delta_r e0) with
+// M_I = 1 1^T + diag(d) and delta_r = sbox(v_r[0] + rc_r) - v_r[0].  Unrolled from the state v = v_0 entering the section:
+//   v_r[0] = a_r . v + sum_{j<r} c_{r-j} delta_j         a_r = e0^T M_I^r,  c_k = (M_I^k)[0][0]
+//   v_21   = M_I^21 v + sum_j delta_j M_I^(21-j) e0      (one 24 x 45 map of [v | delta])
+// so everything but the S-boxes and the 210-term triangular sum is two dense maps over the states of a CTA: GEMM 1 yields
+// a_1..a_20 . v (20 outputs), GEMM 2 yields v_21 (24 outputs).  Both run exactly on the int8 tensor cores: the 32-bit input
+// words are split into their 4 bytes (K = 4 per input), the byte weight 2^(8b) and the Montgomery factor 2^32 are folded
+// into the constant, C'_((i,b),o) = 2^(8b) * m_oi * 2^32 mod p, whose 4 bytes j form 4 output planes (N = 4 per output).
+// Plane j accumulates Q_j = sum bytes * bytes <= 180 * 255^2 < 2^24 in int32; V = sum_j 2^(8j) Q_j < 2^49 < p 2^32, so one
+// Montgomery REDC of V is the Montgomery residue of the output.  The state words need no conversion: a little-endian u32 is
+// already its 4 byte inputs.
+static constexpr uint32_t P2TC_K1 = 96, P2TC_N1 = 80;    // GEMM 1: bytes of v -> 4 planes of a_1..a_20 . v
+static constexpr uint32_t P2TC_K2 = 192, P2TC_N2 = 96;   // GEMM 2: bytes of [v | delta_0..20 | 0 0 0] -> 4 planes of v_21
+static constexpr uint32_t P2TC_B1_BYTES = P2TC_K1 * P2TC_N1, P2TC_B_BYTES = P2TC_B1_BYTES + P2TC_K2 * P2TC_N2;
+// Operand layout of both GEMMs (tcgen05 shared-memory descriptor, K-major, no swizzle): core matrices of 8 rows x 16 bytes,
+// 128 contiguous bytes each; the next 16 bytes along K are 128 bytes further (LBO), the next 8 rows 8 K bytes further (SBO).
+HD uint32_t p2tc_off(uint32_t row, uint32_t k, uint32_t K) { return (row >> 3) * (K * 8) + (k >> 4) * 128 + (row & 7) * 16 + (k & 15); }
+struct P2TcTables {
+    uint8_t b[P2TC_B_BYTES];  // B operands (rows = the N output planes) in the layout above: GEMM 1, then GEMM 2
+};
+
+static inline uint32_t p2_mod_mul(uint32_t a, uint32_t b) { return (uint32_t)((uint64_t)a * b % P); }
+// M_I^k for k = 0..21, canonical entries, exact
+static inline std::vector<std::vector<uint32_t>> p2_m_int_powers() {
+    std::vector<std::vector<uint32_t>> pw(22, std::vector<uint32_t>(24 * 24, 0));
+    for (int i = 0; i < 24; i++) pw[0][i * 24 + i] = 1;
+    for (int k = 1; k < 22; k++)
+        for (int o = 0; o < 24; o++)
+            for (int i = 0; i < 24; i++) {  // (M_I X)[o][i] = sum_l X[l][i] + d_o X[o][i]
+                uint64_t acc = p2_mod_mul(P2_M_INT_DIAG[o], pw[k - 1][o * 24 + i]);
+                for (int l = 0; l < 24; l++) acc += pw[k - 1][l * 24 + i];
+                pw[k][o * 24 + i] = (uint32_t)(acc % P);
+            }
+    return pw;
+}
+// one linear output o = sum_i m_i x_i of a GEMM with K input bytes, written as byte planes n = 4 o + j
+static inline void p2tc_put_output(uint8_t* b, uint32_t K, uint32_t o, const uint32_t* m, int n_in) {
+    for (int i = 0; i < n_in; i++)
+        for (uint32_t bb = 0; bb < 4; bb++) {
+            const uint32_t c = to_mont(p2_mod_mul(m[i], 1u << (8 * bb)));  // 2^(8b) m_i 2^32 mod p
+            for (uint32_t j = 0; j < 4; j++) b[p2tc_off(4 * o + j, 4 * i + bb, K)] = (uint8_t)(c >> (8 * j));
+        }
+}
+static inline P2TcTables p2_make_tc_tables() {
+    P2TcTables t;
+    std::memset(t.b, 0, sizeof t.b);
+    const auto pw = p2_m_int_powers();
+    uint32_t m[45];
+    for (uint32_t r = 1; r <= 20; r++) p2tc_put_output(t.b, P2TC_K1, r - 1, &pw[r][0], 24);  // row 0 of M_I^r
+    for (uint32_t o = 0; o < 24; o++) {
+        for (int i = 0; i < 24; i++) m[i] = pw[21][o * 24 + i];
+        for (int j = 0; j < 21; j++) m[24 + j] = pw[21 - j][o * 24];  // (M_I^(21-j) e0)[o]
+        p2tc_put_output(t.b + P2TC_B1_BYTES, P2TC_K2, o, m, 45);
+    }
+    return t;
+}
 
 static inline P2Consts p2_make_consts() {
     P2Consts c;
@@ -24,16 +83,24 @@ static inline P2Consts p2_make_consts() {
         c.diag_std[i] = P2_M_INT_DIAG[i];
         c.diag_shoup[i] = (uint32_t)(((uint64_t)P2_M_INT_DIAG[i] << 32) / P);
     }
+    const auto pw = p2_m_int_powers();
+    c.tri_c[0] = 0;
+    for (int k = 1; k < 21; k++) {
+        const uint32_t v = to_mont(pw[k][0]);
+        c.tri_c[k] = v > (P - 1) / 2 ? (int32_t)v - (int32_t)P : (int32_t)v;
+    }
     return c;
 }
 
 #if !defined(HFB200_EMU)
 __constant__ P2Consts g_p2c;
 #define P2C_DEV g_p2c
+__device__ __align__(16) uint8_t g_p2tc_b[P2TC_B_BYTES];
 #endif
 static P2Consts g_p2c_host;
+static P2TcTables g_p2tc_host;
 static inline const P2Consts& p2_host_consts() {
-    static const bool once = (g_p2c_host = p2_make_consts(), true);  // thread-safe one-time initialisation
+    static const bool once = (g_p2c_host = p2_make_consts(), g_p2tc_host = p2_make_tc_tables(), true);  // thread-safe one-time initialisation
     (void)once;
     return g_p2c_host;
 }
@@ -144,15 +211,19 @@ HD void p2_m_int(uint32_t* s, const P2Consts& k) {
     for (int i = 0; i < 24; i++) s[i] = padd(sum, fmul_const(s[i], k.diag_std[i], k.diag_shoup[i]));
 }
 
-HD void p2_mix(uint32_t* s) {
-    const P2Consts& k = p2c();
-    p2_m_ext(s);
+HD void p2_full_rounds(uint32_t* s, const uint32_t* rc) {
 #pragma unroll 1
     for (int r = 0; r < 4; r++) {
 #pragma unroll
-        for (int i = 0; i < 24; i++) s[i] = sbox7_rc(s[i], k.rc_first[r * 24 + i]);
+        for (int i = 0; i < 24; i++) s[i] = sbox7_rc(s[i], rc[r * 24 + i]);
         p2_m_ext(s);
     }
+}
+
+HD void p2_mix(uint32_t* s) {
+    const P2Consts& k = p2c();
+    p2_m_ext(s);
+    p2_full_rounds(s, k.rc_first);
 #if P2_DEFERRED_SUM
     // Partial rounds with the row sum carried instead of recomputed.  The round maps y_i -> mu_i y_i + S with S = sum_i y_i
     // (after the S-box on y_0).  With U = sum_{i>=1} y_i kept canonical:  S = y_0 + U,  t_i = mu_i y_i (Shoup: accepts ANY
@@ -193,60 +264,302 @@ HD void p2_mix(uint32_t* s) {
         p2_m_int(s, k);
     }
 #endif
-#pragma unroll 1
-    for (int r = 0; r < 4; r++) {
-#pragma unroll
-        for (int i = 0; i < 24; i++) s[i] = sbox7_rc(s[i], k.rc_last[r * 24 + i]);
-        p2_m_ext(s);
-    }
+    p2_full_rounds(s, k.rc_last);
 }
+
+// ---- permutation with the partial rounds on the tensor cores (see "the 21 partial rounds as two linear maps") ---------------
+// Device: one CTA of 128 threads = 128 states = the 128 TMEM lanes of a tcgen05.mma (M = 128, kind::i8, cta_group::1).
+// Thread t writes its A row (the 48 words [v | delta | 0]) into shared memory, one thread issues the MMAs, tcgen05.commit
+// arrives on an mbarrier, and thread t reads its own row of the int32 planes back with tcgen05.ld.  Every thread of the CTA
+// takes part in every permutation (the barriers are CTA-wide), so kernels run idle states on zeros instead of returning.
+// Emulator (and the nvcc host pass): the same row, tables, recombination and REDC, with plain loops in place of the MMA.
+#ifndef P2_TC
+#define P2_TC 1
+#endif
+static constexpr uint32_t P2TC_A_BYTES = 128 * P2TC_K2;
+static constexpr size_t P2TC_SMEM = P2TC_A_BYTES + P2TC_B_BYTES + 32;  // A tile, B operands, 2 mbarriers + the TMEM address
+static constexpr uint32_t P2TC_TMEM_COLS = 128;                        // >= N1, N2; 4 CTAs fill an SM's 512 columns
+
+struct P2Tc {
+#ifdef __CUDA_ARCH__
+    uint8_t* a;      // A tile, 128 rows x K2 bytes
+    uint8_t* b;      // B operands (P2TcTables::b)
+    uint64_t* bar;   // [0]: B operands loaded, [1]: MMA done
+    uint32_t* tslot; // TMEM base address written by tcgen05.alloc
+    uint32_t tmem, phase, row;
+    bool b_wait;     // thread 0: B operands not yet waited for
+#else
+    uint32_t w[48];  // this state's A row
+#endif
+};
+
+#ifdef __CUDA_ARCH__
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// K-major, no swizzle (layout of p2tc_off): LBO = 128 B, SBO = 8 K B, bits 46-48 = 0b001 (sm_100 descriptor version)
+__device__ __forceinline__ uint64_t p2tc_desc(uint32_t saddr, uint32_t K) {
+    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(128u >> 4) << 16) | ((uint64_t)((8u * K) >> 4) << 32) | (1ull << 46);
+}
+#endif
+
+// Per-CTA set-up: B operands into shared memory (one bulk copy), mbarriers, 128 TMEM columns.  All threads call it.
+HD void p2tc_begin(P2Tc& tc, const KCtx& cx, uint32_t* smem) {
+#ifdef __CUDA_ARCH__
+    uint8_t* base = reinterpret_cast<uint8_t*>(smem);
+    tc.a = base;
+    tc.b = base + P2TC_A_BYTES;
+    tc.bar = reinterpret_cast<uint64_t*>(base + P2TC_A_BYTES + P2TC_B_BYTES);
+    tc.tslot = reinterpret_cast<uint32_t*>(tc.bar + 2);
+    tc.phase = 0;
+    tc.row = (uint32_t)cx.tid;
+    tc.b_wait = cx.tid == 0;
+    if (cx.tid == 0) {
+        mbar_init(&tc.bar[0], 1);
+        mbar_init(&tc.bar[1], 1);
+        mbar_init_fence();
+        mbar_expect_tx(&tc.bar[0], P2TC_B_BYTES);
+        tma_bulk_g2s(tc.b, g_p2tc_b, P2TC_B_BYTES, &tc.bar[0]);
+    }
+    if (cx.tid < 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tc.tslot)), "r"(P2TC_TMEM_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    tc.tmem = *tc.tslot;
+#else
+    (void)tc; (void)cx; (void)smem;
+#endif
+}
+HD void p2tc_end(P2Tc& tc, const KCtx& cx) {
+#ifdef __CUDA_ARCH__
+    tc_fence_before();
+    __syncthreads();
+    if (cx.tid < 32) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tc.tmem), "r"(P2TC_TMEM_COLS) : "memory");
+    }
+#else
+    (void)tc; (void)cx;
+#endif
+}
+// words [w0, w0 + 4 n) of this state's A row
+HD void p2tc_put(P2Tc& tc, uint32_t w0, const uint32_t* v, uint32_t n) {
+#ifdef __CUDA_ARCH__
+#pragma unroll
+    for (uint32_t c = 0; c < n; c++)
+        *reinterpret_cast<uint4*>(tc.a + p2tc_off(tc.row, 4 * (w0 + 4 * c), P2TC_K2)) = make_uint4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
+#else
+    for (uint32_t i = 0; i < 4 * n; i++) tc.w[w0 + i] = v[i];
+#endif
+}
+// GEMM g (1 or 2) over the rows of all threads of the CTA; the planes land in TMEM columns [0, N_g)
+HD void p2tc_gemm(P2Tc& tc, int g) {
+#ifdef __CUDA_ARCH__
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy row stores -> visible to the MMA
+    tc_fence_before();                                             // earlier tcgen05.ld of these columns are complete
+    __syncthreads();
+    if (tc.row == 0) {
+        tc_fence_after();
+        if (tc.b_wait) { mbar_wait(&tc.bar[0], 0); tc.b_wait = false; }
+        const uint32_t K = g == 1 ? P2TC_K1 : P2TC_K2, N = g == 1 ? P2TC_N1 : P2TC_N2;
+        // kind::i8 instruction descriptor: D s32 (bits 4-5 = 2), A and B unsigned 8-bit, both K-major, N >> 3 at 17, M >> 4 at 24
+        const uint32_t idesc = (2u << 4) | ((N >> 3) << 17) | ((128u >> 4) << 24);
+        const uint32_t a0 = smem_u32(tc.a), b0 = smem_u32(tc.b) + (g == 1 ? 0u : P2TC_B1_BYTES);
+        for (uint32_t kk = 0; kk < K / 32; kk++) {  // K = 32 bytes per MMA: two core matrices along K
+            const uint64_t ad = p2tc_desc(a0 + kk * 256, P2TC_K2), bd = p2tc_desc(b0 + kk * 256, K);
+            asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
+                         ::"r"(tc.tmem), "l"(ad), "l"(bd), "r"(idesc), "r"(kk) : "memory");
+        }
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(&tc.bar[1])) : "memory");
+    }
+    mbar_wait(&tc.bar[1], tc.phase);
+    tc.phase ^= 1;
+    tc_fence_after();
+#else
+    (void)tc; (void)g;
+#endif
+}
+// 16 int32 columns [c0, c0 + 16) of this state's row of the last GEMM's result
+HD void p2tc_cols16(P2Tc& tc, int g, uint32_t c0, uint32_t* q) {
+#ifdef __CUDA_ARCH__
+    (void)g;
+    const uint32_t addr = tc.tmem + ((tc.row & ~31u) << 16) + c0;  // a warp reads its own 32 TMEM lanes
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
+                 "tcgen05.wait::ld.sync.aligned;\n"
+                 : "=r"(q[0]), "=r"(q[1]), "=r"(q[2]), "=r"(q[3]), "=r"(q[4]), "=r"(q[5]), "=r"(q[6]), "=r"(q[7]),
+                   "=r"(q[8]), "=r"(q[9]), "=r"(q[10]), "=r"(q[11]), "=r"(q[12]), "=r"(q[13]), "=r"(q[14]), "=r"(q[15])
+                 : "r"(addr) : "memory");
+#else
+    const uint8_t* a = reinterpret_cast<const uint8_t*>(tc.w);  // little-endian: word i = bytes 4i..4i+3
+    const uint32_t K = g == 1 ? P2TC_K1 : P2TC_K2;
+    const uint8_t* b = g_p2tc_host.b + (g == 1 ? 0u : P2TC_B1_BYTES);
+    for (uint32_t n = 0; n < 16; n++) {
+        uint32_t acc = 0;
+        for (uint32_t k = 0; k < K; k++) acc += (uint32_t)a[k] * b[p2tc_off(c0 + n, k, K)];
+        q[n] = acc;
+    }
+#endif
+}
+// REDC(sum_j 2^(8j) q_j) for planes q_j < 2^24: V < 2^49, split into its low and high words without 64-bit arithmetic.
+// Canonical output.
+HD uint32_t p2tc_reduce(const uint32_t* q) {
+    const uint32_t a = q[1] + (q[0] >> 8), b = q[2] + (a >> 8), c = q[3] + (b >> 8);  // c = V >> 24
+    const uint32_t lo = q[0] + (q[1] << 8) + (q[2] << 16) + (q[3] << 24), hi = c >> 8;
+    const uint32_t m = lo * P_INV;
+#ifdef __CUDA_ARCH__
+    const uint32_t mp = __umulhi(m, P);
+#else
+    const uint32_t mp = (uint32_t)(((uint64_t)m * P) >> 32);
+#endif
+    const uint32_t r = hi - mp;  // (V - m p) / 2^32 in (-p, 2^17)
+    return umin32(r, r + P);
+}
+// sum_{j<n} c_j d_j for signed |c_j|, |d_j| <= p/2 and n <= 4: |sum| < p^2 < 2^31 p, so one signed REDC lands in (-p, p).
+// Canonical output (Montgomery: c_j carries the factor 2^32).
+HD uint32_t p2tc_dot4(const int32_t* c, const int32_t* d, int n) {
+    int64_t v = 0;
+#pragma unroll
+    for (int j = 0; j < n; j++) v += (int64_t)c[j] * d[j];
+    const int32_t m = (int32_t)((uint32_t)v * P_INV);
+#ifdef __CUDA_ARCH__
+    const int32_t mp = __mulhi(m, (int32_t)P);
+#else
+    const int32_t mp = (int32_t)(((int64_t)m * (int64_t)P) >> 32);
+#endif
+    const uint32_t r = (uint32_t)((int32_t)(v >> 32) - mp);
+    return umin32(r, r + P);
+}
+
+HD void p2_mix_tc(uint32_t* s, P2Tc& tc) {
+    const P2Consts& k = p2c();
+    p2_m_ext(s);
+    p2_full_rounds(s, k.rc_first);
+    // GEMM 1: L_r = a_r . v, r = 1..20
+    p2tc_put(tc, 0, s, 6);
+    p2tc_gemm(tc, 1);
+    uint32_t L[21];
+    L[0] = s[0];
+#pragma unroll
+    for (uint32_t c = 0; c < P2TC_N1; c += 16) {
+        uint32_t q[16];
+        p2tc_cols16(tc, 1, c, q);
+#pragma unroll
+        for (uint32_t o = 0; o < 4; o++) L[1 + c / 4 + o] = p2tc_reduce(q + 4 * o);
+    }
+    // the S-box chain: v_r[0] = L_r + sum_{j<r} c_{r-j} delta_j, delta_r kept balanced in (-p/2, p/2]
+    int32_t dlt[21];
+#pragma unroll
+    for (int r = 0; r < 21; r++) {
+        uint32_t y = L[r];
+#pragma unroll
+        for (int j0 = 0; j0 < r; j0 += 4) {
+            const int n = r - j0 < 4 ? r - j0 : 4;
+            int32_t cc[4], dd[4];
+#pragma unroll
+            for (int j = 0; j < 4; j++) if (j < n) { cc[j] = k.tri_c[r - j0 - j]; dd[j] = dlt[j0 + j]; }
+            y = fadd(y, p2tc_dot4(cc, dd, n));
+        }
+        const uint32_t d = fsub(sbox7_rc(y, k.rc_partial[r]), y);
+        dlt[r] = d > (P - 1) / 2 ? (int32_t)(d - P) : (int32_t)d;
+    }
+    // GEMM 2: v_21 = M_I^21 v + sum_j delta_j M_I^(21-j) e0 (the v bytes are still in the A row)
+    uint32_t w[24];
+#pragma unroll
+    for (int j = 0; j < 21; j++) { const uint32_t u = (uint32_t)dlt[j]; w[j] = umin32(u, u + P); }
+    w[21] = w[22] = w[23] = 0;
+    p2tc_put(tc, 24, w, 6);
+    p2tc_gemm(tc, 2);
+#pragma unroll
+    for (uint32_t c = 0; c < P2TC_N2; c += 16) {
+        uint32_t q[16];
+        p2tc_cols16(tc, 2, c, q);
+#pragma unroll
+        for (uint32_t o = 0; o < 4; o++) s[c / 4 + o] = p2tc_reduce(q + 4 * o);
+    }
+    p2_full_rounds(s, k.rc_last);
+}
+
+// The permutation the Merkle / permutation kernels run for one state per thread.  kAll: every thread of the block must
+// call mix() (idle states on zeros) and end().
+struct P2Perm {
+#if P2_TC
+    static constexpr bool kAll = true;
+    static constexpr int kMinBlocks = 4;  // 4 x 128 TMEM columns per SM; caps registers at 128
+    static constexpr size_t kSmem = P2TC_SMEM;
+    P2Tc tc;
+    HD P2Perm(const KCtx& cx, uint32_t* smem) { p2tc_begin(tc, cx, smem); }
+    HD void mix(uint32_t* s) { p2_mix_tc(s, tc); }
+    HD void end(const KCtx& cx) { p2tc_end(tc, cx); }
+#else
+    static constexpr bool kAll = false;
+    static constexpr int kMinBlocks = 1;
+    static constexpr size_t kSmem = 0;
+    HD P2Perm(const KCtx&, uint32_t*) {}
+    HD void mix(uint32_t* s) { p2_mix(s); }
+    HD void end(const KCtx&) {}
+#endif
+};
 
 // ---- kernels ------------------------------------------------------------------------------------
 // Hal::hash_rows: leaf r = unpadded sponge over matrix[c * col_stride + r], c < cols.  Digest -> nodes[rows + r].
 struct HashRowsKernel {
     static constexpr bool kBarrier = false;
-    HD static void run(const KCtx& cx, uint32_t*, const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
+    HD static void run(const KCtx& cx, uint32_t* smem, const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
         const uint64_t r = (uint64_t)cx.bx * cx.nt + cx.tid;
-        if (r >= rows) return;
+        const bool live = r < rows;
+        if (!live && !P2Perm::kAll) return;
+        P2Perm h(cx, smem);
         uint32_t s[24];
 #pragma unroll
         for (int i = 0; i < 24; i++) s[i] = 0;
-        const uint32_t* src = matrix + r;
+        const uint32_t* src = matrix + (live ? r : 0);
         uint32_t c = 0;
         for (; c + 16 <= cols; c += 16) {
 #pragma unroll
-            for (int i = 0; i < 16; i++) s[i] = src[(uint64_t)(c + i) * col_stride];
-            p2_mix(s);
+            for (int i = 0; i < 16; i++) s[i] = live ? src[(uint64_t)(c + i) * col_stride] : 0u;
+            h.mix(s);
         }
         if (c < cols || cols == 0) {
 #pragma unroll
-            for (int i = 0; i < 16; i++) s[i] = (c + i < cols) ? src[(uint64_t)(c + i) * col_stride] : 0u;
-            p2_mix(s);
+            for (int i = 0; i < 16; i++) s[i] = (live && c + i < cols) ? src[(uint64_t)(c + i) * col_stride] : 0u;
+            h.mix(s);
         }
-        uint4* dst = reinterpret_cast<uint4*>(nodes + ((uint64_t)rows + r) * 8);
-        dst[0] = make_uint4(s[0], s[1], s[2], s[3]);
-        dst[1] = make_uint4(s[4], s[5], s[6], s[7]);
+        if (live) {
+            uint4* dst = reinterpret_cast<uint4*>(nodes + ((uint64_t)rows + r) * 8);
+            dst[0] = make_uint4(s[0], s[1], s[2], s[3]);
+            dst[1] = make_uint4(s[4], s[5], s[6], s[7]);
+        }
+        h.end(cx);
     }
 };
 
 // Hal::hash_fold for one level: nodes[i] = H(nodes[2i] || nodes[2i+1]) for i in [level_size, 2*level_size).
 struct HashFoldKernel {
     static constexpr bool kBarrier = false;
-    HD static void run(const KCtx& cx, uint32_t*, uint32_t* nodes, uint32_t level_size) {
+    HD static void run(const KCtx& cx, uint32_t* smem, uint32_t* nodes, uint32_t level_size) {
         const uint64_t t = (uint64_t)cx.bx * cx.nt + cx.tid;
-        if (t >= level_size) return;
-        const uint64_t i = level_size + t;
-        const uint4* in = reinterpret_cast<const uint4*>(nodes + 2 * i * 8);
+        const bool live = t < level_size;
+        if (!live && !P2Perm::kAll) return;
+        P2Perm h(cx, smem);
+        const uint64_t i = level_size + (live ? t : 0);
         uint32_t s[24];
-        uint4 v0 = in[0], v1 = in[1], v2 = in[2], v3 = in[3];
-        s[0] = v0.x; s[1] = v0.y; s[2] = v0.z; s[3] = v0.w; s[4] = v1.x; s[5] = v1.y; s[6] = v1.z; s[7] = v1.w;
-        s[8] = v2.x; s[9] = v2.y; s[10] = v2.z; s[11] = v2.w; s[12] = v3.x; s[13] = v3.y; s[14] = v3.z; s[15] = v3.w;
 #pragma unroll
-        for (int k = 16; k < 24; k++) s[k] = 0;
-        p2_mix(s);
-        uint4* dst = reinterpret_cast<uint4*>(nodes + i * 8);
-        dst[0] = make_uint4(s[0], s[1], s[2], s[3]);
-        dst[1] = make_uint4(s[4], s[5], s[6], s[7]);
+        for (int k = 0; k < 24; k++) s[k] = 0;
+        if (live) {
+            const uint4* in = reinterpret_cast<const uint4*>(nodes + 2 * i * 8);
+            uint4 v0 = in[0], v1 = in[1], v2 = in[2], v3 = in[3];
+            s[0] = v0.x; s[1] = v0.y; s[2] = v0.z; s[3] = v0.w; s[4] = v1.x; s[5] = v1.y; s[6] = v1.z; s[7] = v1.w;
+            s[8] = v2.x; s[9] = v2.y; s[10] = v2.z; s[11] = v2.w; s[12] = v3.x; s[13] = v3.y; s[14] = v3.z; s[15] = v3.w;
+        }
+        h.mix(s);
+        if (live) {
+            uint4* dst = reinterpret_cast<uint4*>(nodes + i * 8);
+            dst[0] = make_uint4(s[0], s[1], s[2], s[3]);
+            dst[1] = make_uint4(s[4], s[5], s[6], s[7]);
+        }
+        h.end(cx);
     }
 };
 
@@ -366,13 +679,17 @@ struct HashFoldWarpTailKernel {
 // poseidon2_mix on n independent states (parity probe for the permutation itself).
 struct PermuteKernel {
     static constexpr bool kBarrier = false;
-    HD static void run(const KCtx& cx, uint32_t*, uint32_t* states, uint32_t n) {
+    HD static void run(const KCtx& cx, uint32_t* smem, uint32_t* states, uint32_t n) {
         const uint64_t t = (uint64_t)cx.bx * cx.nt + cx.tid;
-        if (t >= n) return;
+        const bool live = t < n;
+        if (!live && !P2Perm::kAll) return;
+        P2Perm h(cx, smem);
         uint32_t s[24];
-        for (int i = 0; i < 24; i++) s[i] = states[t * 24 + i];
-        p2_mix(s);
-        for (int i = 0; i < 24; i++) states[t * 24 + i] = s[i];
+        for (int i = 0; i < 24; i++) s[i] = live ? states[t * 24 + i] : 0u;
+        h.mix(s);
+        if (live)
+            for (int i = 0; i < 24; i++) states[t * 24 + i] = s[i];
+        h.end(cx);
     }
 };
 
@@ -383,21 +700,26 @@ struct Merkle {
         p2_host_consts();
 #if !defined(HFB200_EMU)
         CUDA_CHECK(cudaMemcpyToSymbol(g_p2c, &g_p2c_host, sizeof(P2Consts)));
+        CUDA_CHECK(cudaMemcpyToSymbol(g_p2tc_b, g_p2tc_host.b, P2TC_B_BYTES));
 #endif
+    }
+    // n independent states (24 words each) permuted in place
+    void permute(uint32_t* states, uint32_t n) {
+        dev->launch<PermuteKernel, 128, P2Perm::kMinBlocks>((n + 127) / 128, 1, 128, P2Perm::kSmem, states, n);
     }
     // nodes: 2*rows digests (heap layout).  matrix element (r, c) at matrix[c*col_stride + r].
     void build(const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
-        const int T = 128;
-        dev->launch<HashRowsKernel, 128, 1>((rows + T - 1) / T, 1, T, 0, matrix, col_stride, rows, cols, nodes);
+        const int T = 128;  // = the M of the tensor-core GEMMs (P2Perm)
+        dev->launch<HashRowsKernel, 128, P2Perm::kMinBlocks>((rows + T - 1) / T, 1, T, P2Perm::kSmem, matrix, col_stride, rows, cols, nodes);
         uint32_t level = rows / 2;
 #ifndef HFB200_EMU
         // big levels: one thread per node (throughput); <= 4096 nodes: one warp per node (latency); <= 32: one block
         static const uint32_t warp_max = [] { const char* e = std::getenv("HFB200_FOLD_WARP_MAX"); const int v = e ? std::atoi(e) : 0; return v >= 64 ? (uint32_t)v : 4096u; }();
-        for (; level > warp_max; level >>= 1) dev->launch<HashFoldKernel, 128, 1>((level + T - 1) / T, 1, T, 0, nodes, level);
+        for (; level > warp_max; level >>= 1) dev->launch<HashFoldKernel, 128, P2Perm::kMinBlocks>((level + T - 1) / T, 1, T, P2Perm::kSmem, nodes, level);
         for (; level > 32; level >>= 1) dev->launch<HashFoldWarpKernel, 256, 1>((level * 32 + 255) / 256, 1, 256, 0, nodes, level);
         if (level >= 1) dev->launch<HashFoldWarpTailKernel, 1024, 1>(1, 1, 1024, 0, nodes, level);
 #else
-        for (; level >= 512; level >>= 1) dev->launch<HashFoldKernel, 128, 1>((level + T - 1) / T, 1, T, 0, nodes, level);
+        for (; level >= 512; level >>= 1) dev->launch<HashFoldKernel, 128, P2Perm::kMinBlocks>((level + T - 1) / T, 1, T, P2Perm::kSmem, nodes, level);
         if (level >= 1) dev->launch<HashFoldTailKernel, 256, 1>(1, 1, 256, 0, nodes, level);
 #endif
     }
