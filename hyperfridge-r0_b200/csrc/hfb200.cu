@@ -628,6 +628,21 @@ const char* hfb200_op_poseidon2(hfb200_ctx* ctx, uint32_t* states, size_t n) {
     d.sync();
     API_CATCH
 }
+#if P2_PHASE_PROBE && !defined(HFB200_EMU)
+// Phase probe builds only (tools/p2_phase_probe.py): out[0..n) = the cycle sums of g_p2_probe, out[n] = permutations
+// sampled, n = 4 + 3 P2TC_BLOCKS phases written to *n_phases.  Clears the counters.
+const char* hfb200_p2_probe_read(hfb200_ctx* ctx, unsigned long long* out, uint32_t* n_phases) {
+    API_TRY
+    if (!ctx || !out || !n_phases) throw Err("p2_probe_read: NULL argument");
+    ctx->p.bind();
+    ctx->p.dev.sync();
+    CUDA_CHECK(cudaMemcpyFromSymbol(out, hf::g_p2_probe, sizeof(unsigned long long) * (hf::P2_PROBE_N + 1)));
+    static const unsigned long long zero[hf::P2_PROBE_N + 1] = {};
+    CUDA_CHECK(cudaMemcpyToSymbol(hf::g_p2_probe, zero, sizeof zero));
+    *n_phases = hf::P2_PROBE_N;
+    API_CATCH
+}
+#endif
 const char* hfb200_op_fri_fold(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t n, const uint32_t* mix4) {
     API_TRY
     if (!ctx || !out || !in || !mix4) throw Err("op_fri_fold: NULL argument");

@@ -13,7 +13,7 @@ namespace hf {
 struct P2Consts {
     uint32_t rc_first[96], rc_partial[21], rc_last[96], diag[24];  // Montgomery form
     uint32_t diag_std[24], diag_shoup[24];  // canonical d_i and floor(d_i * 2^32 / p): constant multiplier in Shoup form
-    int32_t tri_c[21];  // partial rounds in tensor form: c_k = (M_I^k)[0][0] * 2^32 mod p, balanced in (-p/2, p/2], k = 1..20
+    int32_t tri_c[21];  // partial rounds in tensor form: c_k = (M_I^k)[0][0] * 2^32 mod p, balanced in (-p/2, p/2], k = 1..20 (only k < P2TC_BS are read)
 };
 
 // ---- the 21 partial rounds as two linear maps ----------------------------------------------------------------------------
@@ -28,14 +28,35 @@ struct P2Consts {
 // Plane j accumulates Q_j = sum bytes * bytes <= 180 * 255^2 < 2^24 in int32; V = sum_j 2^(8j) Q_j < 2^49 < p 2^32, so one
 // Montgomery REDC of V is the Montgomery residue of the output.  The state words need no conversion: a little-endian u32 is
 // already its 4 byte inputs.
-static constexpr uint32_t P2TC_K1 = 96, P2TC_N1 = 80;    // GEMM 1: bytes of v -> 4 planes of a_1..a_20 . v
-static constexpr uint32_t P2TC_K2 = 192, P2TC_N2 = 96;   // GEMM 2: bytes of [v | delta_0..20 | 0 0 0] -> 4 planes of v_21
-static constexpr uint32_t P2TC_B1_BYTES = P2TC_K1 * P2TC_N1, P2TC_B_BYTES = P2TC_B1_BYTES + P2TC_K2 * P2TC_N2;
-// Operand layout of both GEMMs (tcgen05 shared-memory descriptor, K-major, no swizzle): core matrices of 8 rows x 16 bytes,
+//
+// Blocked chain: the 21 rounds are cut into P2TC_BLOCKS blocks of P2TC_BS rounds.  Once the deltas of block b - 1 are known,
+// one small GEMM (K = the bytes of that block's deltas) adds sum_{j in block b-1} c_{r-j} delta_j to the planes of every
+// later round r, accumulating into the TMEM columns where GEMM 1 left a_r . v.  SIMT then sums only the terms inside a block
+// (3 x 21 = 63 instead of 210 for 3 blocks of 7).  A plane accumulates at most 96 + 4 * 21 bytes * bytes, so Q_j < 2^24 holds.
+// 1 block is the plain two-GEMM form (-DP2TC_BLOCKS=1 through tools/build_variant.sh, for A/B).
+#ifndef P2TC_BLOCKS
+#define P2TC_BLOCKS 3
+#endif
+static_assert(P2TC_BLOCKS >= 1 && P2TC_BLOCKS <= 4, "P2TC_BLOCKS: 1..4");
+static constexpr uint32_t P2TC_NB = P2TC_BLOCKS;
+static constexpr uint32_t P2TC_BS = (21 + P2TC_NB - 1) / P2TC_NB;  // rounds per block (the last may be shorter)
+static constexpr uint32_t P2TC_BW = (P2TC_BS + 7) / 8 * 8;          // A words per block: each block starts on a 32-byte K step
+static constexpr uint32_t P2TC_AW = 24 + P2TC_NB * P2TC_BW;         // A row: [v | delta block 0 | ... | block NB-1], zero-padded
+static constexpr uint32_t P2TC_K1 = 96, P2TC_N1 = 80;    // GEMM 1: bytes of v -> 4 planes of a_1..a_20 . v (round r: columns 4(r-1)..)
+static constexpr uint32_t P2TC_K2 = 4 * P2TC_AW, P2TC_N2 = 96;  // GEMM 2: bytes of the whole A row -> 4 planes of v_21
+static constexpr uint32_t P2TC_B1_BYTES = P2TC_K1 * P2TC_N1;
+// block GEMM b = 1..NB-1 (A = delta block b-1, K = 4 BW) writes TMEM columns [c0, 80): c0 is the 16-aligned column at or below
+// the first plane of round b BS, and the B rows in front of that plane are zero.
+HD constexpr uint32_t p2tc_blk_c0(uint32_t b) { return (4 * (b * P2TC_BS - 1)) & ~15u; }
+HD constexpr uint32_t p2tc_blk_n(uint32_t b) { return P2TC_N1 - p2tc_blk_c0(b); }
+HD constexpr uint32_t p2tc_blk_boff(uint32_t b) { return b <= 1 ? P2TC_B1_BYTES : p2tc_blk_boff(b - 1) + 4 * P2TC_BW * p2tc_blk_n(b - 1); }
+static constexpr uint32_t P2TC_B2_OFF = p2tc_blk_boff(P2TC_NB);  // GEMM 2's B rows follow the block GEMMs'
+static constexpr uint32_t P2TC_B_BYTES = P2TC_B2_OFF + P2TC_K2 * P2TC_N2;
+// Operand layout of all GEMMs (tcgen05 shared-memory descriptor, K-major, no swizzle): core matrices of 8 rows x 16 bytes,
 // 128 contiguous bytes each; the next 16 bytes along K are 128 bytes further (LBO), the next 8 rows 8 K bytes further (SBO).
 HD uint32_t p2tc_off(uint32_t row, uint32_t k, uint32_t K) { return (row >> 3) * (K * 8) + (k >> 4) * 128 + (row & 7) * 16 + (k & 15); }
 struct P2TcTables {
-    uint8_t b[P2TC_B_BYTES];  // B operands (rows = the N output planes) in the layout above: GEMM 1, then GEMM 2
+    uint8_t b[P2TC_B_BYTES];  // B operands (rows = the N output planes) in the layout above: GEMM 1, the block GEMMs, GEMM 2
 };
 
 static inline uint32_t p2_mod_mul(uint32_t a, uint32_t b) { return (uint32_t)((uint64_t)a * b % P); }
@@ -64,12 +85,18 @@ static inline P2TcTables p2_make_tc_tables() {
     P2TcTables t;
     std::memset(t.b, 0, sizeof t.b);
     const auto pw = p2_m_int_powers();
-    uint32_t m[45];
+    uint32_t m[P2TC_AW];
     for (uint32_t r = 1; r <= 20; r++) p2tc_put_output(t.b, P2TC_K1, r - 1, &pw[r][0], 24);  // row 0 of M_I^r
+    for (uint32_t b = 1; b < P2TC_NB; b++)
+        for (uint32_t r = b * P2TC_BS; r <= 20; r++) {  // c_{r-j} for the deltas j of block b-1
+            for (uint32_t i = 0; i < P2TC_BS; i++) m[i] = pw[r - ((b - 1) * P2TC_BS + i)][0];
+            p2tc_put_output(t.b + p2tc_blk_boff(b), 4 * P2TC_BW, (4 * (r - 1) - p2tc_blk_c0(b)) / 4, m, P2TC_BS);
+        }
     for (uint32_t o = 0; o < 24; o++) {
+        std::memset(m, 0, sizeof m);
         for (int i = 0; i < 24; i++) m[i] = pw[21][o * 24 + i];
-        for (int j = 0; j < 21; j++) m[24 + j] = pw[21 - j][o * 24];  // (M_I^(21-j) e0)[o]
-        p2tc_put_output(t.b + P2TC_B1_BYTES, P2TC_K2, o, m, 45);
+        for (uint32_t j = 0; j < 21; j++) m[24 + j / P2TC_BS * P2TC_BW + j % P2TC_BS] = pw[21 - j][o * 24];  // (M_I^(21-j) e0)[o]
+        p2tc_put_output(t.b + P2TC_B2_OFF, P2TC_K2, o, m, P2TC_AW);
     }
     return t;
 }
@@ -269,16 +296,30 @@ HD void p2_mix(uint32_t* s) {
 
 // ---- permutation with the partial rounds on the tensor cores (see "the 21 partial rounds as two linear maps") ---------------
 // Device: one CTA of 128 threads = 128 states = the 128 TMEM lanes of a tcgen05.mma (M = 128, kind::i8, cta_group::1).
-// Thread t writes its A row (the 48 words [v | delta | 0]) into shared memory, one thread issues the MMAs, tcgen05.commit
-// arrives on an mbarrier, and thread t reads its own row of the int32 planes back with tcgen05.ld.  Every thread of the CTA
-// takes part in every permutation (the barriers are CTA-wide), so kernels run idle states on zeros instead of returning.
-// Emulator (and the nvcc host pass): the same row, tables, recombination and REDC, with plain loops in place of the MMA.
+// Thread t writes its A row (the P2TC_AW words [v | delta blocks]) into shared memory, one thread issues the MMAs,
+// tcgen05.commit arrives on an mbarrier, and thread t reads its own row of the int32 planes back with tcgen05.ld.  Every
+// thread of the CTA takes part in every permutation (the barriers are CTA-wide), so kernels run idle states on zeros instead
+// of returning.  Emulator (and the nvcc host pass): the same row, tables, recombination and REDC, with plain loops in place
+// of the MMA accumulating into a per-state column array in place of TMEM.
 #ifndef P2_TC
 #define P2_TC 1
 #endif
 static constexpr uint32_t P2TC_A_BYTES = 128 * P2TC_K2;
 static constexpr size_t P2TC_SMEM = P2TC_A_BYTES + P2TC_B_BYTES + 32;  // A tile, B operands, 2 mbarriers + the TMEM address
 static constexpr uint32_t P2TC_TMEM_COLS = 128;                        // >= N1, N2; 4 CTAs fill an SM's 512 columns
+
+// Phase probe (-DP2_PHASE_PROBE=1, device only): lane 0 of warp 1 of every CTA (a warp that does not issue the MMAs) adds the
+// clock64 cycles of each phase of p2_mix_tc to g_p2_probe[phase]; g_p2_probe[P2_PROBE_N] counts the permutations.  Phases:
+// 0 first full rounds; per block b: 1 + 3b A row stores + MMA round trip (barrier, issue, commit, mbarrier wait),
+// 2 + 3b tcgen05.ld + recombination of the block's rounds, 3 + 3b the block's S-box chain; then 1 + 3 NB GEMM 2 round trip,
+// 2 + 3 NB its loads + recombination, 3 + 3 NB last full rounds.  hfb200_p2_probe_read returns and clears the counters.
+#ifndef P2_PHASE_PROBE
+#define P2_PHASE_PROBE 0
+#endif
+static constexpr uint32_t P2_PROBE_N = 4 + 3 * P2TC_NB;
+#if P2_PHASE_PROBE && !defined(HFB200_EMU)
+__device__ unsigned long long g_p2_probe[P2_PROBE_N + 1];
+#endif
 
 struct P2Tc {
 #ifdef __CUDA_ARCH__
@@ -288,10 +329,26 @@ struct P2Tc {
     uint32_t* tslot; // TMEM base address written by tcgen05.alloc
     uint32_t tmem, phase, row;
     bool b_wait;     // thread 0: B operands not yet waited for
+#if P2_PHASE_PROBE
+    long long t;     // clock64 at the last phase boundary
+#endif
 #else
-    uint32_t w[48];  // this state's A row
+    uint32_t w[P2TC_AW];             // this state's A row
+    uint32_t acc[P2TC_TMEM_COLS];    // this state's TMEM lane
 #endif
 };
+HD void p2tc_mark(P2Tc& tc, uint32_t ph) {
+#if defined(__CUDA_ARCH__) && P2_PHASE_PROBE
+    if (tc.row == 32) {
+        const long long t = clock64();
+        if (ph < P2_PROBE_N) atomicAdd(&g_p2_probe[ph], (unsigned long long)(t - tc.t));
+        else atomicAdd(&g_p2_probe[P2_PROBE_N], 1ull);
+        tc.t = t;
+    }
+#else
+    (void)tc; (void)ph;
+#endif
+}
 
 #ifdef __CUDA_ARCH__
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -354,23 +411,24 @@ HD void p2tc_put(P2Tc& tc, uint32_t w0, const uint32_t* v, uint32_t n) {
     for (uint32_t i = 0; i < 4 * n; i++) tc.w[w0 + i] = v[i];
 #endif
 }
-// GEMM g (1 or 2) over the rows of all threads of the CTA; the planes land in TMEM columns [0, N_g)
-HD void p2tc_gemm(P2Tc& tc, int g) {
+// D[:, c0 .. c0 + N) (+)= A[:, 4 aw0 .. 4 aw0 + K) x B^T over the rows of all threads of the CTA, B the K x N operand at byte
+// boff of the tables; accumulate into the TMEM columns when acc.  aw0 is a multiple of 8 (a 32-byte K step), c0 of 16.
+// first: the CTA's first GEMM of the permutation, the only one whose issue may still have to wait for the B operands.
+HD void p2tc_mma(P2Tc& tc, uint32_t aw0, uint32_t K, uint32_t boff, uint32_t c0, uint32_t N, bool acc, bool first) {
 #ifdef __CUDA_ARCH__
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy row stores -> visible to the MMA
     tc_fence_before();                                             // earlier tcgen05.ld of these columns are complete
     __syncthreads();
     if (tc.row == 0) {
         tc_fence_after();
-        if (tc.b_wait) { mbar_wait(&tc.bar[0], 0); tc.b_wait = false; }
-        const uint32_t K = g == 1 ? P2TC_K1 : P2TC_K2, N = g == 1 ? P2TC_N1 : P2TC_N2;
+        if (first && tc.b_wait) { mbar_wait(&tc.bar[0], 0); tc.b_wait = false; }
         // kind::i8 instruction descriptor: D s32 (bits 4-5 = 2), A and B unsigned 8-bit, both K-major, N >> 3 at 17, M >> 4 at 24
         const uint32_t idesc = (2u << 4) | ((N >> 3) << 17) | ((128u >> 4) << 24);
-        const uint32_t a0 = smem_u32(tc.a), b0 = smem_u32(tc.b) + (g == 1 ? 0u : P2TC_B1_BYTES);
+        const uint32_t a0 = smem_u32(tc.a) + aw0 / 8 * 256, b0 = smem_u32(tc.b) + boff;
         for (uint32_t kk = 0; kk < K / 32; kk++) {  // K = 32 bytes per MMA: two core matrices along K
             const uint64_t ad = p2tc_desc(a0 + kk * 256, P2TC_K2), bd = p2tc_desc(b0 + kk * 256, K);
             asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                         ::"r"(tc.tmem), "l"(ad), "l"(bd), "r"(idesc), "r"(kk) : "memory");
+                         ::"r"(tc.tmem + c0), "l"(ad), "l"(bd), "r"(idesc), "r"((uint32_t)acc | kk) : "memory");
         }
         asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(&tc.bar[1])) : "memory");
     }
@@ -378,28 +436,36 @@ HD void p2tc_gemm(P2Tc& tc, int g) {
     tc.phase ^= 1;
     tc_fence_after();
 #else
-    (void)tc; (void)g;
+    (void)first;
+    const uint8_t* a = reinterpret_cast<const uint8_t*>(tc.w) + 4 * aw0;  // little-endian: word i = bytes 4i..4i+3
+    const uint8_t* b = g_p2tc_host.b + boff;
+    for (uint32_t n = 0; n < N; n++) {
+        uint32_t s = acc ? tc.acc[c0 + n] : 0u;
+        for (uint32_t k = 0; k < K; k++) s += (uint32_t)a[k] * b[p2tc_off(n, k, K)];
+        tc.acc[c0 + n] = s;
+    }
 #endif
 }
-// 16 int32 columns [c0, c0 + 16) of this state's row of the last GEMM's result
-HD void p2tc_cols16(P2Tc& tc, int g, uint32_t c0, uint32_t* q) {
 #ifdef __CUDA_ARCH__
-    (void)g;
+// issue the load of 16 int32 columns [c0, c0 + 16) of this thread's TMEM lane; the values are valid after p2tc_ld_wait
+__device__ __forceinline__ void p2tc_ld16(const P2Tc& tc, uint32_t c0, uint32_t* q) {
     const uint32_t addr = tc.tmem + ((tc.row & ~31u) << 16) + c0;  // a warp reads its own 32 TMEM lanes
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-                 "tcgen05.wait::ld.sync.aligned;\n"
                  : "=r"(q[0]), "=r"(q[1]), "=r"(q[2]), "=r"(q[3]), "=r"(q[4]), "=r"(q[5]), "=r"(q[6]), "=r"(q[7]),
                    "=r"(q[8]), "=r"(q[9]), "=r"(q[10]), "=r"(q[11]), "=r"(q[12]), "=r"(q[13]), "=r"(q[14]), "=r"(q[15])
                  : "r"(addr) : "memory");
+}
+#endif
+// 16 n int32 columns [c0, c0 + 16 n) of this state's TMEM lane: all loads issued, then one wait
+HD void p2tc_cols(P2Tc& tc, uint32_t c0, uint32_t n, uint32_t* q) {
+#ifdef __CUDA_ARCH__
+#pragma unroll
+    for (uint32_t i = 0; i < n; i++) p2tc_ld16(tc, c0 + 16 * i, q + 16 * i);
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (uint32_t i = 0; i < 16 * n; i++) asm volatile("" : "+r"(q[i]));  // no read of q may move above the wait
 #else
-    const uint8_t* a = reinterpret_cast<const uint8_t*>(tc.w);  // little-endian: word i = bytes 4i..4i+3
-    const uint32_t K = g == 1 ? P2TC_K1 : P2TC_K2;
-    const uint8_t* b = g_p2tc_host.b + (g == 1 ? 0u : P2TC_B1_BYTES);
-    for (uint32_t n = 0; n < 16; n++) {
-        uint32_t acc = 0;
-        for (uint32_t k = 0; k < K; k++) acc += (uint32_t)a[k] * b[p2tc_off(c0 + n, k, K)];
-        q[n] = acc;
-    }
+    for (uint32_t i = 0; i < 16 * n; i++) q[i] = tc.acc[c0 + i];
 #endif
 }
 // REDC(sum_j 2^(8j) q_j) for planes q_j < 2^24: V < 2^49, split into its low and high words without 64-bit arithmetic.
@@ -432,53 +498,70 @@ HD uint32_t p2tc_dot4(const int32_t* c, const int32_t* d, int n) {
     return umin32(r, r + P);
 }
 
+// out[i] = REDC of the 4 planes in TMEM columns c_lo + 4 i, for c_lo + 4 i < c_hi: x16 loads, one wait per 3 of them
+HD void p2tc_read(P2Tc& tc, uint32_t c_lo, uint32_t c_hi, uint32_t* out) {
+#pragma unroll
+    for (uint32_t g = c_lo & ~15u; g < c_hi; g += 48) {
+        uint32_t q[48];
+        p2tc_cols(tc, g, umin32((c_hi - g + 15) / 16, 3u), q);
+#pragma unroll
+        for (uint32_t c = g < c_lo ? c_lo : g; c < c_hi && c < g + 48; c += 4) out[(c - c_lo) / 4] = p2tc_reduce(q + (c - g));
+    }
+}
+
 HD void p2_mix_tc(uint32_t* s, P2Tc& tc) {
     const P2Consts& k = p2c();
+    p2tc_mark(tc, P2_PROBE_N);
     p2_m_ext(s);
     p2_full_rounds(s, k.rc_first);
-    // GEMM 1: L_r = a_r . v, r = 1..20
+    p2tc_mark(tc, 0);
+    // GEMM 1: a_r . v for r = 1..20 in columns 4(r-1) .. 4(r-1) + 3
     p2tc_put(tc, 0, s, 6);
-    p2tc_gemm(tc, 1);
-    uint32_t L[21];
-    L[0] = s[0];
+    p2tc_mma(tc, 0, P2TC_K1, 0, 0, P2TC_N1, false, true);
+    p2tc_mark(tc, 1);
+    uint32_t w[P2TC_BW];  // the canonical deltas of the current block and its zero padding: its words of the A row
 #pragma unroll
-    for (uint32_t c = 0; c < P2TC_N1; c += 16) {
-        uint32_t q[16];
-        p2tc_cols16(tc, 1, c, q);
-#pragma unroll
-        for (uint32_t o = 0; o < 4; o++) L[1 + c / 4 + o] = p2tc_reduce(q + 4 * o);
-    }
-    // the S-box chain: v_r[0] = L_r + sum_{j<r} c_{r-j} delta_j, delta_r kept balanced in (-p/2, p/2]
-    int32_t dlt[21];
-#pragma unroll
-    for (int r = 0; r < 21; r++) {
-        uint32_t y = L[r];
-#pragma unroll
-        for (int j0 = 0; j0 < r; j0 += 4) {
-            const int n = r - j0 < 4 ? r - j0 : 4;
-            int32_t cc[4], dd[4];
-#pragma unroll
-            for (int j = 0; j < 4; j++) if (j < n) { cc[j] = k.tri_c[r - j0 - j]; dd[j] = dlt[j0 + j]; }
-            y = fadd(y, p2tc_dot4(cc, dd, n));
+    for (uint32_t b = 0; b < P2TC_NB; b++) {
+        const uint32_t r0 = b * P2TC_BS, r1 = umin32(r0 + P2TC_BS, 21u), rl = r0 ? r0 : 1;
+        if (b > 0) {  // block GEMM b: the deltas of block b - 1 into the columns of rounds >= r0
+            p2tc_put(tc, 24 + (b - 1) * P2TC_BW, w, P2TC_BW / 4);
+            p2tc_mma(tc, 24 + (b - 1) * P2TC_BW, 4 * P2TC_BW, p2tc_blk_boff(b), p2tc_blk_c0(b), p2tc_blk_n(b), true, false);
+            p2tc_mark(tc, 1 + 3 * b);
         }
-        const uint32_t d = fsub(sbox7_rc(y, k.rc_partial[r]), y);
-        dlt[r] = d > (P - 1) / 2 ? (int32_t)(d - P) : (int32_t)d;
+        // L_r = a_r . v + sum_{j < r0} c_{r-j} delta_j for the rounds of this block
+        uint32_t L[P2TC_BS];
+        if (b == 0) L[0] = s[0];
+        p2tc_read(tc, 4 * (rl - 1), 4 * (r1 - 1), L + (rl - r0));
+        p2tc_mark(tc, 2 + 3 * b);
+        // the S-box chain inside the block: v_r[0] = L_r + sum_{r0 <= j < r} c_{r-j} delta_j, delta_r kept balanced in (-p/2, p/2]
+        int32_t dlt[P2TC_BS];
+#pragma unroll
+        for (uint32_t r = r0; r < r1; r++) {
+            uint32_t y = L[r - r0];
+#pragma unroll
+            for (uint32_t j0 = r0; j0 < r; j0 += 4) {
+                const uint32_t n = umin32(r - j0, 4u);
+                int32_t cc[4], dd[4];
+#pragma unroll
+                for (uint32_t j = 0; j < 4; j++) if (j < n) { cc[j] = k.tri_c[r - j0 - j]; dd[j] = dlt[j0 - r0 + j]; }
+                y = fadd(y, p2tc_dot4(cc, dd, (int)n));
+            }
+            const uint32_t d = fsub(sbox7_rc(y, k.rc_partial[r]), y);
+            dlt[r - r0] = d > (P - 1) / 2 ? (int32_t)(d - P) : (int32_t)d;
+            w[r - r0] = d;
+        }
+#pragma unroll
+        for (uint32_t t = r1 - r0; t < P2TC_BW; t++) w[t] = 0;
+        p2tc_mark(tc, 3 + 3 * b);
     }
-    // GEMM 2: v_21 = M_I^21 v + sum_j delta_j M_I^(21-j) e0 (the v bytes are still in the A row)
-    uint32_t w[24];
-#pragma unroll
-    for (int j = 0; j < 21; j++) { const uint32_t u = (uint32_t)dlt[j]; w[j] = umin32(u, u + P); }
-    w[21] = w[22] = w[23] = 0;
-    p2tc_put(tc, 24, w, 6);
-    p2tc_gemm(tc, 2);
-#pragma unroll
-    for (uint32_t c = 0; c < P2TC_N2; c += 16) {
-        uint32_t q[16];
-        p2tc_cols16(tc, 2, c, q);
-#pragma unroll
-        for (uint32_t o = 0; o < 4; o++) s[c / 4 + o] = p2tc_reduce(q + 4 * o);
-    }
+    // GEMM 2: v_21 = M_I^21 v + sum_j delta_j M_I^(21-j) e0 (the v bytes and the earlier blocks are still in the A row)
+    p2tc_put(tc, 24 + (P2TC_NB - 1) * P2TC_BW, w, P2TC_BW / 4);
+    p2tc_mma(tc, 0, P2TC_K2, P2TC_B2_OFF, 0, P2TC_N2, false, false);
+    p2tc_mark(tc, 1 + 3 * P2TC_NB);
+    p2tc_read(tc, 0, P2TC_N2, s);
+    p2tc_mark(tc, 2 + 3 * P2TC_NB);
     p2_full_rounds(s, k.rc_last);
+    p2tc_mark(tc, 3 + 3 * P2TC_NB);
 }
 
 // The permutation the Merkle / permutation kernels run for one state per thread.  kAll: every thread of the block must
