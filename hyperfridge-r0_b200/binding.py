@@ -27,6 +27,7 @@ EXPORTS = [
     "hfb200_set_transcript", "hfb200_graph_launches", "hfb200_digest_bytes", "hfb200_digest_pair", "hfb200_claim_encode", "hfb200_claim_decode", "hfb200_claim_next_state", "hfb200_verify_claims",
     "hfb200_segment_begin_dev", "hfb200_segment_finish_dev", "hfb200_segment_accum_scan", "hfb200_segment_accum_blind", "hfb200_device_count",
     "hfb200_pool_set_accum",
+    "hfb200_segment_witness_dev", "hfb200_segment_data_blind", "hfb200_segment_scratch", "hfb200_pool_set_witgen",
 ]
 
 BLIND_OS_ENTROPY, BLIND_DETERMINISTIC = 0, 1
@@ -122,6 +123,30 @@ class SegmentDev(C.Structure):
 ACCUM_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.POINTER(SegmentDev), C.c_size_t)
 
 
+class WitnessDev(C.Structure):
+    """hfb200_witness_dev: the writable DATA columns between segment_witness_dev and the begin that commits them.  `data` is a
+    device address (a host address in the emulator); `stream` is the context's cudaStream_t."""
+    _fields_ = [("po2", C.c_uint32), ("zk_rows", C.c_uint32), ("w_code", C.c_uint32), ("w_data", C.c_uint32), ("device", C.c_int),
+                ("stream", C.c_void_p), ("data", C.c_void_p)]
+
+    @property
+    def rows(self):
+        return 1 << self.po2
+
+    def host_view(self):
+        """numpy view [w_data, rows] of the data columns -- only where device addresses ARE host addresses (the host emulator)."""
+        return np.ctypeslib.as_array(C.cast(self.data, C.POINTER(C.c_uint32)), shape=(self.w_data * self.rows,)).reshape(self.w_data, self.rows)
+
+
+def scratch_view(addr, nbytes):
+    """numpy uint8 view of a segment scratch buffer -- only in the host emulator, where it is host memory."""
+    return np.ctypeslib.as_array(C.cast(addr, C.POINTER(C.c_uint8)), shape=(nbytes,))
+
+
+# int (*hfb200_witgen_fn)(void* user, hfb200_ctx* ctx, const hfb200_witness_dev* w, size_t job)
+WITGEN_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.POINTER(WitnessDev), C.c_size_t)
+
+
 class PoolStats(C.Structure):
     _fields_ = [("contexts", C.c_size_t), ("contexts_retired", C.c_size_t), ("faults", C.c_uint64), ("retries", C.c_uint64),
                 ("contexts_recreated", C.c_uint64)]
@@ -196,6 +221,10 @@ def load_library(path=None):
         "hfb200_segment_accum_blind": (err, [vp]),
         "hfb200_device_count": (err, [C.POINTER(C.c_int)]),
         "hfb200_pool_set_accum": (err, [vp, vp, vp]),
+        "hfb200_segment_witness_dev": (err, [vp, u32, u64, C.POINTER(WitnessDev)]),
+        "hfb200_segment_data_blind": (err, [vp]),
+        "hfb200_segment_scratch": (err, [vp, sz, C.POINTER(vp)]),
+        "hfb200_pool_set_witgen": (err, [vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -337,6 +366,24 @@ class Context:
 
     def segment_accum_blind(self):
         self._check(self.lib.hfb200_segment_accum_blind(self._h))
+
+    def segment_witness_dev(self, po2, blind_seed):
+        """hfb200_segment_witness_dev: lays the context out for po2, derives the segment's blinding key and returns the WitnessDev
+        whose data columns the caller writes; segment_begin / segment_begin_dev with data=None then commit them as they stand."""
+        w = WitnessDev()
+        self._check(self.lib.hfb200_segment_witness_dev(self._h, po2, blind_seed, C.byref(w)))
+        self._po2 = po2
+        return w
+
+    def segment_data_blind(self):
+        """Writes the blinding rows of every data column from the segment's key (between segment_witness_dev and the begin)."""
+        self._check(self.lib.hfb200_segment_data_blind(self._h))
+
+    def segment_scratch(self, nbytes):
+        """Address of >= nbytes of device memory owned by the context (host memory in the emulator: see scratch_view)."""
+        p = C.c_void_p()
+        self._check(self.lib.hfb200_segment_scratch(self._h, nbytes, C.byref(p)))
+        return p.value
 
     def segment_finish_dev(self):
         """Completes the segment from the accum columns as they stand in device memory."""
@@ -503,6 +550,21 @@ class SegmentHandle:
 
     def accum_blind(self):
         _raise_err(self.lib, self.lib.hfb200_segment_accum_blind(self._h))
+
+
+class WitnessHandle:
+    """What a Python witgen callback of Pool.set_witgen may call on the context it is given."""
+
+    def __init__(self, lib, ctx):
+        self.lib, self._h = lib, ctx
+
+    def scratch(self, nbytes):
+        p = C.c_void_p()
+        _raise_err(self.lib, self.lib.hfb200_segment_scratch(self._h, nbytes, C.byref(p)))
+        return p.value
+
+    def data_blind(self):
+        _raise_err(self.lib, self.lib.hfb200_segment_data_blind(self._h))
 
 
 def verify_segment(seal, code_root, circuit=(16, 192, 48), ir=None, lib=None):
@@ -697,6 +759,33 @@ class Pool:
         self._accum_cb = ACCUM_FN(trampoline)  # kept alive as long as the pool may call it
         self._raise(self.lib.hfb200_pool_set_accum(self._h, C.cast(self._accum_cb, C.c_void_p).value, None))
 
+    def set_witgen(self, fn, user=None):
+        """The caller's witness generator for every job whose data is None (hfb200_pool_set_witgen); None removes it.
+        `fn` is either the address (int) of a C function `int fn(void* user, hfb200_ctx*, const hfb200_witness_dev*, size_t job)`
+        -- `user` is then passed through as a pointer (int or None) -- or a Python callable fn(ctx, w, job) with ctx a
+        WitnessHandle (scratch / data_blind) and w the WitnessDev.  A Python callback runs on the worker threads, one at a time
+        under the GIL; an exception fails that job only and its text appears in the job's error."""
+        self._witgen_errors = {}
+        if fn is None:
+            self._witgen_cb = None
+            self._raise(self.lib.hfb200_pool_set_witgen(self._h, None, None))
+            return
+        if isinstance(fn, int):
+            self._witgen_cb = None
+            self._raise(self.lib.hfb200_pool_set_witgen(self._h, fn, user))
+            return
+        lib, errors = self.lib, self._witgen_errors
+
+        def trampoline(_user, ctx, w, job):
+            try:
+                fn(WitnessHandle(lib, ctx), w.contents, int(job))
+                return 0
+            except BaseException as e:  # noqa: B036 -- nothing may unwind into the C worker thread
+                errors[int(job)] = "%s: %s" % (type(e).__name__, e)
+                return 1
+        self._witgen_cb = WITGEN_FN(trampoline)  # kept alive as long as the pool may call it
+        self._raise(self.lib.hfb200_pool_set_witgen(self._h, C.cast(self._witgen_cb, C.c_void_p).value, None))
+
     def close(self):
         if self._h:
             self.lib.hfb200_pool_destroy(self._h)
@@ -723,7 +812,8 @@ class Pool:
         self._raise(self.lib.hfb200_pool_load_control(self._h, po2, _ptr(code)))
 
     def prove(self, jobs, seal_cap, return_errors=False):
-        """jobs: list of (po2, globals, code, data, blind_seed) with numpy u32 arrays (code may be None after load_control).
+        """jobs: list of (po2, globals, code, data, blind_seed) with numpy u32 arrays (code may be None after load_control, data
+        None with a witgen callback).
         Returns (seals, devices, ms); raises on the first failed job unless return_errors=True, in which case the result is
         (seals, devices, ms, errors) with errors[i] = None or the job's message (failed jobs have an empty seal; the others are
         proved regardless, like the reference's batch tooling sets failed inputs aside)."""
@@ -732,24 +822,31 @@ class Pool:
         keep = []
         seals = [np.empty(seal_cap, np.uint32) for _ in range(n)]
         for i, (po2, g, code, data, seed) in enumerate(jobs):
-            g, data = _u32(g), _u32(data)
+            g = _u32(g)
             code = _u32(code) if code is not None else None
+            data = _u32(data) if data is not None else None
             rows = 1 << po2
-            if g.size != N_GLOBAL or data.size != self.circuit[1] * rows or (code is not None and code.size != self.circuit[0] * rows):
+            if g.size != N_GLOBAL or (data is not None and data.size != self.circuit[1] * rows) or (code is not None and code.size != self.circuit[0] * rows):
                 raise Hfb200Error("pool.prove: job %d: trace shape does not match (circuit, po2)" % i)
             keep.append((g, code, data))
             arr[i].po2, arr[i].blind_seed = po2, seed
-            arr[i].globals, arr[i].code, arr[i].data = g.ctypes.data, (code.ctypes.data if code is not None else None), data.ctypes.data
+            arr[i].globals, arr[i].code = g.ctypes.data, (code.ctypes.data if code is not None else None)
+            arr[i].data = data.ctypes.data if data is not None else None
             arr[i].seal_out, arr[i].seal_cap = seals[i].ctypes.data, seal_cap
         accum_errors = getattr(self, "_accum_errors", {})
         accum_errors.clear()
+        witgen_errors = getattr(self, "_witgen_errors", {})
+        witgen_errors.clear()
         e = self.lib.hfb200_pool_prove(self._h, arr, n)
         errs = [None] * n
         for i in range(n):
             if arr[i].error:
                 errs[i] = C.cast(arr[i].error, C.c_char_p).value.decode(errors="replace")
                 self.lib.hfb200_free_error(arr[i].error)
-                if i in accum_errors:  # the Python accum callback's own exception
+                # a Python callback's own exception
+                if i in witgen_errors and errs[i].startswith("witgen callback returned"):
+                    errs[i] += ": " + witgen_errors[i]
+                elif i in accum_errors:
                     errs[i] += ": " + accum_errors[i]
         self.last_attempts = [arr[i].attempts for i in range(n)]
         out = ([seals[i][:arr[i].seal_words] if errs[i] is None else seals[i][:0] for i in range(n)], [arr[i].device for i in range(n)],
@@ -758,7 +855,7 @@ class Pool:
             if e:
                 self.lib.hfb200_free_error(e)
             return out + (errs,)
-        if e and accum_errors:
+        if e and (accum_errors or witgen_errors):
             self.lib.hfb200_free_error(e)  # the library's message lacks the callback's text: report the job's own
             i = next(k for k in range(n) if errs[k] is not None)
             raise Hfb200Error("job %d: %s" % (i, errs[i]))

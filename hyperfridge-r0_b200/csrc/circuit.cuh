@@ -225,15 +225,17 @@ struct AccumScanKernel {
         }
     }
 };
-// hfb200_segment_accum_blind: the last zk rows of every accum column, exactly the values AccumKernel mode 1 writes there.
-struct AccumBlindKernel {
+// The last zk rows of every column of one group from the segment's key, one thread per element, consecutive threads on
+// consecutive rows of a column (coalesced stores).  GROUP_ACCUM: hfb200_segment_accum_blind, exactly the values AccumKernel
+// mode 1 writes there; GROUP_DATA: hfb200_segment_data_blind, exactly the values GenFreeKernel writes there.
+struct BlindRowsKernel {
     static constexpr bool kBarrier = false;
-    HD static void run(const KCtx& cx, uint32_t*, uint32_t* accum, uint32_t w_accum, uint32_t po2, uint32_t zk, BlindKey blind) {
+    HD static void run(const KCtx& cx, uint32_t*, uint32_t* cols, uint32_t w, uint32_t po2, uint32_t zk, uint32_t group, BlindKey blind) {
         const uint64_t n = 1ull << po2;
         const uint64_t t = (uint64_t)cx.bx * cx.nt + cx.tid;
-        if (t >= (uint64_t)w_accum * zk) return;
+        if (t >= (uint64_t)w * zk) return;
         const uint32_t c = (uint32_t)(t / zk), r = (uint32_t)(n - zk + t % zk);
-        accum[(uint64_t)c * n + r] = blind_value(blind, GROUP_ACCUM, c, r);
+        cols[(uint64_t)c * n + r] = blind_value(blind, group, c, r);
     }
 };
 

@@ -209,6 +209,32 @@ const char* hfb200_segment_accum_blind(hfb200_ctx* ctx) {
     ctx->p.accum_blind();
     API_CATCH
 }
+const char* hfb200_segment_witness_dev(hfb200_ctx* ctx, uint32_t po2, uint64_t blind_seed, hfb200_witness_dev* out) {
+    API_TRY
+    if (!ctx || !out) throw Err("hfb200_segment_witness_dev: NULL argument");
+    Prover& p = ctx->p;
+    p.witness_dev(po2, blind_seed);
+    hfb200_witness_dev w{};
+    w.po2 = p.po2; w.zk_rows = ZK_CYCLES;
+    w.w_code = p.cir.cd.w_code; w.w_data = p.cir.cd.w_data;
+    w.device = p.device_id;
+    w.stream = (void*)p.dev.stream;
+    w.data = p.tr[GROUP_DATA];
+    *out = w;
+    API_CATCH
+}
+const char* hfb200_segment_data_blind(hfb200_ctx* ctx) {
+    API_TRY
+    if (!ctx) throw Err("hfb200_segment_data_blind: NULL ctx");
+    ctx->p.data_blind();
+    API_CATCH
+}
+const char* hfb200_segment_scratch(hfb200_ctx* ctx, size_t bytes, void** out) {
+    API_TRY
+    if (!ctx || !out) throw Err("hfb200_segment_scratch: NULL argument");
+    *out = ctx->p.segment_scratch(bytes);
+    API_CATCH
+}
 const char* hfb200_device_count(int* out) {
     API_TRY
     if (!out) throw Err("hfb200_device_count: out is NULL");
@@ -304,6 +330,9 @@ struct hfb200_pool {
     // the caller's step_accum (hfb200_pool_set_accum): jobs then run begin_dev -> accum_fn -> finish_dev
     hfb200_accum_fn accum_fn = nullptr;
     void* accum_user = nullptr;
+    // the caller's witness generator (hfb200_pool_set_witgen): jobs with data == NULL then run witness_dev -> witgen_fn -> begin ...
+    hfb200_witgen_fn witgen_fn = nullptr;
+    void* witgen_user = nullptr;
     // test hook (hfb200_pool_inject_fault): worker `w` reports a CUDA error instead of proving its n-th job from now
     std::mutex inject_mu;
     std::map<size_t, std::pair<uint64_t, int>> inject;  // worker -> (jobs to let pass, kind)
@@ -345,23 +374,35 @@ static bool is_device_fault(const char* msg) { return msg && std::strncmp(msg, "
 // A nonzero return of the callback fails the job (never retried) and abandons the segment: the stream is drained so that the
 // context is usable for the next job.  If draining it reports a CUDA error, the callback met a device fault: the worker takes
 // the device-fault path (context re-created, job re-queued).
+static const char* abandon_after_callback(hfb200_ctx* ctx, const char* which, int rc) {
+#ifndef HFB200_EMU
+    cudaSetDevice(ctx->p.device_id);
+    const cudaError_t e = cudaStreamSynchronize(ctx->p.dev.stream);
+    ctx->p.quiesce();
+    if (e != cudaSuccess)
+        return dup_err(std::string("CUDA error ") + cudaGetErrorName(e) + " after the " + which + " callback: " + cudaGetErrorString(e));
+#else
+    ctx->p.quiesce();
+#endif
+    return dup_err(std::string(which) + " callback returned " + std::to_string(rc));
+}
 static const char* prove_job_with_accum(hfb200_pool* pool, hfb200_ctx* ctx, hfb200_segment_job& j, size_t idx) {
     hfb200_segment_dev seg;
     if (const char* e = hfb200_segment_begin_dev(ctx, j.po2, j.globals, j.code, j.data, j.blind_seed, 0, &seg)) return e;
     const int rc = pool->accum_fn(pool->accum_user, ctx, &seg, idx);
-    if (rc != 0) {
-#ifndef HFB200_EMU
-        cudaSetDevice(ctx->p.device_id);
-        const cudaError_t e = cudaStreamSynchronize(ctx->p.dev.stream);
-        ctx->p.quiesce();
-        if (e != cudaSuccess)
-            return dup_err(std::string("CUDA error ") + cudaGetErrorName(e) + " after the accum callback: " + cudaGetErrorString(e));
-#else
-        ctx->p.quiesce();
-#endif
-        return dup_err("accum callback returned " + std::to_string(rc));
-    }
+    if (rc != 0) return abandon_after_callback(ctx, "accum", rc);
     return hfb200_segment_finish_dev(ctx, j.seal_out, j.seal_cap, &j.seal_words);
+}
+// A job with data == NULL through the witness seam: witness_dev, the caller's witness generator on this worker thread, then the
+// accum stage (the accum callback, or the built-in step_accum of a built-in pool).  Failures as in prove_job_with_accum.
+static const char* prove_job_with_witgen(hfb200_pool* pool, hfb200_ctx* ctx, hfb200_segment_job& j, size_t idx) {
+    hfb200_witness_dev w;
+    if (const char* e = hfb200_segment_witness_dev(ctx, j.po2, j.blind_seed, &w)) return e;
+    const int rc = pool->witgen_fn(pool->witgen_user, ctx, &w, idx);
+    if (rc != 0) return abandon_after_callback(ctx, "witgen", rc);
+    if (pool->accum_fn) return prove_job_with_accum(pool, ctx, j, idx);
+    if (const char* e = hfb200_segment_begin(ctx, j.po2, j.globals, j.code, nullptr, j.blind_seed, nullptr, 0, nullptr)) return e;
+    return hfb200_segment_finish(ctx, nullptr, j.seal_out, j.seal_cap, &j.seal_words);
 }
 static const char* control_root_impl(hfb200_ctx* ctx, uint32_t po2, const uint32_t* code, uint32_t* root_out, uint64_t gen);
 extern "C" {
@@ -430,7 +471,11 @@ const char* hfb200_pool_prove(hfb200_pool* pool, hfb200_segment_job* jobs, size_
     // argument checks up front: a mis-shaped job must not reach cudaMemcpyAsync
     for (size_t i = 0; i < n_jobs; i++) {
         hfb200_segment_job& j = jobs[i];
-        if (!j.globals || !j.data || !j.seal_out) { j.error = dup_err("job has a NULL globals / data / seal_out pointer"); continue; }
+        if (!j.globals || (!j.data && !pool->witgen_fn) || !j.seal_out) { j.error = dup_err("job has a NULL globals / data / seal_out pointer"); continue; }
+        if (!j.data && pool->is_ir && !pool->accum_fn) {
+            j.error = dup_err("data-defined circuit: step_accum is the caller's (install an accum callback with hfb200_pool_set_accum)");
+            continue;
+        }
         if (j.po2 < MIN_PO2 || j.po2 > pool->max_po2) { j.error = dup_err("job po2 " + std::to_string(j.po2) + " outside [12, " + std::to_string(pool->max_po2) + "]"); continue; }
         const size_t need = hfb200_seal_words(pool->slots.empty() ? nullptr : pool->slots[0].ctx, j.po2);
         if (need && j.seal_cap < need) { j.seal_words = need; j.error = dup_err("seal buffer too small: need " + std::to_string(need) + " words"); }
@@ -486,7 +531,8 @@ const char* hfb200_pool_prove(hfb200_pool* pool, hfb200_segment_job* jobs, size_
                     err = control_root_impl(sl.ctx, j.po2, it->second.code, root, it->second.gen);
                 }
             }
-            if (!err && pool->accum_fn) err = prove_job_with_accum(pool, sl.ctx, j, idx);
+            if (!err && !j.data) err = prove_job_with_witgen(pool, sl.ctx, j, idx);
+            else if (!err && pool->accum_fn) err = prove_job_with_accum(pool, sl.ctx, j, idx);
             else if (!err) err = hfb200_prove_segment(sl.ctx, j.po2, j.globals, j.code, j.data, j.blind_seed, j.seal_out, j.seal_cap, &j.seal_words);
             j.device = sl.device;
             j.ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -548,6 +594,14 @@ const char* hfb200_pool_set_accum(hfb200_pool* pool, hfb200_accum_fn fn, void* u
     if (!pool) throw Err("hfb200_pool_set_accum: NULL pool");
     pool->accum_fn = fn;
     pool->accum_user = fn ? user : nullptr;
+    API_CATCH
+}
+
+const char* hfb200_pool_set_witgen(hfb200_pool* pool, hfb200_witgen_fn fn, void* user) {
+    API_TRY
+    if (!pool) throw Err("hfb200_pool_set_witgen: NULL pool");
+    pool->witgen_fn = fn;
+    pool->witgen_user = fn ? user : nullptr;
     API_CATCH
 }
 

@@ -216,9 +216,12 @@ struct Prover {
         if (dev.stream) cudaStreamSynchronize(dev.stream);
 #endif
         begun = false;
+        witness_open = false;
     }
     void destroy() {
         dev.free(arena.base);
+        dev.free(wit_scratch);
+        wit_scratch = nullptr; wit_scratch_cap = 0;
 #ifndef HFB200_EMU
         drop_graphs();
         if (stage_h) cudaFreeHost(stage_h);
@@ -378,6 +381,13 @@ struct Prover {
     }
     Staged stage_inputs(uint32_t p, const uint32_t* globals_h, const uint32_t* code_h, const uint32_t* data_h, uint64_t blind, bool dev_inputs = false) {
         t_begin = std::chrono::steady_clock::now();
+        // data == NULL after hfb200_segment_witness_dev: the DATA columns are the caller's, already in place, blinded with the key
+        // derived there (one segment, one key)
+        const bool witness = !data_h && witness_open;
+        if (witness && p != po2)
+            throw Err("po2 " + std::to_string(p) + " differs from the one of hfb200_segment_witness_dev (" + std::to_string(po2) + ")");
+        if (witness && blind != witness_seed)
+            throw Err("blind_seed " + std::to_string(blind) + " differs from the one of hfb200_segment_witness_dev (" + std::to_string(witness_seed) + ")");
         bind();
         layout(p);
         const size_t N = (size_t)1 << po2;
@@ -387,11 +397,12 @@ struct Prover {
         launches_at_begin = dev.launches;
         host_syncs_at_begin = host_syncs;
         stage_off = 0;
-        blind_key = make_blind_key(blind);
         // every argument check comes BEFORE the first copy is queued: an error return must not leave DMA from caller memory in flight
         for (uint32_t i = 0; i < N_GLOBAL; i++) if (globals_h[i] >= P) throw Err("globals: non-canonical field element");
-        if (data_h && !code_h && !control_cached) throw Err("code is NULL and no control group is resident for this po2 (hfb200_control_root)");
-        if (!data_h && !have_trace) throw Err("no trace: pass code/data (code may be NULL after hfb200_control_root) or call hfb200_witgen_synth first");
+        if ((data_h || witness) && !code_h && !control_cached) throw Err("code is NULL and no control group is resident for this po2 (hfb200_control_root)");
+        if (!data_h && !witness && !have_trace) throw Err("no trace: pass code/data (code may be NULL after hfb200_control_root) or call hfb200_witgen_synth first");
+        if (!witness) blind_key = make_blind_key(blind);
+        witness_open = false;  // any begin consumes (or, with data, abandons) the open witness
         if (dev_inputs && code_h) check_device_ptr(code_h, "code");
         if (dev_inputs && data_h) check_device_ptr(data_h, "data");
         std::memcpy(globals, globals_h, sizeof globals);
@@ -424,7 +435,7 @@ struct Prover {
         } else
 #endif
         if (data_h && !dev_inputs) { dev.h2d(tr[GROUP_DATA], data_h, (size_t)cir.cd.w_data * N * 4); }
-        const bool use_control = !code_h && data_h && control_cached;
+        const bool use_control = !code_h && (data_h || witness) && control_cached;
         if (code_h) { control_cached = false; control_gen = 0; }  // the resident control columns change
         if (data_h) have_trace = true;
         return Staged{chunked, use_control};
@@ -513,12 +524,49 @@ struct Prover {
         dev.launch<AccumScanKernel, 256, 1>(nblk, n_chains, 256, sm, tr[GROUP_ACCUM], N, rows, first_chain, kind, partial, 1);
         arena.off = save;  // stream order makes reuse by later kernels safe
     }
-    // the ZK_CYCLES blinding rows of every accum column, from this segment's key
+    // the ZK_CYCLES blinding rows of every column of group g, from this segment's key
+    void blind_rows(int g) {
+        bind();
+        const uint32_t w = cir.group_width(g);
+        const uint64_t total = (uint64_t)w * ZK_CYCLES;
+        dev.launch<BlindRowsKernel, 256, 1>((unsigned)((total + 255) / 256), 1, 256, 0, tr[g], w, po2, ZK_CYCLES, (uint32_t)g, blind_key);
+    }
     void accum_blind() {
         if (!begun) throw Err("hfb200_segment_accum_blind: no segment in flight");
+        blind_rows(GROUP_ACCUM);
+    }
+
+    // ---- the device witness seam (hfb200_segment_witness_dev .. the begin that commits the columns) ----
+    // witness_dev lays the context out for po2 and derives the segment's blinding key once; the caller's witness generator then
+    // writes the resident DATA columns, and the next begin with data == NULL commits them as they stand, under that same key.
+    bool witness_open = false;
+    uint64_t witness_seed = 0;
+    void* wit_scratch = nullptr;  // hfb200_segment_scratch: grows on demand, freed in destroy()
+    size_t wit_scratch_cap = 0;
+    void witness_dev(uint32_t p, uint64_t blind) {
+        if (p < MIN_PO2 || p > max_po2)
+            throw Err("hfb200_segment_witness_dev: po2 " + std::to_string(p) + " outside [12, " + std::to_string(max_po2) + "]");
         bind();
-        const uint64_t total = (uint64_t)cir.cd.w_accum * ZK_CYCLES;
-        dev.launch<AccumBlindKernel, 256, 1>((unsigned)((total + 255) / 256), 1, 256, 0, tr[GROUP_ACCUM], cir.cd.w_accum, po2, ZK_CYCLES, blind_key);
+        if (begun) quiesce();  // a segment still in flight is abandoned; its chunked upload must not land over the caller's columns
+        layout(p);             // the same po2 again keeps the resident control group
+        have_trace = false;    // the data columns are the caller's from here on
+        blind_key = make_blind_key(blind);
+        witness_seed = blind;
+        witness_open = true;
+    }
+    void data_blind() {
+        if (!witness_open) throw Err("hfb200_segment_data_blind: no witness open (call hfb200_segment_witness_dev)");
+        blind_rows(GROUP_DATA);
+    }
+    void* segment_scratch(size_t bytes) {
+        if (!witness_open) throw Err("hfb200_segment_scratch: no witness open (call hfb200_segment_witness_dev)");
+        if (bytes > wit_scratch_cap) {
+            bind();
+            if (wit_scratch) { dev.sync(); dev.free(wit_scratch); wit_scratch = nullptr; wit_scratch_cap = 0; }  // earlier users are done
+            wit_scratch = dev.alloc(bytes);
+            wit_scratch_cap = bytes;
+        }
+        return wit_scratch;
     }
 
     // key_dev != NULL: the blinding key is read from device memory (graph replay); the by-value copy is then a placeholder

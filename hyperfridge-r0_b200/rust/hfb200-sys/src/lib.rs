@@ -113,6 +113,25 @@ pub const HFB200_SCAN_SUM: c_int = 1;
 pub type hfb200_accum_fn =
     Option<unsafe extern "C" fn(user: *mut c_void, ctx: *mut hfb200_ctx, seg: *const hfb200_segment_dev, job: usize) -> c_int>;
 
+/// The writable DATA columns between `hfb200_segment_witness_dev` and the begin (data = null) that commits them as they stand.
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct hfb200_witness_dev {
+    pub po2: u32,
+    /// the last `zk_rows` rows of every DATA column are blinding rows (`hfb200_segment_data_blind`)
+    pub zk_rows: u32,
+    pub w_code: u32,
+    pub w_data: u32,
+    pub device: c_int,
+    /// the context's `cudaStream_t` (null in the host emulator)
+    pub stream: *mut c_void,
+    /// device u32[w_data][N]: the context's resident data columns
+    pub data: *mut u32,
+}
+/// The caller's witness generator for every pool job with `data` = null (`hfb200_pool_set_witgen`); nonzero fails the job.
+pub type hfb200_witgen_fn =
+    Option<unsafe extern "C" fn(user: *mut c_void, ctx: *mut hfb200_ctx, w: *const hfb200_witness_dev, job: usize) -> c_int>;
+
 #[repr(C)]
 #[derive(Clone, Copy, Debug, Default)]
 pub struct hfb200_pool_stats_t {
@@ -159,6 +178,13 @@ extern "C" {
     /// Number of CUDA devices; 0 (and success) without a device or a driver.
     pub fn hfb200_device_count(out: *mut c_int) -> *const c_char;
     pub fn hfb200_pool_set_accum(pool: *mut hfb200_pool, f: hfb200_accum_fn, user: *mut c_void) -> *const c_char;
+    /// Lays the context out for `po2`, derives the segment's blinding key and describes the writable DATA columns.
+    pub fn hfb200_segment_witness_dev(ctx: *mut hfb200_ctx, po2: u32, blind_seed: u64, out: *mut hfb200_witness_dev) -> *const c_char;
+    /// The DATA group's blinding rows from the segment's blinding key (between witness_dev and the begin).
+    pub fn hfb200_segment_data_blind(ctx: *mut hfb200_ctx) -> *const c_char;
+    /// Device memory owned by the context for the caller's compact witness input; valid until the segment ends.
+    pub fn hfb200_segment_scratch(ctx: *mut hfb200_ctx, bytes: usize, out: *mut *mut c_void) -> *const c_char;
+    pub fn hfb200_pool_set_witgen(pool: *mut hfb200_pool, f: hfb200_witgen_fn, user: *mut c_void) -> *const c_char;
     pub fn hfb200_pool_create(
         devices: *const c_int, n_devices: c_int, contexts_per_device: c_int, max_po2: u32, circuit: *const hfb200_circuit_desc,
         out: *mut *mut hfb200_pool,

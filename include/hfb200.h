@@ -152,7 +152,8 @@ typedef struct {
  * the context's stream (the copy follows the stream's earlier work; anything writing them on other streams must be complete).
  * A pointer that is not device memory of that device is refused before anything is queued. */
 enum { HFB200_DEV_INPUTS = 1 };
-/* `code == NULL` reuses the resident control group as in hfb200_segment_begin; `data` may be NULL after hfb200_witgen_synth. */
+/* `code == NULL` reuses the resident control group as in hfb200_segment_begin; `data` may be NULL after hfb200_witgen_synth or
+ * hfb200_segment_witness_dev (below). */
 const char* hfb200_segment_begin_dev(hfb200_ctx* ctx, uint32_t po2, const uint32_t* globals, const uint32_t* code, const uint32_t* data,
                                      uint64_t blind_seed, uint32_t flags, hfb200_segment_dev* out);
 /* Completes the segment begun by either begin, from the accum columns as they stand in device memory (no upload, no built-in
@@ -170,6 +171,32 @@ const char* hfb200_segment_accum_scan(hfb200_ctx* ctx, int kind, uint32_t first_
 const char* hfb200_segment_accum_blind(hfb200_ctx* ctx);
 /* Number of CUDA devices.  No device or no driver is a count of 0 (NULL returned), not an error. */
 const char* hfb200_device_count(int* out);
+
+/* The witness on DEVICE memory (upstream's GPU prover generates it there: witgen kernels expand the preflight trace into the
+ * data columns).  witness_dev lays the context out for po2 (12 <= po2 <= max_po2; the same po2 again keeps a resident control
+ * group) and derives the segment's blinding key, once: hfb200_segment_data_blind and the later accum blinding (built-in
+ * step_accum or hfb200_segment_accum_blind) both use it.  It then describes the writable DATA columns.  The caller's kernels
+ * write them on `stream`; the next hfb200_segment_begin / _begin_dev with data == NULL commits them exactly as they stand (no
+ * copy, no upload) and must pass the same po2 and blind_seed.  `code` keeps its rules: host columns (device columns with
+ * HFB200_DEV_INPUTS) are copied in, NULL reuses the resident control group of that po2.  An error return of any entry
+ * abandons the open witness. */
+typedef struct {
+    uint32_t po2;            /* N = 2^po2 rows                                                            */
+    uint32_t zk_rows;        /* the last zk_rows rows of every DATA column are blinding rows               */
+    uint32_t w_code, w_data;
+    int device;              /* CUDA ordinal of the context                                               */
+    void* stream;            /* the context's cudaStream_t (NULL in the host emulator)                     */
+    uint32_t* data;          /* device u32[w_data][N]: the context's resident data columns                 */
+} hfb200_witness_dev;
+const char* hfb200_segment_witness_dev(hfb200_ctx* ctx, uint32_t po2, uint64_t blind_seed, hfb200_witness_dev* out);
+/* Writes rows [N - zk_rows, N) of every DATA column from the segment's key (the rows hfb200_witgen_synth writes there), on
+ * the context's stream.  Valid between hfb200_segment_witness_dev and the begin that follows. */
+const char* hfb200_segment_data_blind(hfb200_ctx* ctx);
+/* Device memory owned by the context, at least `bytes` long, for the caller's compact witness input (e.g. a preflight trace),
+ * which the caller copies in itself with cudaMemcpyAsync on the witness's `stream`.  Valid until the segment is finished or
+ * abandoned; it grows only when a larger request comes (a grow first waits for the context's stream) and is freed by
+ * hfb200_destroy.  Valid to call while a witness is open. */
+const char* hfb200_segment_scratch(hfb200_ctx* ctx, size_t bytes, void** out);
 
 /* Witness stand-in on the device (replaces preflight + WitnessGenerator for the synthetic circuit):
  * fills the context's resident code/data columns; globals_out receives the 32 global words. */
@@ -269,7 +296,7 @@ typedef struct {
     uint32_t po2;
     const uint32_t* globals; /* [32] */
     const uint32_t* code;    /* u32[w_code][N]  host */
-    const uint32_t* data;    /* u32[w_data][N]  host */
+    const uint32_t* data;    /* u32[w_data][N]  host; NULL = from the pool's witgen callback (hfb200_pool_set_witgen) */
     uint64_t blind_seed;
     uint32_t* seal_out;      /* caller buffer, seal_cap words */
     size_t seal_cap;
@@ -318,6 +345,16 @@ const char* hfb200_pool_load_control(hfb200_pool* pool, uint32_t po2, const uint
  * error takes the device-fault path above.  fn = NULL removes the callback. */
 typedef int (*hfb200_accum_fn)(void* user, hfb200_ctx* ctx, const hfb200_segment_dev* seg, size_t job);
 const char* hfb200_pool_set_accum(hfb200_pool* pool, hfb200_accum_fn fn, void* user);
+/* The caller's witness generator for every job with data == NULL (without one such jobs are refused).  Each of them runs
+ * hfb200_segment_witness_dev, fn on the worker thread (the context's device is current), begin with data == NULL (job.code as
+ * usual, NULL = the pool's shared control group), the accum stage (the accum callback if set, else the built-in step_accum; a
+ * pool over a data-defined circuit without an accum callback refuses the job) and finish.  Jobs with data keep their path.
+ * Callbacks run concurrently, one per worker, and may call only hfb200_segment_scratch / _data_blind on the `ctx` they are given
+ * (plus their own kernels and cudaMemcpyAsync on w->stream).  A nonzero return fails that job only ("witgen callback returned
+ * <rc>"), is not retried, and leaves the context usable; a CUDA error takes the device-fault path, so the callback runs again
+ * on a NEW context: it must rebuild its device state (the scratch contents included) from host input.  fn = NULL removes it. */
+typedef int (*hfb200_witgen_fn)(void* user, hfb200_ctx* ctx, const hfb200_witness_dev* w, size_t job);
+const char* hfb200_pool_set_witgen(hfb200_pool* pool, hfb200_witgen_fn fn, void* user);
 void hfb200_pool_destroy(hfb200_pool* pool);
 
 /* ---- HAL-level operators (second seam: risc0-zkp `Hal` methods), host buffers in/out ----------- */
