@@ -28,6 +28,11 @@ EXPORTS = [
     "hfb200_segment_begin_dev", "hfb200_segment_finish_dev", "hfb200_segment_accum_scan", "hfb200_segment_accum_blind", "hfb200_device_count",
     "hfb200_pool_set_accum",
     "hfb200_segment_witness_dev", "hfb200_segment_data_blind", "hfb200_segment_scratch", "hfb200_pool_set_witgen",
+    "hfb200_hal_stream", "hfb200_hal_sync", "hfb200_hal_host_syncs", "hfb200_hal_batch_interpolate_ntt", "hfb200_hal_zk_shift",
+    "hfb200_hal_batch_expand_into_evaluate_ntt", "hfb200_hal_batch_bit_reverse", "hfb200_hal_hash_rows", "hfb200_hal_hash_fold",
+    "hfb200_hal_batch_evaluate_any", "hfb200_hal_mix_poly_coeffs", "hfb200_hal_poly_divide", "hfb200_hal_eltwise_add_elem",
+    "hfb200_hal_eltwise_sum_extelem", "hfb200_hal_eltwise_copy_elem", "hfb200_hal_eltwise_zeroize_elem", "hfb200_hal_gather_sample",
+    "hfb200_hal_scatter", "hfb200_hal_prefix_products", "hfb200_hal_fri_fold",
 ]
 
 BLIND_OS_ENTROPY, BLIND_DETERMINISTIC = 0, 1
@@ -225,6 +230,26 @@ def load_library(path=None):
         "hfb200_segment_data_blind": (err, [vp]),
         "hfb200_segment_scratch": (err, [vp, sz, C.POINTER(vp)]),
         "hfb200_pool_set_witgen": (err, [vp, vp, vp]),
+        "hfb200_hal_stream": (err, [vp, C.POINTER(vp), C.POINTER(C.c_int)]),
+        "hfb200_hal_sync": (err, [vp]),
+        "hfb200_hal_host_syncs": (u64, [vp]),
+        "hfb200_hal_batch_interpolate_ntt": (err, [vp, vp, sz, sz]),
+        "hfb200_hal_zk_shift": (err, [vp, vp, sz, sz]),
+        "hfb200_hal_batch_expand_into_evaluate_ntt": (err, [vp, vp, vp, sz, sz, u32]),
+        "hfb200_hal_batch_bit_reverse": (err, [vp, vp, sz, sz]),
+        "hfb200_hal_hash_rows": (err, [vp, vp, vp, sz, sz]),
+        "hfb200_hal_hash_fold": (err, [vp, vp, sz, sz]),
+        "hfb200_hal_batch_evaluate_any": (err, [vp, vp, sz, sz, vp, vp, vp, sz]),
+        "hfb200_hal_mix_poly_coeffs": (err, [vp, vp, vp, vp, vp, vp, sz, sz, sz]),
+        "hfb200_hal_poly_divide": (err, [vp, vp, sz, vp, vp]),
+        "hfb200_hal_eltwise_add_elem": (err, [vp, vp, vp, vp, sz]),
+        "hfb200_hal_eltwise_sum_extelem": (err, [vp, vp, vp, sz, sz]),
+        "hfb200_hal_eltwise_copy_elem": (err, [vp, vp, vp, sz]),
+        "hfb200_hal_eltwise_zeroize_elem": (err, [vp, vp, sz]),
+        "hfb200_hal_gather_sample": (err, [vp, vp, vp, sz, sz, sz]),
+        "hfb200_hal_scatter": (err, [vp, vp, vp, vp, vp, sz]),
+        "hfb200_hal_prefix_products": (err, [vp, vp, sz]),
+        "hfb200_hal_fri_fold": (err, [vp, vp, vp, sz, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -529,6 +554,139 @@ class Context:
         ms = C.c_float()
         self._check(self.lib.hfb200_mark_elapsed(self._h, slot_a, other._h, slot_b, C.byref(ms)))
         return ms.value
+
+
+class Hal:
+    """The device HAL (hfb200_hal_*) over a Context: risc0-zkp `Hal` operators on buffers in the context's device memory.
+
+    On a GPU build every buffer is a contiguous torch CUDA tensor of dtype int32 / uint32 on the context's device (its
+    data_ptr() goes to the library); in the host emulator, whose device memory is host memory, buffers are contiguous uint32
+    numpy arrays.  Shapes follow include/hfb200.h: base-field matrices [count, n], Fp4 buffers [..., 4].  Work is queued on the
+    context's stream; call sync() before reading results on the host.  Host Fp4 values (mix, z) are sequences of 4 ints."""
+
+    def __init__(self, ctx):
+        self.ctx, self.lib, self._h = ctx, ctx.lib, ctx._h
+        self.emulator = b"EMULATOR" in self.lib.hfb200_version()
+        st, dev = C.c_void_p(), C.c_int()
+        ctx._check(self.lib.hfb200_hal_stream(self._h, C.byref(st), C.byref(dev)))
+        self.stream, self.device = st.value, dev.value
+
+    def _a(self, buf, name):
+        """Device address of `buf` after the checks the library cannot make (dtype, contiguity, and which memory kind)."""
+        if self.emulator:
+            if not isinstance(buf, np.ndarray) or buf.dtype != np.uint32 or not buf.flags.c_contiguous:
+                raise Hfb200Error("Hal.%s: the host emulator takes contiguous uint32 numpy arrays" % name)
+            return buf.ctypes.data
+        import torch
+        if not isinstance(buf, torch.Tensor) or not buf.is_cuda or buf.device.index != self.device:
+            raise Hfb200Error("Hal.%s: expects a torch CUDA tensor on cuda:%d" % (name, self.device))
+        if buf.dtype not in (torch.int32, torch.uint32) or not buf.is_contiguous():
+            raise Hfb200Error("Hal.%s: expects a contiguous int32 / uint32 tensor" % name)
+        return buf.data_ptr()
+
+    def _run(self, e):
+        self.ctx._check(e)
+
+    @staticmethod
+    def _e4(v):
+        return np.ascontiguousarray(np.asarray(v, dtype=np.uint64).reshape(4), dtype=np.uint32)
+
+    def sync(self):
+        self._run(self.lib.hfb200_hal_sync(self._h))
+
+    def host_syncs(self):
+        return self.lib.hfb200_hal_host_syncs(self._h)
+
+    def batch_interpolate_ntt(self, io):
+        count, n = io.shape
+        self._run(self.lib.hfb200_hal_batch_interpolate_ntt(self._h, self._a(io, "batch_interpolate_ntt"), count, n))
+
+    def zk_shift(self, io):
+        count, n = io.shape
+        self._run(self.lib.hfb200_hal_zk_shift(self._h, self._a(io, "zk_shift"), count, n))
+
+    def batch_expand_into_evaluate_ntt(self, out, inp, expand_bits):
+        count, n_in = inp.shape
+        if tuple(out.shape) != (count, n_in << expand_bits):
+            raise Hfb200Error("Hal.batch_expand_into_evaluate_ntt: out must be [count, n_in << expand_bits]")
+        self._run(self.lib.hfb200_hal_batch_expand_into_evaluate_ntt(self._h, self._a(out, "expand"), self._a(inp, "expand"), count, n_in, expand_bits))
+
+    def batch_bit_reverse(self, io):
+        count, n = io.shape
+        self._run(self.lib.hfb200_hal_batch_bit_reverse(self._h, self._a(io, "batch_bit_reverse"), count, n))
+
+    def hash_rows(self, digests, matrix):
+        """digests [rows, 8] <- leaf digest of every row of matrix [cols, rows]."""
+        cols, rows = matrix.shape
+        if tuple(digests.shape) != (rows, 8):
+            raise Hfb200Error("Hal.hash_rows: digests must be [rows, 8]")
+        self._run(self.lib.hfb200_hal_hash_rows(self._h, self._a(digests, "hash_rows"), self._a(matrix, "hash_rows"), rows, cols))
+
+    def hash_fold(self, io, input_size, output_size):
+        """io [2 * rows, 8] heap-layout nodes: level output_size from level input_size."""
+        self._run(self.lib.hfb200_hal_hash_fold(self._h, self._a(io, "hash_fold"), input_size, output_size))
+
+    def merkle_tree(self, nodes, matrix):
+        """hash_rows into the leaf level of nodes [2 * rows, 8], then every fold: the whole tree through the HAL."""
+        rows = matrix.shape[1]
+        self.hash_rows(nodes[rows:], matrix)
+        size = rows
+        while size > 1:
+            self.hash_fold(nodes, size, size // 2)
+            size //= 2
+
+    def batch_evaluate_any(self, coeffs, which, xs, out):
+        """out[j] = sum_k coeffs[which[j]][k] * xs[j]^k; coeffs [poly_count, n], which [count], xs / out [count, 4]."""
+        poly_count, n = coeffs.shape
+        count = which.shape[0]
+        self._run(self.lib.hfb200_hal_batch_evaluate_any(self._h, self._a(coeffs, "batch_evaluate_any"), poly_count, n, self._a(which, "batch_evaluate_any"),
+                                                         self._a(xs, "batch_evaluate_any"), self._a(out, "batch_evaluate_any"), count))
+
+    def mix_poly_coeffs(self, out, mix_start, mix, inp, combo_of_col):
+        """out [n_combos, n, 4] += mix_start * mix^c * inp[c] into combo combo_of_col[c]; inp [n_cols, n]."""
+        n_cols, n = inp.shape
+        n_combos = out.shape[0]
+        ms, m = self._e4(mix_start), self._e4(mix)
+        self._run(self.lib.hfb200_hal_mix_poly_coeffs(self._h, self._a(out, "mix_poly_coeffs"), _ptr(ms), _ptr(m), self._a(inp, "mix_poly_coeffs"),
+                                                      self._a(combo_of_col, "mix_poly_coeffs"), n_cols, n, n_combos))
+
+    def poly_divide(self, poly, z, remainder):
+        """poly [n, 4] <- quotient of poly / (x - z) (last element 0); remainder [4] (device) <- poly(z)."""
+        zz = self._e4(z)
+        self._run(self.lib.hfb200_hal_poly_divide(self._h, self._a(poly, "poly_divide"), poly.shape[0], _ptr(zz), self._a(remainder, "poly_divide")))
+
+    def eltwise_add_elem(self, out, x, y):
+        self._run(self.lib.hfb200_hal_eltwise_add_elem(self._h, self._a(out, "eltwise_add_elem"), self._a(x, "eltwise_add_elem"), self._a(y, "eltwise_add_elem"), _numel(out)))
+
+    def eltwise_sum_extelem(self, out, inp):
+        """out [4, count] <- components of sum_g inp[g]; inp [to_add, count, 4]."""
+        to_add, count = inp.shape[0], inp.shape[1]
+        self._run(self.lib.hfb200_hal_eltwise_sum_extelem(self._h, self._a(out, "eltwise_sum_extelem"), self._a(inp, "eltwise_sum_extelem"), count, to_add))
+
+    def eltwise_copy_elem(self, out, inp):
+        self._run(self.lib.hfb200_hal_eltwise_copy_elem(self._h, self._a(out, "eltwise_copy_elem"), self._a(inp, "eltwise_copy_elem"), _numel(out)))
+
+    def eltwise_zeroize_elem(self, io):
+        self._run(self.lib.hfb200_hal_eltwise_zeroize_elem(self._h, self._a(io, "eltwise_zeroize_elem"), _numel(io)))
+
+    def gather_sample(self, dst, src, idx, stride):
+        self._run(self.lib.hfb200_hal_gather_sample(self._h, self._a(dst, "gather_sample"), self._a(src, "gather_sample"), idx, _numel(dst), stride))
+
+    def scatter(self, into, index, offsets, values):
+        self._run(self.lib.hfb200_hal_scatter(self._h, self._a(into, "scatter"), self._a(index, "scatter"), self._a(offsets, "scatter"),
+                                              self._a(values, "scatter"), _numel(index) - 1))
+
+    def prefix_products(self, io):
+        """io [n, 4] <- inclusive running product."""
+        self._run(self.lib.hfb200_hal_prefix_products(self._h, self._a(io, "prefix_products"), io.shape[0]))
+
+    def fri_fold(self, out, inp, mix):
+        """out [4, n/16] <- fold of inp [4, n] by mix ([4], device)."""
+        self._run(self.lib.hfb200_hal_fri_fold(self._h, self._a(out, "fri_fold"), self._a(inp, "fri_fold"), inp.shape[1], self._a(mix, "fri_fold")))
+
+
+def _numel(a):
+    return int(a.numel()) if hasattr(a, "numel") and callable(a.numel) else int(a.size)
 
 
 def device_count(lib=None):

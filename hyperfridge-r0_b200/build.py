@@ -8,7 +8,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libhfb200.so")
 SOURCES = ["hfb200.cu"]
-DEPS = ["hfb200.cu", "prover.cuh", "ntt.cuh", "ntt_tma.cuh", "ntt_mid.cuh", "transcript.cuh", "poseidon2.cuh", "poseidon2_consts.inc", "circuit.cuh", "deep.cuh", "dev.cuh", "blind.cuh", "field.cuh", "probe.cuh", "jit.cuh", "verify.cuh"]
+DEPS = ["hfb200.cu", "prover.cuh", "ntt.cuh", "ntt_tma.cuh", "ntt_mid.cuh", "transcript.cuh", "poseidon2.cuh", "poseidon2_consts.inc", "circuit.cuh", "deep.cuh", "dev.cuh", "blind.cuh", "field.cuh", "probe.cuh", "jit.cuh", "verify.cuh", "hal.cuh"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-ldl"]
 
 

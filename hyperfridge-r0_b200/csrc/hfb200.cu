@@ -3,6 +3,7 @@
 #include "prover.cuh"
 #include "probe.cuh"
 #include "verify.cuh"
+#include "hal.cuh"
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -19,6 +20,9 @@ struct hfb200_ctx {
 #ifndef HFB200_EMU
     cudaEvent_t marks[4] = {nullptr, nullptr, nullptr, nullptr};
 #endif
+    // device HAL (hfb200_hal_*): scratch of the operators that need it, grown on demand, freed by hfb200_destroy
+    void* hal_scratch = nullptr;
+    size_t hal_scratch_cap = 0;
 };
 
 // the one message that is NOT malloc'd (returned when malloc itself fails); hfb200_free_error recognises it by address
@@ -98,7 +102,7 @@ void hfb200_destroy(hfb200_ctx* ctx) {
 #ifndef HFB200_EMU
     for (auto& m : ctx->marks) if (m) { cudaEventDestroy(m); m = nullptr; }
 #endif
-    try { ctx->p.destroy(); } catch (...) {}
+    try { ctx->p.dev.free(ctx->hal_scratch); ctx->p.destroy(); } catch (...) {}
     delete ctx;
 }
 
@@ -712,6 +716,281 @@ const char* hfb200_op_fri_fold(hfb200_ctx* ctx, uint32_t* out, const uint32_t* i
     d.launch<FriFoldKernel, 256, 1>((unsigned)((n / 16 + 255) / 256), 1, 256, 0, fa);
     d.d2h(out, bo.p, (4 * n / 16) * 4);
     d.sync();
+    API_CATCH
+}
+
+// ---- device HAL: risc0-zkp `Hal` operators on caller device buffers ------------------------------------------------------
+// Every entry checks its sizes, then its pointers, before anything is queued; the work goes on the context's stream and the
+// call returns without waiting for it.
+} // extern "C"
+static void hal_ptr(const hfb200_ctx* ctx, const void* p, const char* fn, const char* what) {
+    if (!p) throw Err(std::string(fn) + ": " + what + " is NULL");
+#ifndef HFB200_EMU
+    cudaPointerAttributes a{};
+    const cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) cudaGetLastError();  // not a pointer the driver knows: clear the error, refuse below
+    if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != ctx->p.device_id)
+        throw Err(std::string(fn) + ": " + what + " is not device memory of device " + std::to_string(ctx->p.device_id));
+#else
+    (void)ctx;
+#endif
+}
+static void hal_aligned16(const void* p, const char* fn, const char* what) {
+    if (reinterpret_cast<uintptr_t>(p) & 15u) throw Err(std::string(fn) + ": " + what + " must be 16-byte aligned");
+}
+// log2 of a power of two n in [lo, 2^max_lg]
+static int hal_po2(size_t n, size_t lo, int max_lg, const char* fn, const char* what) {
+    if (n < lo || (n & (n - 1)) || ilog2(n) > max_lg)
+        throw Err(std::string(fn) + ": " + what + " = " + std::to_string(n) + " is not a power of two in [" + std::to_string(lo) + ", 2^" + std::to_string(max_lg) + "]");
+    return ilog2(n);
+}
+static void hal_limit(size_t v, size_t lo, size_t hi, const char* fn, const char* what) {
+    if (v < lo || v > hi) throw Err(std::string(fn) + ": " + what + " = " + std::to_string(v) + " outside [" + std::to_string(lo) + ", " + std::to_string(hi) + "]");
+}
+static hfb200_ctx* hal_ctx(hfb200_ctx* ctx, const char* fn) {
+    if (!ctx) throw Err(std::string(fn) + ": NULL ctx");
+    ctx->p.bind();
+    return ctx;
+}
+// context-owned scratch: grows when a larger request comes (after the stream's earlier users are done), never shrinks
+static void* hal_scratch(hfb200_ctx* ctx, size_t bytes) {
+    if (bytes > ctx->hal_scratch_cap) {
+        if (ctx->hal_scratch) { ctx->p.sync(); ctx->p.dev.free(ctx->hal_scratch); ctx->hal_scratch = nullptr; ctx->hal_scratch_cap = 0; }
+        bytes = std::max<size_t>(bytes, (size_t)1 << 20);
+        ctx->hal_scratch = ctx->p.dev.alloc(bytes);
+        ctx->hal_scratch_cap = bytes;
+    }
+    return ctx->hal_scratch;
+}
+static unsigned hal_blocks(uint64_t items) { return (unsigned)((items + HAL_T - 1) / HAL_T); }
+static constexpr size_t HAL_MAX_ELEMS = (size_t)1 << 34;  // words per buffer (64 GB)
+static E4 hal_e4(const uint32_t* h) { for (int k = 0; k < 4; k++) if (h[k] >= P) throw Err("Fp4 argument holds a non-canonical field element"); return e4(h[0], h[1], h[2], h[3]); }
+extern "C" {
+
+const char* hfb200_hal_stream(hfb200_ctx* ctx, void** stream, int* device) {
+    API_TRY
+    static const char* fn = "hfb200_hal_stream";
+    hal_ctx(ctx, fn);
+    if (!stream) throw Err(std::string(fn) + ": stream is NULL");
+    *stream = (void*)ctx->p.dev.stream;
+    if (device) *device = ctx->p.device_id;
+    API_CATCH
+}
+const char* hfb200_hal_sync(hfb200_ctx* ctx) {
+    API_TRY
+    hal_ctx(ctx, "hfb200_hal_sync")->p.sync();
+    API_CATCH
+}
+uint64_t hfb200_hal_host_syncs(const hfb200_ctx* ctx) { return ctx ? ctx->p.host_syncs : 0; }
+
+const char* hfb200_hal_batch_interpolate_ntt(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n) {
+    API_TRY
+    static const char* fn = "hfb200_hal_batch_interpolate_ntt";
+    hal_ctx(ctx, fn);
+    const int lg = hal_po2(n, 2, 24, fn, "n");
+    hal_limit(count, 1, HAL_MAX_ELEMS >> lg, fn, "count");
+    hal_ptr(ctx, io, fn, "io");
+    ctx->p.ntt.interpolate(io, n, io, n, (uint32_t)count, lg, false);
+    API_CATCH
+}
+const char* hfb200_hal_zk_shift(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n) {
+    API_TRY
+    static const char* fn = "hfb200_hal_zk_shift";
+    hal_ctx(ctx, fn);
+    const int lg = hal_po2(n, 1, 24, fn, "n");
+    hal_limit(count, 1, HAL_MAX_ELEMS >> lg, fn, "count");
+    hal_ptr(ctx, io, fn, "io");
+    const RootTables& rt = ctx->p.ntt.rt;
+    ctx->p.dev.launch<HalZkShiftKernel, HAL_T, 1>(hal_blocks((uint64_t)count << lg), 1, HAL_T, 0, io, (uint64_t)count << lg, (uint32_t)lg, rt.p3_lo, rt.p3_hi);
+    API_CATCH
+}
+const char* hfb200_hal_batch_expand_into_evaluate_ntt(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t n_in, uint32_t expand_bits) {
+    API_TRY
+    static const char* fn = "hfb200_hal_batch_expand_into_evaluate_ntt";
+    hal_ctx(ctx, fn);
+    if (expand_bits != 0 && expand_bits != 2) throw Err(std::string(fn) + ": expand_bits = " + std::to_string(expand_bits) + " is not supported (0 or 2)");
+    const int lg = hal_po2(n_in, 2, 24 - (int)expand_bits, fn, "n_in");
+    hal_limit(count, 1, HAL_MAX_ELEMS >> (lg + expand_bits), fn, "count");
+    hal_ptr(ctx, out, fn, "out");
+    hal_ptr(ctx, in, fn, "in");
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + ((count * n_in) << expand_bits) * 4, i0 = (uintptr_t)in, i1 = i0 + count * n_in * 4;
+    if (o0 < i1 && i0 < o1) throw Err(std::string(fn) + ": out and in overlap");
+    ctx->p.ntt.expand_evaluate(in, n_in, out, (uint64_t)n_in << expand_bits, (uint32_t)count, lg, (int)expand_bits);
+    API_CATCH
+}
+const char* hfb200_hal_batch_bit_reverse(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n) {
+    API_TRY
+    static const char* fn = "hfb200_hal_batch_bit_reverse";
+    hal_ctx(ctx, fn);
+    const int lg = hal_po2(n, 1, 31, fn, "n");
+    hal_limit(count, 1, HAL_MAX_ELEMS >> lg, fn, "count");
+    hal_ptr(ctx, io, fn, "io");
+    ctx->p.dev.launch<HalBitRevKernel, HAL_T, 1>(hal_blocks((uint64_t)count << lg), 1, HAL_T, 0, io, (uint64_t)count << lg, (uint32_t)lg);
+    API_CATCH
+}
+const char* hfb200_hal_hash_rows(hfb200_ctx* ctx, uint32_t* digests, const uint32_t* matrix, size_t rows, size_t cols) {
+    API_TRY
+    static const char* fn = "hfb200_hal_hash_rows";
+    hal_ctx(ctx, fn);
+    hal_limit(rows, 1, 0xFFFFFFFFull, fn, "rows");
+    hal_limit(cols, 1, HAL_MAX_ELEMS / rows, fn, "cols");
+    hal_ptr(ctx, digests, fn, "digests");
+    hal_ptr(ctx, matrix, fn, "matrix");
+    hal_aligned16(digests, fn, "digests");
+    ctx->p.merkle.hash_rows(matrix, rows, (uint32_t)rows, (uint32_t)cols, digests);
+    API_CATCH
+}
+const char* hfb200_hal_hash_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size) {
+    API_TRY
+    static const char* fn = "hfb200_hal_hash_fold";
+    hal_ctx(ctx, fn);
+    hal_limit(output_size, 1, 0x7FFFFFFFull, fn, "output_size");
+    if (input_size != 2 * output_size) throw Err(std::string(fn) + ": input_size must be 2 * output_size");
+    hal_ptr(ctx, io, fn, "io");
+    hal_aligned16(io, fn, "io");
+    ctx->p.merkle.fold_level(io, (uint32_t)output_size);
+    API_CATCH
+}
+const char* hfb200_hal_batch_evaluate_any(hfb200_ctx* ctx, const uint32_t* coeffs, size_t poly_count, size_t n, const uint32_t* which,
+                                          const uint32_t* xs, uint32_t* out, size_t count) {
+    API_TRY
+    static const char* fn = "hfb200_hal_batch_evaluate_any";
+    hal_ctx(ctx, fn);
+    hal_limit(n, 1, HAL_MAX_ELEMS, fn, "n");
+    hal_limit(poly_count, 1, HAL_MAX_ELEMS / n, fn, "poly_count");
+    hal_limit(count, 1, (size_t)65535 * HAL_EV_PTS, fn, "count");
+    hal_ptr(ctx, coeffs, fn, "coeffs");
+    hal_ptr(ctx, which, fn, "which");
+    hal_ptr(ctx, xs, fn, "xs");
+    hal_ptr(ctx, out, fn, "out");
+    const uint32_t nblk = (uint32_t)((n + HAL_EV_RPB - 1) / HAL_EV_RPB);
+    E4* partial = (E4*)hal_scratch(ctx, (size_t)count * nblk * sizeof(E4));
+    Dev& d = ctx->p.dev;
+    d.launch<HalEvalKernel, HAL_T, 1>(nblk, (unsigned)((count + HAL_EV_PTS - 1) / HAL_EV_PTS), HAL_T, (size_t)HAL_EV_PTS * HAL_T * sizeof(E4),
+                                      coeffs, (uint64_t)n, which, xs, (uint64_t)count, partial);
+    d.launch<HalEvalReduceKernel, HAL_T, 1>(hal_blocks(count), 1, HAL_T, 0, (const E4*)partial, nblk, (uint64_t)count, out);
+    API_CATCH
+}
+const char* hfb200_hal_mix_poly_coeffs(hfb200_ctx* ctx, uint32_t* out, const uint32_t* mix_start, const uint32_t* mix, const uint32_t* in,
+                                       const uint32_t* combo_of_col, size_t n_cols, size_t n, size_t n_combos) {
+    API_TRY
+    static const char* fn = "hfb200_hal_mix_poly_coeffs";
+    hal_ctx(ctx, fn);
+    hal_limit(n, 1, HAL_MAX_ELEMS, fn, "n");
+    hal_limit(n_cols, 1, 8192, fn, "n_cols");
+    hal_limit(n_combos, 1, HAL_MAX_ELEMS / 4 / n, fn, "n_combos");
+    if (!mix_start || !mix) throw Err(std::string(fn) + ": mix_start / mix is NULL");
+    const E4 ms = hal_e4(mix_start), m = hal_e4(mix);
+    hal_ptr(ctx, out, fn, "out");
+    hal_ptr(ctx, in, fn, "in");
+    hal_ptr(ctx, combo_of_col, fn, "combo_of_col");
+    E4* w = (E4*)hal_scratch(ctx, n_cols * sizeof(E4));
+    Dev& d = ctx->p.dev;
+    d.launch<HalMixPowKernel, HAL_T, 1>(hal_blocks(n_cols), 1, HAL_T, 0, w, (uint32_t)n_cols, ms, m);
+    d.launch<HalMixPolyKernel, HAL_T, 1>(hal_blocks(n), 1, HAL_T, n_cols * (sizeof(E4) + 4), out, (const E4*)w, in, combo_of_col, (uint32_t)n_cols, (uint64_t)n);
+    API_CATCH
+}
+} // extern "C"
+template <class Op>
+static void hal_scan(hfb200_ctx* ctx, const HalScanArgs& a) {
+    using T = typename Op::T;
+    const uint32_t nblk = (uint32_t)((a.n + HAL_SC_RPB - 1) / HAL_SC_RPB);
+    T* partial = (T*)hal_scratch(ctx, (size_t)nblk * sizeof(T));
+    Dev& d = ctx->p.dev;
+    const size_t sm = 2 * HAL_T * sizeof(T);
+    d.launch<HalScanKernel<Op>, HAL_T, 1>(nblk, 1, HAL_T, sm, a, partial, 0);
+    d.launch<HalScanOffsetsKernel<Op>, HAL_T, 1>(1, 1, HAL_T, sm, partial, nblk);
+    d.launch<HalScanKernel<Op>, HAL_T, 1>(nblk, 1, HAL_T, sm, a, partial, 1);
+}
+extern "C" {
+const char* hfb200_hal_poly_divide(hfb200_ctx* ctx, uint32_t* poly, size_t n, const uint32_t* z, uint32_t* remainder_out) {
+    API_TRY
+    static const char* fn = "hfb200_hal_poly_divide";
+    hal_ctx(ctx, fn);
+    hal_limit(n, 1, (size_t)1 << 30, fn, "n");
+    if (!z) throw Err(std::string(fn) + ": z is NULL");
+    const E4 zz = hal_e4(z);
+    hal_ptr(ctx, poly, fn, "poly");
+    hal_ptr(ctx, remainder_out, fn, "remainder_out");
+    HalScanArgs a{poly, (uint64_t)n, zz, remainder_out};
+    hal_scan<DivScan>(ctx, a);
+    API_CATCH
+}
+const char* hfb200_hal_prefix_products(hfb200_ctx* ctx, uint32_t* io, size_t n) {
+    API_TRY
+    static const char* fn = "hfb200_hal_prefix_products";
+    hal_ctx(ctx, fn);
+    hal_limit(n, 1, (size_t)1 << 30, fn, "n");
+    hal_ptr(ctx, io, fn, "io");
+    HalScanArgs a{io, (uint64_t)n, e4_zero(), nullptr};
+    hal_scan<ProdScan>(ctx, a);
+    API_CATCH
+}
+const char* hfb200_hal_eltwise_add_elem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* x, const uint32_t* y, size_t count) {
+    API_TRY
+    static const char* fn = "hfb200_hal_eltwise_add_elem";
+    hal_ctx(ctx, fn);
+    hal_limit(count, 1, HAL_MAX_ELEMS, fn, "count");
+    hal_ptr(ctx, out, fn, "out"); hal_ptr(ctx, x, fn, "x"); hal_ptr(ctx, y, fn, "y");
+    ctx->p.dev.launch<HalAddElemKernel, HAL_T, 1>(hal_blocks(count), 1, HAL_T, 0, out, x, y, (uint64_t)count);
+    API_CATCH
+}
+const char* hfb200_hal_eltwise_sum_extelem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t to_add) {
+    API_TRY
+    static const char* fn = "hfb200_hal_eltwise_sum_extelem";
+    hal_ctx(ctx, fn);
+    hal_limit(count, 1, HAL_MAX_ELEMS / 4, fn, "count");
+    hal_limit(to_add, 1, HAL_MAX_ELEMS / 4 / count, fn, "to_add");
+    hal_ptr(ctx, out, fn, "out"); hal_ptr(ctx, in, fn, "in");
+    ctx->p.dev.launch<HalSumExtKernel, HAL_T, 1>(hal_blocks(count), 1, HAL_T, 0, out, in, (uint64_t)count, (uint32_t)to_add);
+    API_CATCH
+}
+const char* hfb200_hal_eltwise_copy_elem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count) {
+    API_TRY
+    static const char* fn = "hfb200_hal_eltwise_copy_elem";
+    hal_ctx(ctx, fn);
+    hal_limit(count, 1, HAL_MAX_ELEMS, fn, "count");
+    hal_ptr(ctx, out, fn, "out"); hal_ptr(ctx, in, fn, "in");
+    ctx->p.dev.d2d(out, in, count * 4);
+    API_CATCH
+}
+const char* hfb200_hal_eltwise_zeroize_elem(hfb200_ctx* ctx, uint32_t* io, size_t count) {
+    API_TRY
+    static const char* fn = "hfb200_hal_eltwise_zeroize_elem";
+    hal_ctx(ctx, fn);
+    hal_limit(count, 1, HAL_MAX_ELEMS, fn, "count");
+    hal_ptr(ctx, io, fn, "io");
+    ctx->p.dev.zero(io, count * 4);
+    API_CATCH
+}
+const char* hfb200_hal_gather_sample(hfb200_ctx* ctx, uint32_t* dst, const uint32_t* src, size_t idx, size_t size, size_t stride) {
+    API_TRY
+    static const char* fn = "hfb200_hal_gather_sample";
+    hal_ctx(ctx, fn);
+    hal_limit(size, 1, HAL_MAX_ELEMS, fn, "size");
+    hal_limit(stride, 1, HAL_MAX_ELEMS, fn, "stride");
+    hal_limit(size - 1, 0, HAL_MAX_ELEMS / stride, fn, "size - 1 (times stride)");
+    hal_limit(idx, 0, HAL_MAX_ELEMS - (size - 1) * stride, fn, "idx");
+    hal_ptr(ctx, dst, fn, "dst"); hal_ptr(ctx, src, fn, "src");
+    ctx->p.dev.launch<HalGatherKernel, HAL_T, 1>(hal_blocks(size), 1, HAL_T, 0, dst, src, (uint64_t)idx, (uint64_t)size, (uint64_t)stride);
+    API_CATCH
+}
+const char* hfb200_hal_scatter(hfb200_ctx* ctx, uint32_t* into, const uint32_t* index, const uint32_t* offsets, const uint32_t* values, size_t count) {
+    API_TRY
+    static const char* fn = "hfb200_hal_scatter";
+    hal_ctx(ctx, fn);
+    hal_limit(count, 1, HAL_MAX_ELEMS, fn, "count");
+    hal_ptr(ctx, into, fn, "into"); hal_ptr(ctx, index, fn, "index"); hal_ptr(ctx, offsets, fn, "offsets"); hal_ptr(ctx, values, fn, "values");
+    ctx->p.dev.launch<HalScatterKernel, HAL_T, 1>(hal_blocks(count), 1, HAL_T, 0, into, index, offsets, values, (uint64_t)count);
+    API_CATCH
+}
+const char* hfb200_hal_fri_fold(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t n, const uint32_t* mix) {
+    API_TRY
+    static const char* fn = "hfb200_hal_fri_fold";
+    hal_ctx(ctx, fn);
+    if (n < 16 || (n & 15) || n > HAL_MAX_ELEMS / 4) throw Err(std::string(fn) + ": n = " + std::to_string(n) + " must be a positive multiple of 16");
+    hal_ptr(ctx, out, fn, "out"); hal_ptr(ctx, in, fn, "in"); hal_ptr(ctx, mix, fn, "mix");
+    ctx->p.dev.launch<HalFriFoldKernel, HAL_T, 1>(hal_blocks(n / 16), 1, HAL_T, 16 * sizeof(E4), out, in, (uint64_t)n, mix);
     API_CATCH
 }
 

@@ -589,7 +589,7 @@ struct P2Perm {
 // Hal::hash_rows: leaf r = unpadded sponge over matrix[c * col_stride + r], c < cols.  Digest -> nodes[rows + r].
 struct HashRowsKernel {
     static constexpr bool kBarrier = false;
-    HD static void run(const KCtx& cx, uint32_t* smem, const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
+    HD static void run(const KCtx& cx, uint32_t* smem, const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* leaves) {
         const uint64_t r = (uint64_t)cx.bx * cx.nt + cx.tid;
         const bool live = r < rows;
         if (!live && !P2Perm::kAll) return;
@@ -610,7 +610,7 @@ struct HashRowsKernel {
             h.mix(s);
         }
         if (live) {
-            uint4* dst = reinterpret_cast<uint4*>(nodes + ((uint64_t)rows + r) * 8);
+            uint4* dst = reinterpret_cast<uint4*>(leaves + r * 8);
             dst[0] = make_uint4(s[0], s[1], s[2], s[3]);
             dst[1] = make_uint4(s[4], s[5], s[6], s[7]);
         }
@@ -790,19 +790,36 @@ struct Merkle {
     void permute(uint32_t* states, uint32_t n) {
         dev->launch<PermuteKernel, 128, P2Perm::kMinBlocks>((n + 127) / 128, 1, 128, P2Perm::kSmem, states, n);
     }
+    // Hal::hash_rows: leaves[r] = digest of row r (8 words each), matrix element (r, c) at matrix[c*col_stride + r]
+    void hash_rows(const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* leaves) {
+        const int T = 128;  // = the M of the tensor-core GEMMs (P2Perm)
+        dev->launch<HashRowsKernel, 128, P2Perm::kMinBlocks>((rows + T - 1) / T, 1, T, P2Perm::kSmem, matrix, col_stride, rows, cols, leaves);
+    }
+#ifndef HFB200_EMU
+    // big levels: one thread per node (throughput); <= 4096 nodes: one warp per node (latency)
+    static uint32_t fold_warp_max() {
+        static const uint32_t v = [] { const char* e = std::getenv("HFB200_FOLD_WARP_MAX"); const int x = e ? std::atoi(e) : 0; return x >= 64 ? (uint32_t)x : 4096u; }();
+        return v;
+    }
+#endif
+    // Hal::hash_fold of one level: nodes[level + i] = H(nodes[2 (level + i)] || nodes[2 (level + i) + 1]), i < level
+    void fold_level(uint32_t* nodes, uint32_t level) {
+        const int T = 128;
+#ifndef HFB200_EMU
+        if (level <= fold_warp_max()) { dev->launch<HashFoldWarpKernel, 256, 1>((level * 32 + 255) / 256, 1, 256, 0, nodes, level); return; }
+#endif
+        dev->launch<HashFoldKernel, 128, P2Perm::kMinBlocks>((level + T - 1) / T, 1, T, P2Perm::kSmem, nodes, level);
+    }
     // nodes: 2*rows digests (heap layout).  matrix element (r, c) at matrix[c*col_stride + r].
     void build(const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
-        const int T = 128;  // = the M of the tensor-core GEMMs (P2Perm)
-        dev->launch<HashRowsKernel, 128, P2Perm::kMinBlocks>((rows + T - 1) / T, 1, T, P2Perm::kSmem, matrix, col_stride, rows, cols, nodes);
+        hash_rows(matrix, col_stride, rows, cols, nodes + (uint64_t)rows * 8);
         uint32_t level = rows / 2;
 #ifndef HFB200_EMU
-        // big levels: one thread per node (throughput); <= 4096 nodes: one warp per node (latency); <= 32: one block
-        static const uint32_t warp_max = [] { const char* e = std::getenv("HFB200_FOLD_WARP_MAX"); const int v = e ? std::atoi(e) : 0; return v >= 64 ? (uint32_t)v : 4096u; }();
-        for (; level > warp_max; level >>= 1) dev->launch<HashFoldKernel, 128, P2Perm::kMinBlocks>((level + T - 1) / T, 1, T, P2Perm::kSmem, nodes, level);
-        for (; level > 32; level >>= 1) dev->launch<HashFoldWarpKernel, 256, 1>((level * 32 + 255) / 256, 1, 256, 0, nodes, level);
+        // <= 32 nodes: the remaining levels in one block
+        for (; level > 32; level >>= 1) fold_level(nodes, level);
         if (level >= 1) dev->launch<HashFoldWarpTailKernel, 1024, 1>(1, 1, 1024, 0, nodes, level);
 #else
-        for (; level >= 512; level >>= 1) dev->launch<HashFoldKernel, 128, P2Perm::kMinBlocks>((level + T - 1) / T, 1, T, P2Perm::kSmem, nodes, level);
+        for (; level >= 512; level >>= 1) fold_level(nodes, level);
         if (level >= 1) dev->launch<HashFoldTailKernel, 256, 1>(1, 1, 256, 0, nodes, level);
 #endif
     }

@@ -223,6 +223,42 @@ extern "C" {
     pub fn hfb200_graph_launches(ctx: *const hfb200_ctx) -> u64;
     /// Control id of (circuit, po2): Merkle root of the committed control columns, computed on the GPU.
     pub fn hfb200_control_root(ctx: *mut hfb200_ctx, po2: u32, code: *const u32, root_out: *mut u32) -> *const c_char;
+
+    // ---- device HAL: risc0-zkp `Hal` operators on caller device buffers (include/hfb200.h states each one's semantics) ----
+    // Every pointer is device memory of the context's device; work goes on the context's stream, nothing synchronises until
+    // hfb200_hal_sync.  Fp4 buffers: 4 consecutive u32 per element.
+    pub fn hfb200_hal_stream(ctx: *mut hfb200_ctx, stream: *mut *mut c_void, device: *mut c_int) -> *const c_char;
+    pub fn hfb200_hal_sync(ctx: *mut hfb200_ctx) -> *const c_char;
+    pub fn hfb200_hal_host_syncs(ctx: *const hfb200_ctx) -> u64;
+    pub fn hfb200_hal_batch_interpolate_ntt(ctx: *mut hfb200_ctx, io: *mut u32, count: usize, n: usize) -> *const c_char;
+    pub fn hfb200_hal_zk_shift(ctx: *mut hfb200_ctx, io: *mut u32, count: usize, n: usize) -> *const c_char;
+    pub fn hfb200_hal_batch_expand_into_evaluate_ntt(
+        ctx: *mut hfb200_ctx, out: *mut u32, input: *const u32, count: usize, n_in: usize, expand_bits: u32,
+    ) -> *const c_char;
+    pub fn hfb200_hal_batch_bit_reverse(ctx: *mut hfb200_ctx, io: *mut u32, count: usize, n: usize) -> *const c_char;
+    pub fn hfb200_hal_hash_rows(ctx: *mut hfb200_ctx, digests: *mut u32, matrix: *const u32, rows: usize, cols: usize) -> *const c_char;
+    pub fn hfb200_hal_hash_fold(ctx: *mut hfb200_ctx, io: *mut u32, input_size: usize, output_size: usize) -> *const c_char;
+    pub fn hfb200_hal_batch_evaluate_any(
+        ctx: *mut hfb200_ctx, coeffs: *const u32, poly_count: usize, n: usize, which: *const u32, xs: *const u32, out: *mut u32, count: usize,
+    ) -> *const c_char;
+    /// `mix_start` / `mix`: HOST Fp4 values (4 words each).
+    pub fn hfb200_hal_mix_poly_coeffs(
+        ctx: *mut hfb200_ctx, out: *mut u32, mix_start: *const u32, mix: *const u32, input: *const u32, combo_of_col: *const u32,
+        n_cols: usize, n: usize, n_combos: usize,
+    ) -> *const c_char;
+    /// `z`: HOST Fp4 value; `remainder_out`: one device Fp4.
+    pub fn hfb200_hal_poly_divide(ctx: *mut hfb200_ctx, poly: *mut u32, n: usize, z: *const u32, remainder_out: *mut u32) -> *const c_char;
+    pub fn hfb200_hal_eltwise_add_elem(ctx: *mut hfb200_ctx, out: *mut u32, x: *const u32, y: *const u32, count: usize) -> *const c_char;
+    pub fn hfb200_hal_eltwise_sum_extelem(ctx: *mut hfb200_ctx, out: *mut u32, input: *const u32, count: usize, to_add: usize) -> *const c_char;
+    pub fn hfb200_hal_eltwise_copy_elem(ctx: *mut hfb200_ctx, out: *mut u32, input: *const u32, count: usize) -> *const c_char;
+    pub fn hfb200_hal_eltwise_zeroize_elem(ctx: *mut hfb200_ctx, io: *mut u32, count: usize) -> *const c_char;
+    pub fn hfb200_hal_gather_sample(ctx: *mut hfb200_ctx, dst: *mut u32, src: *const u32, idx: usize, size: usize, stride: usize) -> *const c_char;
+    pub fn hfb200_hal_scatter(
+        ctx: *mut hfb200_ctx, into: *mut u32, index: *const u32, offsets: *const u32, values: *const u32, count: usize,
+    ) -> *const c_char;
+    pub fn hfb200_hal_prefix_products(ctx: *mut hfb200_ctx, io: *mut u32, n: usize) -> *const c_char;
+    /// `mix`: one Fp4 in DEVICE memory.
+    pub fn hfb200_hal_fri_fold(ctx: *mut hfb200_ctx, out: *mut u32, input: *const u32, n: usize, mix: *const u32) -> *const c_char;
 }
 
 /// Same contract as `risc0_sys::ffi_wrap`.

@@ -386,6 +386,77 @@ const char* hfb200_bench_modmul(hfb200_ctx* ctx, int kind, uint32_t iters, doubl
 const char* hfb200_mark(hfb200_ctx* ctx, int slot);
 const char* hfb200_mark_elapsed(hfb200_ctx* a, int slot_a, hfb200_ctx* b, int slot_b, float* ms);
 
+/* ---- device HAL: risc0-zkp `Hal` operators on caller DEVICE buffers ------------------------------------------------
+ * The second seam (upstream's `Prover`, `MerkleTreeProver` and `fri_prove` are written against `risc0_zkp::hal::Hal`): the
+ * operators a `Hal` implementation needs, on device memory the caller owns (INTEGRATION.md sketches `impl Hal for B200Hal`).
+ *   - any context works (one made with max_po2 = 12 is cheap); sizes are bounded by the kernels, not by max_po2;
+ *   - every buffer pointer must be device memory of the context's device: sizes are checked first, then pointers, and a
+ *     refused call queues nothing;
+ *   - work is enqueued on the context's stream (hfb200_hal_stream) and the call returns without synchronising; results are
+ *     visible to later work on that stream, and to the host after hfb200_hal_sync;
+ *   - operators that need scratch (batch_evaluate_any, mix_poly_coeffs, poly_divide, prefix_products) use a buffer owned by
+ *     the context that grows when a larger request comes (a grow first waits for the stream) and is freed by hfb200_destroy.
+ * Layouts: base-field matrices column-major u32[count][n] (Montgomery form); Fp4 buffers hold 4 consecutive words per element
+ * (upstream's Buffer<ExtElem>), c0 + c1 x + c2 x^2 + c3 x^3 with x^4 = -11. */
+/* The context's cudaStream_t (NULL in the host emulator) and device ordinal (device may be NULL). */
+const char* hfb200_hal_stream(hfb200_ctx* ctx, void** stream, int* device);
+/* Waits for everything queued on the context's stream. */
+const char* hfb200_hal_sync(hfb200_ctx* ctx);
+/* Stream synchronisations the context has made since it was created: the segment prover's transcript waits, hfb200_hal_sync
+ * and the waits of a scratch grow.  A sequence of HAL calls that needs no larger scratch leaves it unchanged. */
+uint64_t hfb200_hal_host_syncs(const hfb200_ctx* ctx);
+/* Hal::batch_interpolate_ntt: per column, natural-order evaluations on the 2^k-th roots of unity -> coefficients in
+ * bit-reversed order (scaled by 1/n), in place.  n = 2^k, 2 <= n <= 2^24. */
+const char* hfb200_hal_batch_interpolate_ntt(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n);
+/* Hal::zk_shift: the coefficient at bit-reversed position i (true index j = bitrev(i)) times 3^j, so f(x) -> f(3x).
+ * n = 2^k <= 2^24. */
+const char* hfb200_hal_zk_shift(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n);
+/* Hal::batch_expand_into_evaluate_ntt: bit-reversed coefficients u32[count][n_in] -> natural-order evaluations
+ * u32[count][n_in << expand_bits] on the 2^expand_bits times larger domain.  expand_bits in {0, 2}; 2 <= n_in,
+ * n_in << expand_bits <= 2^24; out and in must not overlap. */
+const char* hfb200_hal_batch_expand_into_evaluate_ntt(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t n_in, uint32_t expand_bits);
+/* Hal::batch_bit_reverse: io[c][i] <-> io[c][bitrev(i)] per column, in place.  n = 2^k <= 2^31. */
+const char* hfb200_hal_batch_bit_reverse(hfb200_ctx* ctx, uint32_t* io, size_t count, size_t n);
+/* Hal::hash_rows: digests[r] (8 words) = Poseidon2 sponge over row r of the column-major matrix u32[cols][rows], 16 elements
+ * per absorption, zero padded (the leaves of hfb200_op_merkle and of the segment prover's trees).  Any rows >= 1; digests
+ * 16-byte aligned. */
+const char* hfb200_hal_hash_rows(hfb200_ctx* ctx, uint32_t* digests, const uint32_t* matrix, size_t rows, size_t cols);
+/* Hal::hash_fold: io[output_size + i] = hash_pair(io[input_size + 2i], io[input_size + 2i + 1]) for i < output_size, digests
+ * of 8 words, input_size = 2 * output_size: one level of the heap layout of hfb200_op_merkle (node 1 = root).  16-byte aligned. */
+const char* hfb200_hal_hash_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size);
+/* Hal::batch_evaluate_any: out[j] = sum_{k < n} coeffs[which[j]][k] * xs[j]^k for j < count, coeffs u32[poly_count][n]
+ * (natural order), which u32[count] (each < poly_count), xs and out Fp4[count].  count <= 262140. */
+const char* hfb200_hal_batch_evaluate_any(hfb200_ctx* ctx, const uint32_t* coeffs, size_t poly_count, size_t n, const uint32_t* which,
+                                          const uint32_t* xs, uint32_t* out, size_t count);
+/* Hal::mix_poly_coeffs (the DEEP combos): out[combo_of_col[c]][i] += mix_start * mix^c * in[c][i] for c < n_cols, i < n;
+ * in u32[n_cols][n], combo_of_col u32[n_cols] (each < n_combos), out Fp4[n_combos][n].  mix_start and mix are HOST Fp4 values
+ * (4 words each, read during the call).  n_cols <= 8192. */
+const char* hfb200_hal_mix_poly_coeffs(hfb200_ctx* ctx, uint32_t* out, const uint32_t* mix_start, const uint32_t* mix, const uint32_t* in,
+                                       const uint32_t* combo_of_col, size_t n_cols, size_t n, size_t n_combos);
+/* risc0-zkp poly_divide: synthetic division of the Fp4 polynomial poly[0..n) (natural order) by (x - z), in place:
+ * afterwards poly[k] = r_{k+1} with r_k = poly[k] + z r_{k+1}, r_n = 0 (poly[0..n-1) is the quotient, poly[n-1] = 0), and
+ * remainder_out (device, one Fp4) = r_0 = p(z).  z is a HOST Fp4 value.  Runs as a parallel scan over the affine maps
+ * r -> c + z r.  1 <= n <= 2^30. */
+const char* hfb200_hal_poly_divide(hfb200_ctx* ctx, uint32_t* poly, size_t n, const uint32_t* z, uint32_t* remainder_out);
+/* Hal::eltwise_add_elem: out[i] = x[i] + y[i], i < count. */
+const char* hfb200_hal_eltwise_add_elem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* x, const uint32_t* y, size_t count);
+/* Hal::eltwise_sum_extelem: s_i = sum_{g < to_add} in[g * count + i] over Fp4 in[to_add * count]; out u32[4][count] holds the
+ * four components: out[k * count + i] = s_i.c_k. */
+const char* hfb200_hal_eltwise_sum_extelem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t to_add);
+/* Hal::eltwise_copy_elem: out[i] = in[i], i < count (one cudaMemcpyAsync). */
+const char* hfb200_hal_eltwise_copy_elem(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count);
+/* Hal::eltwise_zeroize_elem: io[i] = 0, i < count. */
+const char* hfb200_hal_eltwise_zeroize_elem(hfb200_ctx* ctx, uint32_t* io, size_t count);
+/* Hal::gather_sample: dst[i] = src[idx + i * stride], i < size. */
+const char* hfb200_hal_gather_sample(hfb200_ctx* ctx, uint32_t* dst, const uint32_t* src, size_t idx, size_t size, size_t stride);
+/* Hal::scatter: for every cycle c < count, into[offsets[j]] = values[j] for j in [index[c], index[c + 1]); index u32[count + 1]. */
+const char* hfb200_hal_scatter(hfb200_ctx* ctx, uint32_t* into, const uint32_t* index, const uint32_t* offsets, const uint32_t* values, size_t count);
+/* Hal::prefix_products: io[i] <- io[0] * io[1] * ... * io[i] over Fp4[n], in place (two-pass block scan). */
+const char* hfb200_hal_prefix_products(hfb200_ctx* ctx, uint32_t* io, size_t n);
+/* Hal::fri_fold: in = 4 component columns u32[4][n] of Fp4 coefficients in bit-reversed order -> out u32[4][n/16],
+ * out[.][idx] = sum_{i < 16} mix^i * in[.][bitrev4(i) * n/16 + idx]; mix = one Fp4 in DEVICE memory.  n a multiple of 16. */
+const char* hfb200_hal_fri_fold(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t n, const uint32_t* mix);
+
 #ifdef __cplusplus
 }
 #endif
