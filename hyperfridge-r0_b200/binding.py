@@ -16,7 +16,8 @@ P = 2013265921
 
 # Every symbol include/hfb200.h declares (tests check that the built library exports all of them).
 EXPORTS = [
-    "hfb200_init", "hfb200_init_ir", "hfb200_ir_source", "hfb200_ir_jit_active", "hfb200_verify_segment", "hfb200_verify_segments", "hfb200_control_root", "hfb200_destroy", "hfb200_free_error", "hfb200_version", "hfb200_host_alloc", "hfb200_host_free",
+    "hfb200_init", "hfb200_init_ir", "hfb200_ir_source", "hfb200_ir_jit_active", "hfb200_ir_compile", "hfb200_ir_load_kernels",
+    "hfb200_ir_nvrtc_programs", "hfb200_verify_segment", "hfb200_verify_segments", "hfb200_control_root", "hfb200_destroy", "hfb200_free_error", "hfb200_version", "hfb200_host_alloc", "hfb200_host_free",
     "hfb200_prove_segment", "hfb200_segment_begin", "hfb200_segment_finish", "hfb200_witgen_synth",
     "hfb200_prove_resident", "hfb200_read_group", "hfb200_seal_words", "hfb200_checkpoint", "hfb200_last_stats",
     "hfb200_total_launches", "hfb200_op_interpolate_ntt", "hfb200_op_expand_ntt", "hfb200_op_lde", "hfb200_op_merkle",
@@ -174,6 +175,9 @@ def load_library(path=None):
         "hfb200_init_ir": (err, [C.c_int, u32, C.POINTER(CircuitIR), C.POINTER(vp)]),
         "hfb200_ir_source": (err, [C.POINTER(CircuitIR), C.c_char_p, sz, C.POINTER(sz)]),
         "hfb200_ir_jit_active": (C.c_int, [vp, C.POINTER(C.c_float)]),
+        "hfb200_ir_compile": (err, [C.POINTER(CircuitIR), C.POINTER(u32), sz, C.c_uint, vp, sz, C.POINTER(sz)]),
+        "hfb200_ir_load_kernels": (err, [C.c_char_p, sz, C.POINTER(sz)]),
+        "hfb200_ir_nvrtc_programs": (u64, []),
         "hfb200_verify_segment": (err, [C.POINTER(CircuitDesc), C.POINTER(CircuitIR), vp, sz, vp, C.POINTER(u32)]),
         "hfb200_control_root": (err, [vp, u32, vp, vp]),
         "hfb200_destroy": (None, [vp]),
@@ -849,6 +853,40 @@ def ir_source(ir, circuit, lib=None):
     if e:
         msg = C.cast(e, C.c_char_p).value.decode(errors="replace"); lib.hfb200_free_error(e); raise Hfb200Error(msg)
     return buf.value.decode()
+
+
+def ir_compile(ir, circuit, po2s, threads=0, lib=None, bundle=True):
+    """Compiles the specialised eval_check kernels of a data-defined circuit for every po2 in `po2s` into the process cache
+    (hfb200_ir_compile; needs NVRTC, not a device; cached sizes are not recompiled).  Returns the kernel bundle that
+    ir_load_kernels takes, or None with bundle=False (only warm the cache)."""
+    lib = lib or load_library()
+    taps, steps = _u32(ir["taps"]), _u32(ir["steps"])
+    desc = _mk_ir(ir, circuit[0], circuit[1], circuit[2], int(ir["n_mix"]), taps.ctypes.data, taps.size // 3, steps.ctypes.data, steps.size // 4, int(ir["ret"]))
+    p = (C.c_uint32 * max(1, len(po2s)))(*[int(x) for x in po2s])
+    if not bundle:
+        _raise_err(lib, lib.hfb200_ir_compile(C.byref(desc), p, len(po2s), threads, None, 0, None))
+        return None
+    need = C.c_size_t()
+    _raise_err(lib, lib.hfb200_ir_compile(C.byref(desc), p, len(po2s), threads, None, 0, C.byref(need)))
+    buf = C.create_string_buffer(need.value)
+    _raise_err(lib, lib.hfb200_ir_compile(C.byref(desc), p, len(po2s), threads, buf, need.value, C.byref(need)))
+    return buf.raw[:need.value]
+
+
+def ir_load_kernels(bundle, lib=None):
+    """Adds a kernel bundle from ir_compile to the process cache (hfb200_ir_load_kernels; needs no device and no NVRTC).
+    Returns the number of (circuit, po2) specialisations it carries."""
+    lib = lib or load_library()
+    bundle = bytes(bundle)
+    n = C.c_size_t()
+    _raise_err(lib, lib.hfb200_ir_load_kernels(bundle, len(bundle), C.byref(n)))
+    return n.value
+
+
+def ir_nvrtc_programs(lib=None):
+    """NVRTC programs this process has compiled (hfb200_ir_nvrtc_programs)."""
+    lib = lib or load_library()
+    return int(lib.hfb200_ir_nvrtc_programs())
 
 
 class Pool:

@@ -97,6 +97,62 @@ int hfb200_ir_jit_active(const hfb200_ctx* ctx, float* compile_ms) {
     if (compile_ms) *compile_ms = ctx->p.jit.compile_ms;
     return ctx->p.jit.ready ? 1 : 0;
 }
+const char* hfb200_ir_compile(const hfb200_circuit_ir* c, const uint32_t* po2s, size_t n_po2, unsigned threads, void* bundle_out, size_t cap,
+                              size_t* need) {
+    API_TRY
+#ifdef HFB200_EMU
+    (void)c; (void)po2s; (void)n_po2; (void)threads; (void)bundle_out; (void)cap; (void)need;
+    throw Err("hfb200_ir_compile: the host emulator build has no sm_100a kernels to compile");
+#else
+    if (!c || (!po2s && n_po2)) throw Err("hfb200_ir_compile: NULL argument");
+    if (need) *need = 0;
+    for (size_t i = 0; i < n_po2; i++) if (po2s[i] < MIN_PO2 || po2s[i] > MAX_PO2) throw Err("po2 must be in [12, 22]");
+    GenericCircuitHost g;  // the checks of hfb200_init_ir, without a device
+    g.init(nullptr, c->w_code, c->w_data, c->w_accum, c->n_mix, reinterpret_cast<const IrTap*>(c->taps), c->n_taps,
+           reinterpret_cast<const IrStep*>(c->steps), c->n_steps, c->ret);
+    std::vector<uint32_t> sizes(po2s, po2s + n_po2);  // ascending, each once: the bundle does not depend on the request's order
+    std::sort(sizes.begin(), sizes.end());
+    sizes.erase(std::unique(sizes.begin(), sizes.end()), sizes.end());
+    std::vector<JitSpec> specs;
+    std::vector<std::vector<JitCubin>> bins;
+    for (uint32_t po2 : sizes) {
+        specs.push_back(jit_spec(g, po2, threads));
+        bins.push_back(JitCache::get().fetch(specs.back(), threads));
+        for (const JitCubin& b : bins.back())
+            if (!b) { std::string why; JitCache::get().nvrtc(&why); throw Err("hfb200_ir_compile: po2 " + std::to_string(po2) + " is not cached and NVRTC is unavailable: " + why); }
+    }
+    if (!bundle_out && !need) return nullptr;
+    const std::string b = jit_bundle(specs, bins, threads);
+    if (need) *need = b.size();
+    if (bundle_out) {
+        if (cap < b.size()) throw Err("hfb200_ir_compile: bundle buffer too small: need " + std::to_string(b.size()) + " bytes");
+        std::memcpy(bundle_out, b.data(), b.size());
+    }
+#endif
+    API_CATCH
+}
+const char* hfb200_ir_load_kernels(const void* bundle, size_t bytes, size_t* specialisations) {
+    API_TRY
+    if (specialisations) *specialisations = 0;
+#ifdef HFB200_EMU
+    (void)bundle; (void)bytes;
+    throw Err("hfb200_ir_load_kernels: the host emulator build runs no sm_100a kernels");
+#else
+    if (!bundle && bytes) throw Err("hfb200_ir_load_kernels: NULL bundle");
+    size_t n = 0;
+    const auto recs = jit_parse_bundle(static_cast<const uint8_t*>(bundle), bytes, &n);
+    JitCache::get().add(recs);
+    if (specialisations) *specialisations = n;
+#endif
+    API_CATCH
+}
+uint64_t hfb200_ir_nvrtc_programs(void) {
+#ifdef HFB200_EMU
+    return 0;
+#else
+    return JitCache::get().programs.load();
+#endif
+}
 void hfb200_destroy(hfb200_ctx* ctx) {
     if (!ctx) return;
 #ifndef HFB200_EMU
@@ -1087,18 +1143,8 @@ const char* hfb200_verify_segments(const hfb200_circuit_desc* c, const hfb200_ci
 //   words 8..15  pre-state digest     words 16..23  post-state digest            words 24..31  output (journal) digest, 0 if not last
 // Digests are Poseidon2 digests (8 field elements, Montgomery form), so every word is a valid global.
 static Digest8 digest_bytes_impl(const uint8_t* bytes, size_t n) {
-    // length first, then 3 bytes per element (24 bits < p), Montgomery form, unpadded_hash
     if (n >= P) throw Err("hfb200_digest_bytes: input too long");
-    std::vector<uint32_t> el;
-    el.reserve(1 + (n + 2) / 3);
-    el.push_back(to_mont((uint32_t)n));
-    for (size_t i = 0; i < n; i += 3) {
-        uint32_t v = bytes[i];
-        if (i + 1 < n) v |= (uint32_t)bytes[i + 1] << 8;
-        if (i + 2 < n) v |= (uint32_t)bytes[i + 2] << 16;
-        el.push_back(to_mont(v));
-    }
-    return host_hash_elems(el.data(), el.size());
+    return host_digest_bytes(bytes, n);
 }
 static Digest8 digest_pair_impl(const uint32_t* a, const uint32_t* b) {
     p2_host_consts();

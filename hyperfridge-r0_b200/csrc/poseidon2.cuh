@@ -840,6 +840,20 @@ static inline Digest8 host_hash_elems(const uint32_t* in, size_t n) {
     Digest8 d; for (int i = 0; i < 8; i++) d.w[i] = s[i];
     return d;
 }
+// digest of a byte string (hfb200_digest_bytes): length first, then 3 bytes per element (24 bits < p), Montgomery form,
+// unpadded_hash.  n < p.
+static inline Digest8 host_digest_bytes(const uint8_t* bytes, size_t n) {
+    std::vector<uint32_t> el;
+    el.reserve(1 + (n + 2) / 3);
+    el.push_back(to_mont((uint32_t)n));
+    for (size_t i = 0; i < n; i += 3) {
+        uint32_t v = bytes[i];
+        if (i + 1 < n) v |= (uint32_t)bytes[i + 1] << 8;
+        if (i + 2 < n) v |= (uint32_t)bytes[i + 2] << 16;
+        el.push_back(to_mont(v));
+    }
+    return host_hash_elems(el.data(), el.size());
+}
 
 struct HostRng {
     uint32_t cells[24] = {0};

@@ -669,7 +669,7 @@ struct Prover {
             h2d_small(d_mp, mp.data(), mp.size() * sizeof(E4));
             uint32_t* d_gl = arena.take<uint32_t>(N_GLOBAL);
             h2d_small(d_gl, globals, N_GLOBAL * 4);
-            if (jit.ready) {
+            if (jit.ensure(po2)) {  // per size: the interpreter runs a size whose kernels are neither cached nor compilable
                 JitEvalArgs ja{};
                 ja.ev[0] = ev[GROUP_ACCUM]; ja.ev[1] = ev[GROUP_CODE]; ja.ev[2] = ev[GROUP_DATA];
                 ja.check = check; ja.mixpow = d_mp; ja.mix = d_mix; ja.globals = d_gl; ja.po2 = po2;

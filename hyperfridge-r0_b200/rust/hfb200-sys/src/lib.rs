@@ -149,6 +149,15 @@ extern "C" {
     pub fn hfb200_ir_source(circuit: *const hfb200_circuit_ir, out: *mut c_char, cap: usize, need: *mut usize) -> *const c_char;
     /// 1 when the context's eval_check runs the NVRTC-specialised kernel (0: interpreter kernel / built-in circuit).
     pub fn hfb200_ir_jit_active(ctx: *const hfb200_ctx, compile_ms: *mut f32) -> c_int;
+    /// Compiles the specialised eval_check kernels of `circuit` for each po2 in `po2s` (12..22) into the process cache (needs
+    /// NVRTC, not a device).  `bundle_out` NULL and `need` NULL: only warm the cache; otherwise `*need` = bundle bytes and,
+    /// with `cap >= *need`, the bundle for `hfb200_ir_load_kernels`.  `threads` 0: up to 8.
+    pub fn hfb200_ir_compile(circuit: *const hfb200_circuit_ir, po2s: *const u32, n_po2: usize, threads: c_uint, bundle_out: *mut c_void,
+                             cap: usize, need: *mut usize) -> *const c_char;
+    /// Adds a bundle's cubins to the process cache (no device, no NVRTC); a malformed bundle is refused whole.
+    pub fn hfb200_ir_load_kernels(bundle: *const c_void, bytes: usize, specialisations: *mut usize) -> *const c_char;
+    /// NVRTC programs this process has compiled.
+    pub fn hfb200_ir_nvrtc_programs() -> u64;
     pub fn hfb200_destroy(ctx: *mut hfb200_ctx);
     pub fn hfb200_free_error(msg: *const c_char);
     /// Seal length in words for `po2`; 0 for po2 outside [12, 22].

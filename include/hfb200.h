@@ -76,13 +76,34 @@ const char* hfb200_init_ir(int device, uint32_t max_po2, const hfb200_circuit_ir
 /* Same, for a circuit given as data.  The constraint polynomial is cut along its top-level AndEqz / AndCond chain into chunks of
  * ~400 steps (HFB200_IR_CHUNK); every chunk becomes one straight-line kernel (its body looped over the rows, so that it runs out of the
  * instruction cache), specialised with NVRTC for sm_100a AND for the segment
- * size (tap offsets become literals): compiled on up to 8 host threads at init for max_po2, for other sizes when first proved. */
+ * size (tap offsets become literals): loaded at init for max_po2, for other sizes when first proved.
+ * The cubins live in a process-wide cache keyed by a Poseidon2 digest of each chunk's whole NVRTC input (options, prelude,
+ * source), so every (circuit, po2) is compiled once per process, on up to 8 host threads; concurrent contexts wait for that
+ * one compile.  A size that is not cached while NVRTC is unavailable runs the interpreter kernel (same seals).
+ * HFB200_NVRTC_LIB=<path> names the NVRTC library in place of the built-in search list. */
 /* The CUDA source of those kernels for po2 = 20 (one thread per LDE row, one kernel per chunk).  Needs no device.  Writes at most
  * `cap` bytes including the terminating NUL; *need = bytes required. */
 const char* hfb200_ir_source(const hfb200_circuit_ir* circuit, char* out, size_t cap, size_t* need);
-/* 1 when the context's eval_check runs the NVRTC-specialised kernel, 0 when it runs the interpreter kernel (built-in
- * circuit: 0).  *compile_ms (may be NULL) = wall time of the most recent specialisation (source + NVRTC on <= 8 threads + load). */
+/* 1 when the context's eval_check runs the NVRTC-specialised kernel for its max_po2, 0 when it runs the interpreter kernel
+ * (built-in circuit: 0).  *compile_ms (may be NULL) = wall time of the most recent specialisation (sources + cache lookup +
+ * NVRTC for the chunks not cached + load). */
 int hfb200_ir_jit_active(const hfb200_ctx* ctx, float* compile_ms);
+/* Compiles the specialised eval_check kernels of `circuit` for each po2 in po2s (12..22) into the process cache.
+ * Needs NVRTC, not a device.  Sizes already cached are not recompiled.
+ * bundle_out == NULL and need == NULL: only warm the cache.  need != NULL: *need = bytes of the bundle that serialises every
+ * requested specialisation, ready for hfb200_ir_load_kernels.  bundle_out != NULL: that bundle (cap >= *need, else an error).
+ * Serialised from the cache, so the same request gives the same bytes.  threads = 0: up to 8 compile threads.
+ * Bundle: magic "HFB200KB", format version, arch ("sm_100a"), per (circuit, po2) its (key, cubin) records, then a Poseidon2
+ * digest over everything before it.  The host emulator build returns an error. */
+const char* hfb200_ir_compile(const hfb200_circuit_ir* circuit, const uint32_t* po2s, size_t n_po2, unsigned threads,
+                              void* bundle_out, size_t cap, size_t* need);
+/* Adds a bundle's cubins to the process cache.  Needs no device and no NVRTC.  A bundle for another circuit or other
+ * code-generation settings loads but never matches.  A malformed bundle (bad magic, version or arch, truncated, digest
+ * mismatch) is refused whole, with nothing added.  *specialisations (optional) = (circuit, po2) entries the bundle carries,
+ * all of them now cached.  The host emulator build returns an error. */
+const char* hfb200_ir_load_kernels(const void* bundle, size_t bytes, size_t* specialisations);
+/* NVRTC programs this process has compiled (tests, probes). */
+uint64_t hfb200_ir_nvrtc_programs(void);
 void hfb200_destroy(hfb200_ctx* ctx);
 void hfb200_free_error(const char* msg);
 
