@@ -34,9 +34,20 @@ EXPORTS = [
     "hfb200_hal_batch_evaluate_any", "hfb200_hal_mix_poly_coeffs", "hfb200_hal_poly_divide", "hfb200_hal_eltwise_add_elem",
     "hfb200_hal_eltwise_sum_extelem", "hfb200_hal_eltwise_copy_elem", "hfb200_hal_eltwise_zeroize_elem", "hfb200_hal_gather_sample",
     "hfb200_hal_scatter", "hfb200_hal_prefix_products", "hfb200_hal_fri_fold",
+    "hfb200_set_hash_suite", "hfb200_pool_set_hash_suite", "hfb200_verify_segment_suite", "hfb200_verify_segments_suite",
+    "hfb200_hal_sha_rows", "hfb200_hal_sha_fold", "hfb200_sha256", "hfb200_hash_elems", "hfb200_hash_pair", "hfb200_rng_script",
 ]
 
 BLIND_OS_ENTROPY, BLIND_DETERMINISTIC = 0, 1
+HASH_POSEIDON2, HASH_SHA256 = 0, 1
+HASH_SUITES = {"poseidon2": HASH_POSEIDON2, "sha-256": HASH_SHA256}  # upstream's `hashfn` names
+
+
+def hash_suite(hashfn):
+    """upstream's hashfn name ("poseidon2" | "sha-256") -> HFB200_HASH_*; "blake2b" and anything else is refused."""
+    if hashfn not in HASH_SUITES:
+        raise Hfb200Error("hashfn %r is not supported (supported: %s)" % (hashfn, ", ".join(sorted(HASH_SUITES))))
+    return HASH_SUITES[hashfn]
 
 
 def _default_blinding(deterministic):
@@ -254,6 +265,17 @@ def load_library(path=None):
         "hfb200_hal_scatter": (err, [vp, vp, vp, vp, vp, sz]),
         "hfb200_hal_prefix_products": (err, [vp, vp, sz]),
         "hfb200_hal_fri_fold": (err, [vp, vp, vp, sz, vp]),
+        "hfb200_set_hash_suite": (err, [vp, C.c_int]),
+        "hfb200_pool_set_hash_suite": (err, [vp, C.c_int]),
+        "hfb200_verify_segment_suite": (err, [C.POINTER(CircuitDesc), C.POINTER(CircuitIR), vp, sz, vp, C.POINTER(u32), C.c_int]),
+        "hfb200_verify_segments_suite": (err, [C.POINTER(CircuitDesc), C.POINTER(CircuitIR), C.POINTER(vp), C.POINTER(sz), sz, vp, vp, C.c_uint,
+                                               C.POINTER(sz), C.c_int]),
+        "hfb200_hal_sha_rows": (err, [vp, vp, vp, sz, sz]),
+        "hfb200_hal_sha_fold": (err, [vp, vp, sz, sz]),
+        "hfb200_sha256": (err, [C.c_char_p, sz, vp]),
+        "hfb200_hash_elems": (err, [C.c_int, vp, sz, vp]),
+        "hfb200_hash_pair": (err, [C.c_int, vp, vp, vp]),
+        "hfb200_rng_script": (err, [C.c_int, vp, sz, vp, sz, vp, sz, C.POINTER(sz)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -309,6 +331,11 @@ class Context:
 
     def graph_launches(self):
         return self.lib.hfb200_graph_launches(self._h)
+
+    def set_hash_suite(self, hashfn):
+        """upstream's `segment_prover(hashfn)`: "poseidon2" (default) or "sha-256" for the segments that follow (hfb200_set_hash_suite:
+        drops the resident control group; SHA-256 takes the host transcript only)."""
+        self._check(self.lib.hfb200_set_hash_suite(self._h, hash_suite(hashfn)))
 
     def _check(self, e):
         if e:
@@ -630,6 +657,17 @@ class Hal:
         """io [2 * rows, 8] heap-layout nodes: level output_size from level input_size."""
         self._run(self.lib.hfb200_hal_hash_fold(self._h, self._a(io, "hash_fold"), input_size, output_size))
 
+    def sha_rows(self, digests, matrix):
+        """hash_rows of the SHA-256 suite: digests [rows, 8] <- leaf digest of every row of matrix [cols, rows]."""
+        cols, rows = matrix.shape
+        if tuple(digests.shape) != (rows, 8):
+            raise Hfb200Error("Hal.sha_rows: digests must be [rows, 8]")
+        self._run(self.lib.hfb200_hal_sha_rows(self._h, self._a(digests, "sha_rows"), self._a(matrix, "sha_rows"), rows, cols))
+
+    def sha_fold(self, io, input_size, output_size):
+        """hash_fold of the SHA-256 suite over io [2 * rows, 8] heap-layout nodes."""
+        self._run(self.lib.hfb200_hal_sha_fold(self._h, self._a(io, "sha_fold"), input_size, output_size))
+
     def merkle_tree(self, nodes, matrix):
         """hash_rows into the leaf level of nodes [2 * rows, 8], then every fold: the whole tree through the HAL."""
         rows = matrix.shape[1]
@@ -729,9 +767,11 @@ class WitnessHandle:
         _raise_err(self.lib, self.lib.hfb200_segment_data_blind(self._h))
 
 
-def verify_segment(seal, code_root, circuit=(16, 192, 48), ir=None, lib=None):
-    """`Receipt::verify` for one segment seal (hfb200_verify_segment; host-side like the reference's verifier, no GPU
-    needed).  Returns the segment's po2; raises Hfb200Error with the reason when the seal is rejected."""
+def verify_segment(seal, code_root, circuit=(16, 192, 48), ir=None, lib=None, hashfn="poseidon2"):
+    """`Receipt::verify` for one segment seal (hfb200_verify_segment_suite; host-side like the reference's verifier, no GPU
+    needed).  `code_root` is the control id of the seal's hash suite `hashfn`.  Returns the segment's po2; raises Hfb200Error
+    with the reason when the seal is rejected."""
+    suite = hash_suite(hashfn)
     lib = lib or load_library()
     seal, code_root = _u32(seal), _u32(code_root)
     if code_root.size != 8:
@@ -740,10 +780,10 @@ def verify_segment(seal, code_root, circuit=(16, 192, 48), ir=None, lib=None):
     if ir is not None:
         taps, steps = _u32(ir["taps"]), _u32(ir["steps"])
         d = _mk_ir(ir, circuit[0], circuit[1], circuit[2], int(ir["n_mix"]), taps.ctypes.data, taps.size // 3, steps.ctypes.data, steps.size // 4, int(ir["ret"]))
-        e = lib.hfb200_verify_segment(None, C.byref(d), _ptr(seal), seal.size, _ptr(code_root), C.byref(po2))
+        e = lib.hfb200_verify_segment_suite(None, C.byref(d), _ptr(seal), seal.size, _ptr(code_root), C.byref(po2), suite)
     else:
         d = CircuitDesc(circuit[0], circuit[1], circuit[2], 0)
-        e = lib.hfb200_verify_segment(C.byref(d), None, _ptr(seal), seal.size, _ptr(code_root), C.byref(po2))
+        e = lib.hfb200_verify_segment_suite(C.byref(d), None, _ptr(seal), seal.size, _ptr(code_root), C.byref(po2), suite)
     if e:
         msg = C.cast(e, C.c_char_p).value.decode(errors="replace")
         lib.hfb200_free_error(e)
@@ -800,10 +840,11 @@ def claim_decode(seal, lib=None):
     return c
 
 
-def verify_segments(seals, code_roots, circuit=(16, 192, 48), ir=None, threads=0, lib=None):
-    """`hfb200_verify_segments`: the segment seals of a composite receipt checked on `threads` host threads (0 = all hardware
-    threads).  `code_roots`: one 8-word control id per seal.  Returns the po2 of every seal; raises Hfb200Error naming the
-    first rejected seal."""
+def verify_segments(seals, code_roots, circuit=(16, 192, 48), ir=None, threads=0, lib=None, hashfn="poseidon2"):
+    """`hfb200_verify_segments_suite`: the segment seals of a composite receipt checked on `threads` host threads (0 = all
+    hardware threads).  `code_roots`: one 8-word control id (of suite `hashfn`) per seal.  Returns the po2 of every seal;
+    raises Hfb200Error naming the first rejected seal."""
+    suite = hash_suite(hashfn)
     lib = lib or load_library()
     seals = [_u32(s) for s in seals]
     roots = np.ascontiguousarray(np.stack([_u32(r) for r in code_roots]) if len(code_roots) else np.zeros((0, 8), np.uint32), dtype=np.uint32)
@@ -817,12 +858,49 @@ def verify_segments(seals, code_roots, circuit=(16, 192, 48), ir=None, threads=0
     if ir is not None:
         taps, steps = _u32(ir["taps"]), _u32(ir["steps"])
         d = _mk_ir(ir, circuit[0], circuit[1], circuit[2], int(ir["n_mix"]), taps.ctypes.data, taps.size // 3, steps.ctypes.data, steps.size // 4, int(ir["ret"]))
-        e = lib.hfb200_verify_segments(None, C.byref(d), ptrs, lens, n, _ptr(roots) if n else None, _ptr(po2), threads, C.byref(bad))
+        e = lib.hfb200_verify_segments_suite(None, C.byref(d), ptrs, lens, n, _ptr(roots) if n else None, _ptr(po2), threads, C.byref(bad), suite)
     else:
         d = CircuitDesc(circuit[0], circuit[1], circuit[2], 0)
-        e = lib.hfb200_verify_segments(C.byref(d), None, ptrs, lens, n, _ptr(roots) if n else None, _ptr(po2), threads, C.byref(bad))
+        e = lib.hfb200_verify_segments_suite(C.byref(d), None, ptrs, lens, n, _ptr(roots) if n else None, _ptr(po2), threads, C.byref(bad), suite)
     _raise_err(lib, e)
     return [int(x) for x in po2[:n]]
+
+
+def sha256(data, lib=None):
+    """Standard SHA-256 of a byte string (hfb200_sha256) as 8 digest words (little-endian bytes = the standard output)."""
+    lib = lib or load_library()
+    data, out = bytes(data), np.zeros(8, np.uint32)
+    _raise_err(lib, lib.hfb200_sha256(data, len(data), _ptr(out)))
+    return out
+
+
+def hash_elems(elems, hashfn="poseidon2", lib=None):
+    """The hash suite's hash of a word slice (hfb200_hash_elems): Merkle leaves and the transcript's element hashes."""
+    lib = lib or load_library()
+    e, out = _u32(elems).reshape(-1), np.zeros(8, np.uint32)
+    _raise_err(lib, lib.hfb200_hash_elems(hash_suite(hashfn), _ptr(e) if e.size else None, e.size, _ptr(out)))
+    return out
+
+
+def hash_pair(a, b, hashfn="poseidon2", lib=None):
+    """The hash suite's hash of two digests (hfb200_hash_pair): Merkle nodes."""
+    lib = lib or load_library()
+    a, b, out = _u32(a), _u32(b), np.zeros(8, np.uint32)
+    _raise_err(lib, lib.hfb200_hash_pair(hash_suite(hashfn), _ptr(a), _ptr(b), _ptr(out)))
+    return out
+
+
+def rng_script(ops, digests, hashfn="poseidon2", lib=None):
+    """Runs the suite's transcript RNG (hfb200_rng_script) through `ops`, a list of ("mix",), ("elem",) or ("bits", b);
+    mixes take the 8-word digests in order.  Returns the draws."""
+    lib = lib or load_library()
+    code = {"mix": 0, "elem": 1, "bits": 2}
+    o = np.array([[code[op[0]], op[1] if len(op) > 1 else 0] for op in ops], dtype=np.uint32).reshape(-1)
+    d = _u32(digests).reshape(-1)
+    cap = max(1, sum(1 for op in ops if op[0] != "mix"))
+    out, n = np.zeros(cap, np.uint32), C.c_size_t()
+    _raise_err(lib, lib.hfb200_rng_script(hash_suite(hashfn), _ptr(o), len(ops), _ptr(d) if d.size else None, d.size // 8, _ptr(out), cap, C.byref(n)))
+    return out[:n.value]
 
 
 def verify_claims(seals, image_id, journal_bytes, lib=None):
@@ -917,6 +995,10 @@ class Pool:
         st = PoolStats()
         self._raise(self.lib.hfb200_pool_stats(self._h, C.byref(st)))
         return st.as_dict()
+
+    def set_hash_suite(self, hashfn):
+        """Hash suite ("poseidon2" | "sha-256") of every worker context, kept across context re-creation (hfb200_pool_set_hash_suite)."""
+        self._raise(self.lib.hfb200_pool_set_hash_suite(self._h, hash_suite(hashfn)))
 
     def inject_fault(self, worker, after_jobs=0, kind=0):
         """Test hook (hfb200_pool_inject_fault): kind 0 = device fault (context re-created, job re-queued), 1 = plain failure."""

@@ -176,7 +176,15 @@ const char* hfb200_set_transcript(hfb200_ctx* ctx, int on_device) {
     if (!ctx) throw Err("hfb200_set_transcript: NULL ctx");
     if (ctx->p.begun) throw Err("hfb200_set_transcript: a segment is in flight");
     if (on_device < 0 || on_device > 2) throw Err("hfb200_set_transcript: mode must be 0 (host), 1 (device) or 2 (device + CUDA-graph replay)");
+    if (on_device >= 1 && ctx->p.hash_suite == HASH_SHA256) throw Err("hfb200_set_transcript: the SHA-256 suite runs the host transcript only");
     ctx->p.transcript_mode = on_device;
+    API_CATCH
+}
+
+const char* hfb200_set_hash_suite(hfb200_ctx* ctx, int suite) {
+    API_TRY
+    if (!ctx) throw Err("hfb200_set_hash_suite: NULL ctx");
+    try { ctx->p.set_hash_suite(suite); } catch (const Err& e) { throw Err(std::string("hfb200_set_hash_suite: ") + e.what()); }
     API_CATCH
 }
 
@@ -387,6 +395,7 @@ struct hfb200_pool {
     bool is_ir = false;
     std::vector<IrTap> ir_taps; std::vector<IrStep> ir_steps; uint32_t ir_ret = 0, ir_n_mix = 0; uint8_t ir_info[16] = {0};
     int blind_mode = BLIND_OS_ENTROPY;
+    int hash_suite = HASH_POSEIDON2;
     // the caller's step_accum (hfb200_pool_set_accum): jobs then run begin_dev -> accum_fn -> finish_dev
     hfb200_accum_fn accum_fn = nullptr;
     void* accum_user = nullptr;
@@ -404,6 +413,7 @@ struct hfb200_pool {
             if (is_ir) ctx->p.init(device, max_po2, desc.w_code, desc.w_data, desc.w_accum, ir_taps.data(), ir_taps.size(), ir_steps.data(), ir_steps.size(), ir_ret, ir_n_mix, ir_info);
             else ctx->p.init(device, max_po2, desc.w_code, desc.w_data, desc.w_accum);
             ctx->p.blind_mode = blind_mode;
+            ctx->p.set_hash_suite(hash_suite);
         } catch (...) { try { ctx->p.destroy(); } catch (...) {} delete ctx; throw; }
         return ctx;
     }
@@ -503,6 +513,14 @@ const char* hfb200_pool_set_blinding(hfb200_pool* pool, int mode) {
     if (mode != BLIND_OS_ENTROPY && mode != BLIND_DETERMINISTIC) throw Err("hfb200_pool_set_blinding: bad mode");
     pool->blind_mode = mode;
     for (auto& sl : pool->slots) if (sl.ctx) sl.ctx->p.blind_mode = mode;
+    API_CATCH
+}
+const char* hfb200_pool_set_hash_suite(hfb200_pool* pool, int suite) {
+    API_TRY
+    if (!pool) throw Err("hfb200_pool_set_hash_suite: NULL pool");
+    if (!hash_suite_valid(suite)) throw Err("hfb200_pool_set_hash_suite: suite must be HFB200_HASH_POSEIDON2 (0) or HFB200_HASH_SHA256 (1)");
+    for (auto& sl : pool->slots) if (sl.ctx) sl.ctx->p.set_hash_suite(suite);
+    pool->hash_suite = suite;
     API_CATCH
 }
 const char* hfb200_pool_inject_fault(hfb200_pool* pool, size_t worker, uint64_t after_jobs, int kind) {
@@ -893,7 +911,7 @@ const char* hfb200_hal_hash_rows(hfb200_ctx* ctx, uint32_t* digests, const uint3
     hal_ptr(ctx, digests, fn, "digests");
     hal_ptr(ctx, matrix, fn, "matrix");
     hal_aligned16(digests, fn, "digests");
-    ctx->p.merkle.hash_rows(matrix, rows, (uint32_t)rows, (uint32_t)cols, digests);
+    ctx->p.merkle.hash_rows(HASH_POSEIDON2, matrix, rows, (uint32_t)rows, (uint32_t)cols, digests);
     API_CATCH
 }
 const char* hfb200_hal_hash_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size) {
@@ -904,7 +922,30 @@ const char* hfb200_hal_hash_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_siz
     if (input_size != 2 * output_size) throw Err(std::string(fn) + ": input_size must be 2 * output_size");
     hal_ptr(ctx, io, fn, "io");
     hal_aligned16(io, fn, "io");
-    ctx->p.merkle.fold_level(io, (uint32_t)output_size);
+    ctx->p.merkle.fold_level(HASH_POSEIDON2, io, (uint32_t)output_size);
+    API_CATCH
+}
+const char* hfb200_hal_sha_rows(hfb200_ctx* ctx, uint32_t* digests, const uint32_t* matrix, size_t rows, size_t cols) {
+    API_TRY
+    static const char* fn = "hfb200_hal_sha_rows";
+    hal_ctx(ctx, fn);
+    hal_limit(rows, 1, 0xFFFFFFFFull, fn, "rows");
+    hal_limit(cols, 1, HAL_MAX_ELEMS / rows, fn, "cols");
+    hal_ptr(ctx, digests, fn, "digests");
+    hal_ptr(ctx, matrix, fn, "matrix");
+    hal_aligned16(digests, fn, "digests");
+    ctx->p.merkle.hash_rows(HASH_SHA256, matrix, rows, (uint32_t)rows, (uint32_t)cols, digests);
+    API_CATCH
+}
+const char* hfb200_hal_sha_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size) {
+    API_TRY
+    static const char* fn = "hfb200_hal_sha_fold";
+    hal_ctx(ctx, fn);
+    hal_limit(output_size, 1, 0x7FFFFFFFull, fn, "output_size");
+    if (input_size != 2 * output_size) throw Err(std::string(fn) + ": input_size must be 2 * output_size");
+    hal_ptr(ctx, io, fn, "io");
+    hal_aligned16(io, fn, "io");
+    ctx->p.merkle.fold_level(HASH_SHA256, io, (uint32_t)output_size);
     API_CATCH
 }
 const char* hfb200_hal_batch_evaluate_any(hfb200_ctx* ctx, const uint32_t* coeffs, size_t poly_count, size_t n, const uint32_t* which,
@@ -1088,14 +1129,19 @@ const char* hfb200_bench_merkle(hfb200_ctx* ctx, uint32_t po2, uint32_t count, u
 
 const char* hfb200_verify_segment(const hfb200_circuit_desc* c, const hfb200_circuit_ir* ir, const uint32_t* seal, size_t seal_words,
                                   const uint32_t* code_root, uint32_t* po2_out) {
+    return hfb200_verify_segment_suite(c, ir, seal, seal_words, code_root, po2_out, HASH_POSEIDON2);
+}
+const char* hfb200_verify_segment_suite(const hfb200_circuit_desc* c, const hfb200_circuit_ir* ir, const uint32_t* seal, size_t seal_words,
+                                        const uint32_t* code_root, uint32_t* po2_out, int suite) {
     API_TRY
     if ((c == nullptr) == (ir == nullptr)) throw Err("hfb200_verify_segment: pass exactly one of circuit / ir");
     if (!seal || !code_root) throw Err("hfb200_verify_segment: NULL seal or code_root");
+    if (!hash_suite_valid(suite)) throw Err("hfb200_verify_segment: suite must be HFB200_HASH_POSEIDON2 (0) or HFB200_HASH_SHA256 (1)");
     VCircuit vc;
     if (c) vc.init_builtin(c->w_code, c->w_data, c->w_accum);
     else vc.init_ir(ir->w_code, ir->w_data, ir->w_accum, ir->n_mix, reinterpret_cast<const IrTap*>(ir->taps), ir->n_taps,
                     reinterpret_cast<const IrStep*>(ir->steps), ir->n_steps, ir->ret, ir->info);
-    verify_segment(vc, seal, seal_words, code_root, po2_out);
+    verify_segment(vc, seal, seal_words, code_root, po2_out, suite);
     API_CATCH
 }
 // n seals at once on up to `threads` host threads (0 = one per hardware thread): what `receipt.verify` does over the segment
@@ -1103,9 +1149,14 @@ const char* hfb200_verify_segment(const hfb200_circuit_desc* c, const hfb200_cir
 // is reported, prefixed with its index; `first_bad` receives that index (or n when all verify).
 const char* hfb200_verify_segments(const hfb200_circuit_desc* c, const hfb200_circuit_ir* ir, const uint32_t* const* seals, const size_t* seal_words,
                                    size_t n, const uint32_t* code_roots, uint32_t* po2_out, unsigned threads, size_t* first_bad) {
+    return hfb200_verify_segments_suite(c, ir, seals, seal_words, n, code_roots, po2_out, threads, first_bad, HASH_POSEIDON2);
+}
+const char* hfb200_verify_segments_suite(const hfb200_circuit_desc* c, const hfb200_circuit_ir* ir, const uint32_t* const* seals, const size_t* seal_words,
+                                         size_t n, const uint32_t* code_roots, uint32_t* po2_out, unsigned threads, size_t* first_bad, int suite) {
     API_TRY
     if ((c == nullptr) == (ir == nullptr)) throw Err("hfb200_verify_segments: pass exactly one of circuit / ir");
     if (n && (!seals || !seal_words || !code_roots)) throw Err("hfb200_verify_segments: NULL argument");
+    if (!hash_suite_valid(suite)) throw Err("hfb200_verify_segments: suite must be HFB200_HASH_POSEIDON2 (0) or HFB200_HASH_SHA256 (1)");
     if (first_bad) *first_bad = n;
     VCircuit vc;
     if (c) vc.init_builtin(c->w_code, c->w_data, c->w_accum);
@@ -1123,7 +1174,7 @@ const char* hfb200_verify_segments(const hfb200_circuit_desc* c, const hfb200_ci
             try {
                 if (!seals[i]) throw Err("NULL seal");
                 uint32_t po2 = 0;
-                verify_segment(vc, seals[i], seal_words[i], code_roots + 8 * i, &po2);
+                verify_segment(vc, seals[i], seal_words[i], code_roots + 8 * i, &po2, suite);
                 if (po2_out) po2_out[i] = po2;
             } catch (const std::exception& e) { errs[i] = e.what(); bad[i] = 1; } catch (...) { errs[i] = "unknown error"; bad[i] = 1; }
         }
@@ -1231,6 +1282,57 @@ const char* hfb200_verify_claims(const uint32_t* const* seals, const size_t* sea
     API_CATCH
 }
 
+// ---- the hash suites' host primitives (the ones the transcript and the verifier use) ----------------------------------
+static void suite_arg(int suite, const char* fn) {
+    if (!hash_suite_valid(suite)) throw Err(std::string(fn) + ": suite must be HFB200_HASH_POSEIDON2 (0) or HFB200_HASH_SHA256 (1)");
+}
+const char* hfb200_sha256(const uint8_t* bytes, size_t n, uint32_t* out8) {
+    API_TRY
+    if ((!bytes && n) || !out8) throw Err("hfb200_sha256: NULL argument");
+    sha256_bytes(bytes, n, out8);
+    API_CATCH
+}
+const char* hfb200_hash_elems(int suite, const uint32_t* elems, size_t n, uint32_t* out8) {
+    API_TRY
+    suite_arg(suite, "hfb200_hash_elems");
+    if ((!elems && n) || !out8) throw Err("hfb200_hash_elems: NULL argument");
+    const Digest8 d = suite_hash_elems(suite, elems, n);
+    std::memcpy(out8, d.w, 32);
+    API_CATCH
+}
+const char* hfb200_hash_pair(int suite, const uint32_t* a8, const uint32_t* b8, uint32_t* out8) {
+    API_TRY
+    suite_arg(suite, "hfb200_hash_pair");
+    if (!a8 || !b8 || !out8) throw Err("hfb200_hash_pair: NULL argument");
+    Digest8 a, b;
+    std::memcpy(a.w, a8, 32); std::memcpy(b.w, b8, 32);
+    const Digest8 d = suite_hash_pair(suite, a, b);
+    std::memcpy(out8, d.w, 32);
+    API_CATCH
+}
+const char* hfb200_rng_script(int suite, const uint32_t* ops, size_t n_ops, const uint32_t* digests, size_t n_digests, uint32_t* out, size_t cap,
+                              size_t* n_out) {
+    API_TRY
+    suite_arg(suite, "hfb200_rng_script");
+    if ((!ops && n_ops) || (!digests && n_digests) || (!out && cap) || !n_out) throw Err("hfb200_rng_script: NULL argument");
+    HostRng rng(suite);
+    size_t d = 0, o = 0;
+    for (size_t i = 0; i < n_ops; i++) {
+        const uint32_t op = ops[2 * i], arg = ops[2 * i + 1];
+        if (op > 2) throw Err("hfb200_rng_script: op must be 0 (mix), 1 (random_elem) or 2 (random_bits)");
+        if (op == 2 && (arg < 1 || arg > 31)) throw Err("hfb200_rng_script: random_bits takes 1..31 bits");
+        if (op == 0) {
+            if (d >= n_digests) throw Err("hfb200_rng_script: more mix ops than digests");
+            rng.mix(digests + 8 * d++);
+            continue;
+        }
+        if (o >= cap) throw Err("hfb200_rng_script: out buffer too small");
+        out[o++] = op == 1 ? rng.random_elem() : rng.random_bits(arg);
+    }
+    *n_out = o;
+    API_CATCH
+}
+
 const char* hfb200_control_root(hfb200_ctx* ctx, uint32_t po2, const uint32_t* code, uint32_t* root_out) {
     return control_root_impl(ctx, po2, code, root_out, 0);
 }
@@ -1295,7 +1397,7 @@ static const char* control_root_impl(hfb200_ctx* ctx, uint32_t po2, const uint32
     p.merkle.build(p.ev[GROUP_CODE], D, (uint32_t)D, w, p.nodes[GROUP_CODE]);
     // keep the committed control group for the segments that follow with code == NULL
     p.commit_tree(Tree{p.ev[GROUP_CODE], D, (uint32_t)D, w, p.nodes[GROUP_CODE]}, "code_root", &p.control_top);
-    p.proof.clear(); p.cps.clear(); p.rng = HostRng();  // commit_tree wrote into the transcript of no segment
+    p.proof.clear(); p.cps.clear(); p.rng = HostRng(p.hash_suite);  // commit_tree wrote into the transcript of no segment
     std::memcpy(root_out, &p.control_top[8], 32);       // heap layout: node 1 is the root
     p.control_cached = true;
     p.control_gen = gen;

@@ -5,6 +5,7 @@
 // registers; a warp owns 32 consecutive rows so every column read is one coalesced 128-byte line.
 #pragma once
 #include "dev.cuh"
+#include "sha256.cuh"
 
 namespace hf {
 
@@ -778,6 +779,7 @@ struct PermuteKernel {
 
 struct Merkle {
     Dev* dev = nullptr;
+    int suite = HASH_POSEIDON2;  // the context's hash suite: build() commits with it
     void init(Dev* d) {
         dev = d;
         p2_host_consts();
@@ -790,8 +792,12 @@ struct Merkle {
     void permute(uint32_t* states, uint32_t n) {
         dev->launch<PermuteKernel, 128, P2Perm::kMinBlocks>((n + 127) / 128, 1, 128, P2Perm::kSmem, states, n);
     }
-    // Hal::hash_rows: leaves[r] = digest of row r (8 words each), matrix element (r, c) at matrix[c*col_stride + r]
-    void hash_rows(const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* leaves) {
+    // Hal::hash_rows of suite s: leaves[r] = digest of row r (8 words each), matrix element (r, c) at matrix[c*col_stride + r]
+    void hash_rows(int s, const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* leaves) {
+        if (s == HASH_SHA256) {
+            dev->launch<ShaRowsKernel, 256, 1>((rows + 255) / 256, 1, 256, 0, matrix, col_stride, rows, cols, leaves);
+            return;
+        }
         const int T = 128;  // = the M of the tensor-core GEMMs (P2Perm)
         dev->launch<HashRowsKernel, 128, P2Perm::kMinBlocks>((rows + T - 1) / T, 1, T, P2Perm::kSmem, matrix, col_stride, rows, cols, leaves);
     }
@@ -802,8 +808,12 @@ struct Merkle {
         return v;
     }
 #endif
-    // Hal::hash_fold of one level: nodes[level + i] = H(nodes[2 (level + i)] || nodes[2 (level + i) + 1]), i < level
-    void fold_level(uint32_t* nodes, uint32_t level) {
+    // Hal::hash_fold of one level in suite s: nodes[level + i] = H(nodes[2 (level + i)] || nodes[2 (level + i) + 1]), i < level
+    void fold_level(int s, uint32_t* nodes, uint32_t level) {
+        if (s == HASH_SHA256) {
+            dev->launch<ShaFoldKernel, 256, 1>((level + 255) / 256, 1, 256, 0, nodes, level);
+            return;
+        }
         const int T = 128;
 #ifndef HFB200_EMU
         if (level <= fold_warp_max()) { dev->launch<HashFoldWarpKernel, 256, 1>((level * 32 + 255) / 256, 1, 256, 0, nodes, level); return; }
@@ -812,14 +822,20 @@ struct Merkle {
     }
     // nodes: 2*rows digests (heap layout).  matrix element (r, c) at matrix[c*col_stride + r].
     void build(const uint32_t* matrix, uint64_t col_stride, uint32_t rows, uint32_t cols, uint32_t* nodes) {
-        hash_rows(matrix, col_stride, rows, cols, nodes + (uint64_t)rows * 8);
+        hash_rows(suite, matrix, col_stride, rows, cols, nodes + (uint64_t)rows * 8);
         uint32_t level = rows / 2;
+        if (suite == HASH_SHA256) {
+            // <= 32 nodes: the remaining levels in one block
+            for (; level > 32; level >>= 1) fold_level(suite, nodes, level);
+            if (level >= 1) dev->launch<ShaFoldTailKernel, 32, 1>(1, 1, 32, 0, nodes, level);
+            return;
+        }
 #ifndef HFB200_EMU
         // <= 32 nodes: the remaining levels in one block
-        for (; level > 32; level >>= 1) fold_level(nodes, level);
+        for (; level > 32; level >>= 1) fold_level(suite, nodes, level);
         if (level >= 1) dev->launch<HashFoldWarpTailKernel, 1024, 1>(1, 1, 1024, 0, nodes, level);
 #else
-        for (; level >= 512; level >>= 1) fold_level(nodes, level);
+        for (; level >= 512; level >>= 1) fold_level(suite, nodes, level);
         if (level >= 1) dev->launch<HashFoldTailKernel, 256, 1>(1, 1, 256, 0, nodes, level);
 #endif
     }
@@ -854,21 +870,46 @@ static inline Digest8 host_digest_bytes(const uint8_t* bytes, size_t n) {
     }
     return host_hash_elems(el.data(), el.size());
 }
+// the transcript's hash of n elements (hash_elem_slice) and of two digests in suite s
+static inline Digest8 suite_hash_elems(int s, const uint32_t* in, size_t n) {
+    if (s != HASH_SHA256) return host_hash_elems(in, n);
+    Digest8 d;
+    sha_hash_words(in, n, d.w);
+    return d;
+}
+static inline Digest8 suite_hash_pair(int s, const Digest8& a, const Digest8& b) {
+    Digest8 d;
+    if (s == HASH_SHA256) { sha_hash_pair(a.w, b.w, d.w); return d; }
+    uint32_t in[16];
+    for (int i = 0; i < 8; i++) { in[i] = a.w[i]; in[8 + i] = b.w[i]; }
+    return host_hash_elems(in, 16);
+}
 
+// The Fiat-Shamir RNG of the transcript: Poseidon2Rng, or ShaRng (sha256.cuh) for the SHA-256 suite
 struct HostRng {
+    int suite = HASH_POSEIDON2;
+    ShaRng sha;
     uint32_t cells[24] = {0};
     int pool_used = 0;
+    HostRng() = default;
+    explicit HostRng(int s) : suite(s) {}
     // Poseidon2Rng::mix: a permutation first when elements were drawn since the last mix (upstream: "if switching from squeezing,
     // do a poseidon2 mix"), then add the 8 digest words into the rate and permute
     void mix(const uint32_t* d8) {
+        if (suite == HASH_SHA256) { sha.mix(d8); return; }
         p2_host_consts();
         if (pool_used != 0) { p2_mix(cells); pool_used = 0; }
         for (int i = 0; i < 8; i++) cells[i] = fadd(cells[i], d8[i]);
         p2_mix(cells);
     }
-    uint32_t random_elem() { if (pool_used == 16) { p2_mix(cells); pool_used = 0; } return cells[pool_used++]; }
+    uint32_t random_elem() {
+        if (suite == HASH_SHA256) return sha.random_elem();
+        if (pool_used == 16) { p2_mix(cells); pool_used = 0; }
+        return cells[pool_used++];
+    }
     E4 random_ext() { uint32_t a = random_elem(), b = random_elem(), c = random_elem(), d = random_elem(); return e4(a, b, c, d); }
     uint32_t random_bits(unsigned bits) {
+        if (suite == HASH_SHA256) return sha.random_bits(bits);
         uint32_t v = from_mont(random_elem());
         for (int i = 0; i < 3; i++) { uint32_t n = from_mont(random_elem()); if (v == 0) v = n; }
         return v & (uint32_t)((1ull << bits) - 1);
@@ -880,7 +921,7 @@ struct HostRng {
 // transcript with context information about the proof system and circuit":
 //   commit(H(PROOF_SYSTEM_INFO.encode())); commit(H(CIRCUIT_INFO.encode()));         (`ProtocolInfo`: 16 bytes, one element per byte)
 //   header = globals ++ [po2 as a raw word]; commit(H(header)); write header
-// Returns the header digest.  Host code, shared by the prover (both transcript modes) and the verifier.
+// Returns the header digest.  Host code, shared by the prover (both transcript modes) and the verifier; hashes in rng's suite.
 static constexpr char PROOF_SYSTEM_INFO[17] = "RISC0_STARK:v1__";      // risc0-zkp PROOF_SYSTEM_INFO
 static constexpr char BUILTIN_CIRCUIT_INFO[17] = "SYNTH_RV32IM:v1_";   // the declared stand-in circuit names itself
 static constexpr char DEFAULT_IR_CIRCUIT_INFO[17] = "RV32IM:v2_______"; // data-defined circuits: upstream's rv32im-v2 string unless given
@@ -892,17 +933,17 @@ static inline void set_circuit_info(char* dst, bool data_defined, const uint8_t*
     else if (given) { std::memcpy(dst, info16, 16); dst[16] = 0; }
     else std::memcpy(dst, DEFAULT_IR_CIRCUIT_INFO, 17);
 }
-static inline Digest8 protocol_info_digest(const char* info16) {
+static inline Digest8 protocol_info_digest(int suite, const char* info16) {
     uint32_t e[16];
     for (int i = 0; i < 16; i++) e[i] = to_mont((uint32_t)(uint8_t)info16[i]);
-    return host_hash_elems(e, 16);
+    return suite_hash_elems(suite, e, 16);
 }
 static inline Digest8 transcript_header(HostRng& rng, const char* circuit_info16, const uint32_t* globals, size_t n_globals, uint32_t po2) {
-    rng.mix(protocol_info_digest(PROOF_SYSTEM_INFO).w);
-    rng.mix(protocol_info_digest(circuit_info16).w);
+    rng.mix(protocol_info_digest(rng.suite, PROOF_SYSTEM_INFO).w);
+    rng.mix(protocol_info_digest(rng.suite, circuit_info16).w);
     std::vector<uint32_t> header(globals, globals + n_globals);
     header.push_back(po2);
-    const Digest8 d = host_hash_elems(header.data(), header.size());
+    const Digest8 d = suite_hash_elems(rng.suite, header.data(), header.size());
     rng.mix(d.w);
     return d;
 }

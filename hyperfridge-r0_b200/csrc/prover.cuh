@@ -87,6 +87,8 @@ struct Prover {
     JitEvalCheck jit;        // their eval_check, specialised at registration (NVRTC, sm_100a)
     uint32_t max_po2 = 0;
     char circuit_info[17] = {0};  // upstream CircuitImpl::CIRCUIT_INFO: second commit of every transcript (poseidon2.cuh)
+    // HASH_POSEIDON2 or HASH_SHA256 (upstream's `hashfn`): the Merkle trees (merkle.suite) and the host transcript hash with it
+    int hash_suite = HASH_POSEIDON2;
     int device_id = 0;
     Arena arena;
     bool debug_checkpoints = false;
@@ -96,7 +98,7 @@ struct Prover {
     bool have_trace = false, begun = false;
     // Control-group commitment kept across segments (opt-in: hfb200_control_root loads it, code == NULL uses it).  The
     // control columns depend on (circuit, po2) only -- upstream's verifier checks their root against a per-po2 table --
-    // so their LDE and Merkle tree need not be rebuilt per segment.  Valid while the context stays at this po2.
+    // so their LDE and Merkle tree need not be rebuilt per segment.  Valid while the context stays at this po2 and hash suite.
     bool control_cached = false;
     uint64_t control_gen = 0;           // which hfb200_pool_load_control call the cached group came from (0: not from a pool)
     std::vector<uint32_t> control_top;  // the tree's top layers as commit_tree reads them
@@ -392,7 +394,7 @@ struct Prover {
         layout(p);
         const size_t N = (size_t)1 << po2;
         arena.off = seg_mark;
-        proof.clear(); cps.clear(); rng = HostRng(); stats = Stats();
+        proof.clear(); cps.clear(); rng = HostRng(hash_suite); stats = Stats();
         for (auto& s : stage_ms) s = 0;
         launches_at_begin = dev.launches;
         host_syncs_at_begin = host_syncs;
@@ -794,7 +796,7 @@ struct Prover {
         }
         }
         proof.insert(proof.end(), reinterpret_cast<uint32_t*>(coeff_u.data()), reinterpret_cast<uint32_t*>(coeff_u.data()) + 4 * coeff_u.size());
-        const Digest8 hash_u = host_hash_elems(reinterpret_cast<uint32_t*>(coeff_u.data()), 4 * coeff_u.size());
+        const Digest8 hash_u = suite_hash_elems(hash_suite, reinterpret_cast<uint32_t*>(coeff_u.data()), 4 * coeff_u.size());
         rng.mix(hash_u.w);
         cp_add("hash_u", hash_u.w, 8);
 
@@ -862,7 +864,7 @@ struct Prover {
         if (debug_checkpoints) {
             std::vector<uint32_t> fc(4 * N);
             dev.d2h(fc.data(), fin, fc.size() * 4); sync();
-            const Digest8 d = host_hash_elems(fc.data(), fc.size());
+            const Digest8 d = suite_hash_elems(hash_suite, fc.data(), fc.size());
             cp_add("final_poly_hash", d.w, 8);
         }
 
@@ -897,7 +899,7 @@ struct Prover {
             std::vector<uint32_t> fc(4 * n);
             dev.d2h(fc.data(), nat, fc.size() * 4); sync();  // the final coefficients feed the transcript
             proof.insert(proof.end(), fc.begin(), fc.end());
-            const Digest8 d = host_hash_elems(fc.data(), fc.size());
+            const Digest8 d = suite_hash_elems(hash_suite, fc.data(), fc.size());
             rng.mix(d.w);
             cp_add("fri_final_hash", d.w, 8);
         }
@@ -962,8 +964,9 @@ struct Prover {
     int transcript_mode = -1;  // -1: environment, 0: host, 1: device, 2: device + CUDA-graph replay
     static int env_transcript() { static const int v = [] { const char* e = std::getenv("HFB200_DEVICE_TRANSCRIPT"); return e ? std::atoi(e) : 0; }(); return v; }
     int transcript_setting() const { return transcript_mode < 0 ? env_transcript() : transcript_mode; }
-    bool device_transcript() const { return transcript_setting() >= 1 && !gen.active; }
-    bool graph_replay() const { return transcript_setting() >= 2 && !gen.active && !debug_checkpoints; }
+    // the device transcript runs Poseidon2Rng only: SHA-256 contexts always take the host transcript
+    bool device_transcript() const { return transcript_setting() >= 1 && !gen.active && hash_suite == HASH_POSEIDON2; }
+    bool graph_replay() const { return device_transcript() && transcript_setting() >= 2 && !debug_checkpoints; }
     uint64_t graph_launches = 0;  // segments issued as one cudaGraphLaunch
     uint8_t* out_h = nullptr;     // pinned landing area of the seal and the checkpoint words (device-transcript path), allocated in init
     size_t out_cap = 0;
@@ -1230,6 +1233,17 @@ struct Prover {
         stats.ntt_main_bytes = 28ull * W * N;
         stats.host_syncs = host_syncs - host_syncs_at_begin;
         emit_metrics();
+    }
+
+    // between segments: a different suite commits the control columns to a different root, so the resident group is dropped
+    void set_hash_suite(int s) {
+        if (!hash_suite_valid(s)) throw Err("hash suite must be HFB200_HASH_POSEIDON2 (0) or HFB200_HASH_SHA256 (1)");
+        if (begun) throw Err("a segment is in flight");
+        if (s == HASH_SHA256 && transcript_mode >= 1)
+            throw Err("the SHA-256 suite runs the host transcript only (this context is in device transcript mode " + std::to_string(transcript_mode) + ")");
+        if (s != hash_suite) { control_cached = false; control_gen = 0; }
+        hash_suite = s;
+        merkle.suite = s;
     }
 
     void witgen(uint32_t p, uint64_t trace_seed, uint64_t blind, uint32_t* globals_out) {

@@ -5,7 +5,7 @@
 // sites of the reference: /root/reference/host/src/main.rs:622-624 and /root/reference/verifier/src/main.rs:124-126;
 // SURVEY.md Appendix A.8).  Like upstream's, it runs on the HOST: verification is O(queries * log N) hashes and a few
 // thousand extension-field operations -- there is no data-parallel hot path to put on the GPU, and a verifier must not
-// need one.  It shares the field / Poseidon2 / transcript code with the prover's host side (field.cuh, poseidon2.cuh)
+// need one.  It shares the field / hash suite / transcript code with the prover's host side (field.cuh, poseidon2.cuh)
 // and is independent of oracle/ (tests compare the two verifiers on good and tampered seals).
 #pragma once
 #include <functional>
@@ -24,17 +24,12 @@ static inline uint32_t v_rou_rev(unsigned k) { return finv(v_rou_fwd(k)); }
 static inline unsigned v_log2(uint64_t n) { unsigned k = 0; while ((1ull << k) < n) k++; if ((1ull << k) != n) vfail("size is not a power of two"); return k; }
 static inline E4 e4_mul_fp(const E4& a, uint32_t s) { return e4_scale(a, s); }
 static inline E4 v_poly_eval(const E4* c, size_t n, const E4& x) { E4 r = e4_zero(); for (size_t i = n; i-- > 0;) r = e4_add(e4_mul(r, x), c[i]); return r; }
-static inline Digest8 v_hash_pair(const Digest8& a, const Digest8& b) {
-    uint32_t in[16];
-    for (int i = 0; i < 8; i++) { in[i] = a.w[i]; in[8 + i] = b.w[i]; }
-    return host_hash_elems(in, 16);
-}
 static inline bool v_eq(const Digest8& a, const Digest8& b) { for (int i = 0; i < 8; i++) if (a.w[i] != b.w[i]) return false; return true; }
 
 struct VReadIOP {  // verify::read_iop::ReadIOP
     const uint32_t* p; size_t len, pos = 0;
-    HostRng rng;
-    VReadIOP(const uint32_t* s, size_t n) : p(s), len(n) {}
+    HostRng rng;  // its suite is the seal's hash suite: every hash of the verifier follows it
+    VReadIOP(const uint32_t* s, size_t n, int suite) : p(s), len(n), rng(suite) {}
     void need(size_t n) { if (pos + n > len) vfail("seal truncated"); }
     uint32_t read_u32() { need(1); return p[pos++]; }
     void read_elems(uint32_t* out, size_t n) { need(n); for (size_t i = 0; i < n; i++) { const uint32_t w = p[pos++]; if (w >= P) vfail("non-canonical field element"); out[i] = w; } }
@@ -54,7 +49,7 @@ struct VMerkle {  // verify::merkle::MerkleTreeVerifier (top layer in the seal, 
         top_size = (size_t)1 << top_layer;
         top.resize(2 * top_size);
         for (size_t i = 0; i < top_size; i++) top[top_size + i] = iop.read_digest();
-        for (size_t i = top_size - 1; i >= 1; i--) top[i] = v_hash_pair(top[2 * i], top[2 * i + 1]);
+        for (size_t i = top_size - 1; i >= 1; i--) top[i] = suite_hash_pair(iop.rng.suite, top[2 * i], top[2 * i + 1]);
         iop.commit(top[1]);
     }
     const Digest8& root() const { return top[1]; }
@@ -62,11 +57,12 @@ struct VMerkle {  // verify::merkle::MerkleTreeVerifier (top layer in the seal, 
         if (idx >= rows) vfail("merkle index out of range");
         std::vector<uint32_t> row(cols);
         iop.read_elems(row.data(), cols);
-        Digest8 cur = host_hash_elems(row.data(), cols);
+        const int s = iop.rng.suite;
+        Digest8 cur = suite_hash_elems(s, row.data(), cols);
         size_t i = idx + rows;
         while (i >= 2 * top_size) {
             const Digest8 other = iop.read_digest();
-            cur = (i & 1) ? v_hash_pair(other, cur) : v_hash_pair(cur, other);
+            cur = (i & 1) ? suite_hash_pair(s, other, cur) : suite_hash_pair(s, cur, other);
             i >>= 1;
         }
         if (!v_eq(top[i], cur)) vfail("merkle path does not match the committed top layer");
@@ -218,7 +214,7 @@ static inline void v_fri_verify(VReadIOP& iop, size_t degree, const std::functio
     while (degree > V_FRI_MIN_DEGREE) { rounds.emplace_back(iop, domain); domain /= V_FRI_FOLD; degree /= V_FRI_FOLD; }
     std::vector<uint32_t> fc(4 * degree);
     iop.read_elems(fc.data(), fc.size());
-    iop.commit(host_hash_elems(fc.data(), fc.size()));
+    iop.commit(suite_hash_elems(iop.rng.suite, fc.data(), fc.size()));
     const uint32_t gen = v_rou_fwd(v_log2(domain));
     std::vector<E4> poly(degree);
     for (size_t i = 0; i < degree; i++) poly[i] = e4(fc[i], fc[degree + i], fc[2 * degree + i], fc[3 * degree + i]);
@@ -231,10 +227,11 @@ static inline void v_fri_verify(VReadIOP& iop, size_t degree, const std::functio
     }
 }
 
-// verify::Verifier::verify for one segment seal.  code_root = the control id of (circuit, po2).
-static inline void verify_segment(const VCircuit& vc, const uint32_t* seal, size_t seal_words, const uint32_t* code_root, uint32_t* po2_out) {
+// verify::Verifier::verify for one segment seal.  code_root = the control id of (circuit, po2, suite).
+static inline void verify_segment(const VCircuit& vc, const uint32_t* seal, size_t seal_words, const uint32_t* code_root, uint32_t* po2_out,
+                                  int suite) {
     const GenericCircuitHost& g = vc.g;
-    VReadIOP iop(seal, seal_words);
+    VReadIOP iop(seal, seal_words, suite);
     uint32_t globals[N_GLOBAL];
     iop.read_elems(globals, N_GLOBAL);
     const uint32_t po2 = iop.read_u32();
@@ -257,7 +254,7 @@ static inline void verify_segment(const VCircuit& vc, const uint32_t* seal, size
     const size_t T = g.taps.size();
     std::vector<E4> coeff_u(T + V_CHECK_SIZE);
     iop.read_ext(coeff_u.data(), coeff_u.size());
-    iop.commit(host_hash_elems(reinterpret_cast<const uint32_t*>(coeff_u.data()), 4 * coeff_u.size()));
+    iop.commit(suite_hash_elems(suite, reinterpret_cast<const uint32_t*>(coeff_u.data()), 4 * coeff_u.size()));
 
     // tap evaluations at z w^-back from the per-register interpolants
     std::vector<E4> eval_u(T);

@@ -81,6 +81,9 @@ pub const HFB200_EXIT_HALTED: u32 = 0;
 pub const HFB200_EXIT_SYSTEM_SPLIT: u32 = 1;
 pub const HFB200_BLIND_OS_ENTROPY: c_int = 0;
 pub const HFB200_BLIND_DETERMINISTIC: c_int = 1;
+/// Hash suites: upstream's `segment_prover(hashfn)` with "poseidon2" / "sha-256".
+pub const HFB200_HASH_POSEIDON2: c_int = 0;
+pub const HFB200_HASH_SHA256: c_int = 1;
 
 /// The segment in flight between `hfb200_segment_begin_dev` and `hfb200_segment_finish_dev`: device pointers of the committed
 /// columns, the mix and the writable accum columns (valid until the segment is finished), and the context's stream.
@@ -203,6 +206,8 @@ extern "C" {
         out: *mut *mut hfb200_pool,
     ) -> *const c_char;
     pub fn hfb200_pool_set_blinding(pool: *mut hfb200_pool, mode: c_int) -> *const c_char;
+    /// Hash suite of every worker context, kept across contexts re-created after a device fault.
+    pub fn hfb200_pool_set_hash_suite(pool: *mut hfb200_pool, suite: c_int) -> *const c_char;
     pub fn hfb200_pool_stats(pool: *const hfb200_pool, out: *mut hfb200_pool_stats_t) -> *const c_char;
     pub fn hfb200_set_blinding(ctx: *mut hfb200_ctx, mode: c_int) -> *const c_char;
     pub fn hfb200_pool_prove(pool: *mut hfb200_pool, jobs: *mut hfb200_segment_job, n_jobs: usize) -> *const c_char;
@@ -227,8 +232,28 @@ extern "C" {
         circuit: *const hfb200_circuit_desc, ir: *const hfb200_circuit_ir, seals: *const *const u32, seal_words: *const usize, n: usize,
         code_roots: *const u32, po2_out: *mut u32, threads: c_uint, first_bad: *mut usize,
     ) -> *const c_char;
+    /// `hfb200_verify_segment` / `_segments` for seals of hash suite `suite` (HFB200_HASH_*), against control ids of that suite.
+    pub fn hfb200_verify_segment_suite(
+        circuit: *const hfb200_circuit_desc, ir: *const hfb200_circuit_ir, seal: *const u32, seal_words: usize,
+        code_root: *const u32, po2_out: *mut u32, suite: c_int,
+    ) -> *const c_char;
+    pub fn hfb200_verify_segments_suite(
+        circuit: *const hfb200_circuit_desc, ir: *const hfb200_circuit_ir, seals: *const *const u32, seal_words: *const usize, n: usize,
+        code_roots: *const u32, po2_out: *mut u32, threads: c_uint, first_bad: *mut usize, suite: c_int,
+    ) -> *const c_char;
     /// Where the Fiat-Shamir transcript runs: 0 host (default), 1 device, 2 device replayed as a CUDA graph.  Identical seals.
+    /// SHA-256 contexts take the host transcript only.
     pub fn hfb200_set_transcript(ctx: *mut hfb200_ctx, mode: c_int) -> *const c_char;
+    /// Hash suite of the context (HFB200_HASH_*), between segments; drops the resident control group.
+    pub fn hfb200_set_hash_suite(ctx: *mut hfb200_ctx, suite: c_int) -> *const c_char;
+    /// The suites' host primitives: padded SHA-256 of bytes, the suite's hash of n words, of two digests, and its transcript RNG
+    /// run through `n_ops` (op, arg) pairs (0 mix the next digest, 1 random_elem, 2 random_bits(arg)).
+    pub fn hfb200_sha256(bytes: *const u8, n: usize, out8: *mut u32) -> *const c_char;
+    pub fn hfb200_hash_elems(suite: c_int, elems: *const u32, n: usize, out8: *mut u32) -> *const c_char;
+    pub fn hfb200_hash_pair(suite: c_int, a8: *const u32, b8: *const u32, out8: *mut u32) -> *const c_char;
+    pub fn hfb200_rng_script(
+        suite: c_int, ops: *const u32, n_ops: usize, digests: *const u32, n_digests: usize, out: *mut u32, cap: usize, n_out: *mut usize,
+    ) -> *const c_char;
     pub fn hfb200_graph_launches(ctx: *const hfb200_ctx) -> u64;
     /// Control id of (circuit, po2): Merkle root of the committed control columns, computed on the GPU.
     pub fn hfb200_control_root(ctx: *mut hfb200_ctx, po2: u32, code: *const u32, root_out: *mut u32) -> *const c_char;
@@ -247,6 +272,9 @@ extern "C" {
     pub fn hfb200_hal_batch_bit_reverse(ctx: *mut hfb200_ctx, io: *mut u32, count: usize, n: usize) -> *const c_char;
     pub fn hfb200_hal_hash_rows(ctx: *mut hfb200_ctx, digests: *mut u32, matrix: *const u32, rows: usize, cols: usize) -> *const c_char;
     pub fn hfb200_hal_hash_fold(ctx: *mut hfb200_ctx, io: *mut u32, input_size: usize, output_size: usize) -> *const c_char;
+    /// `hash_rows` / `hash_fold` of the SHA-256 suite (upstream's `Hal` with `HashSuite = Sha256HashSuite`).
+    pub fn hfb200_hal_sha_rows(ctx: *mut hfb200_ctx, digests: *mut u32, matrix: *const u32, rows: usize, cols: usize) -> *const c_char;
+    pub fn hfb200_hal_sha_fold(ctx: *mut hfb200_ctx, io: *mut u32, input_size: usize, output_size: usize) -> *const c_char;
     pub fn hfb200_hal_batch_evaluate_any(
         ctx: *mut hfb200_ctx, coeffs: *const u32, poly_count: usize, n: usize, which: *const u32, xs: *const u32, out: *mut u32, count: usize,
     ) -> *const c_char;

@@ -125,6 +125,21 @@ const char* hfb200_set_blinding(hfb200_ctx* ctx, int mode);
  * segments (hfb200_last_stats reports ms_device only).  HFB200_DEVICE_TRANSCRIPT=1|2 in the environment selects a mode for
  * contexts that never call this. */
 const char* hfb200_set_transcript(hfb200_ctx* ctx, int mode);
+/* Hash suite of the context: upstream's `segment_prover(hashfn)` with hashfn "poseidon2" (default) or "sha-256".  It selects the
+ * Merkle hash of every tree the context commits (leaves: hash of the row's raw Montgomery words; nodes: hash_pair of two
+ * digests) and the transcript's hash and RNG (Poseidon2Rng, or ShaRng).  Digests are 8 words in both suites, so the seal layout,
+ * hfb200_seal_words and the checkpoint names stay the same; the control id differs (upstream keeps one control-id table per
+ * hashfn).  SHA-256 digest words, read as little-endian bytes, are the standard SHA-256 output bytes.
+ *   - valid between segments; a change drops the resident control group (a code == NULL segment then needs hfb200_control_root
+ *     again, and a pool re-commits its loaded control group on that context);
+ *   - hfb200_control_root, hfb200_op_merkle, the one-shot, two-phase and device entries, the accum / witgen callbacks of a pool
+ *     and hfb200_bench_merkle follow the context's suite; the hfb200_hal_* operators name their suite themselves;
+ *   - SHA-256 runs the host transcript only: hfb200_set_transcript(ctx, 1 | 2) on a SHA-256 context is an error, so is
+ *     switching a context set to mode 1 or 2 to SHA-256, and HFB200_DEVICE_TRANSCRIPT does not apply to SHA-256 contexts;
+ *   - seals verify with hfb200_verify_segment_suite / _segments_suite under the same suite;
+ *   - the claim digests (hfb200_digest_bytes, hfb200_digest_pair) stay Poseidon2 in both suites. */
+enum { HFB200_HASH_POSEIDON2 = 0, HFB200_HASH_SHA256 = 1 };
+const char* hfb200_set_hash_suite(hfb200_ctx* ctx, int suite);
 /* Segments of this context that were issued as one cudaGraphLaunch (transcript mode 2). */
 uint64_t hfb200_graph_launches(const hfb200_ctx* ctx);
 const char* hfb200_version(void);
@@ -252,6 +267,13 @@ const char* hfb200_verify_segment(const hfb200_circuit_desc* circuit, const hfb2
 const char* hfb200_verify_segments(const hfb200_circuit_desc* circuit, const hfb200_circuit_ir* ir, const uint32_t* const* seals,
                                    const size_t* seal_words, size_t n, const uint32_t* code_roots /*[n][8]*/, uint32_t* po2_out /*[n] or NULL*/,
                                    unsigned threads, size_t* first_bad);
+/* hfb200_verify_segment / hfb200_verify_segments for seals of hash suite `suite` (HFB200_HASH_*); `code_root(s)` must be control
+ * ids of that suite.  The two entries above are these with HFB200_HASH_POSEIDON2. */
+const char* hfb200_verify_segment_suite(const hfb200_circuit_desc* circuit, const hfb200_circuit_ir* ir, const uint32_t* seal, size_t seal_words,
+                                        const uint32_t* code_root /*[8]*/, uint32_t* po2_out, int suite);
+const char* hfb200_verify_segments_suite(const hfb200_circuit_desc* circuit, const hfb200_circuit_ir* ir, const uint32_t* const* seals,
+                                         const size_t* seal_words, size_t n, const uint32_t* code_roots /*[n][8]*/, uint32_t* po2_out /*[n] or NULL*/,
+                                         unsigned threads, size_t* first_bad, int suite);
 /* ---- receipt claims: the rest of `receipt.verify(image_id)` (host only; no device, no context) -------------------------
  * Upstream's Receipt::verify also decodes each segment's ReceiptClaim from the seal's globals, chains pre/post state digests
  * from the image id and ties the journal digest to the last claim's output (/root/reference/verifier/src/main.rs:124-126 trusts
@@ -277,7 +299,21 @@ const char* hfb200_claim_next_state(const uint32_t* pre8, uint32_t index, uint32
 const char* hfb200_verify_claims(const uint32_t* const* seals, const size_t* seal_words, size_t n, const uint32_t* image_id8,
                                  const uint8_t* journal, size_t journal_len);
 
-/* Control id: Merkle root of the x4 LDE of the code (control) columns, u32[w_code][2^po2] on the host.
+/* ---- the hash suites' host primitives (host only; no device, no context) ------------------------------------------------
+ * The pieces of the transcript and of the verifier of each suite (HFB200_HASH_*), for known-answer tests and for hosts that
+ * recompute a digest.  hfb200_sha256: the standard, padded SHA-256 of a byte string as digest words (little-endian bytes =
+ * the standard output).  hfb200_hash_elems: the suite's hash of n words (hash_elem_slice: Merkle leaves, the transcript
+ * header, hash_u).  hfb200_hash_pair: the suite's hash of two digests (Merkle nodes).  hfb200_rng_script: runs the suite's
+ * transcript RNG (Poseidon2Rng or ShaRng) from its initial state through n_ops ops, ops[2i] = 0: mix(the next 8 words of
+ * `digests`), 1: random_elem (Montgomery form), 2: random_bits(ops[2i + 1] in 1..31); every draw is appended to out
+ * (cap words), *n_out = draws written. */
+const char* hfb200_sha256(const uint8_t* bytes, size_t n, uint32_t* out8);
+const char* hfb200_hash_elems(int suite, const uint32_t* elems, size_t n, uint32_t* out8);
+const char* hfb200_hash_pair(int suite, const uint32_t* a8, const uint32_t* b8, uint32_t* out8);
+const char* hfb200_rng_script(int suite, const uint32_t* ops, size_t n_ops, const uint32_t* digests, size_t n_digests, uint32_t* out, size_t cap,
+                              size_t* n_out);
+
+/* Control id: Merkle root of the x4 LDE of the code (control) columns, u32[w_code][2^po2] on the host, in the context's hash suite.
  * The committed control group stays resident: until the context sees another po2 or another `code` pointer, segments may
  * pass code == NULL to hfb200_prove_segment / hfb200_segment_begin and reuse it (the control columns depend on
  * (circuit, po2) only; the seal is bit-identical to the one produced with the columns passed again). */
@@ -334,6 +370,9 @@ const char* hfb200_pool_create_ir(const int* devices, int n_devices, int context
                                   const hfb200_circuit_ir* circuit, hfb200_pool** out);
 /* Blinding mode of every worker context (see hfb200_set_blinding; default HFB200_BLIND_OS_ENTROPY). */
 const char* hfb200_pool_set_blinding(hfb200_pool* pool, int mode);
+/* Hash suite of every worker context (see hfb200_set_hash_suite; default HFB200_HASH_POSEIDON2).  Kept by the pool: a context
+ * re-created after a device fault gets it again.  Not while hfb200_pool_prove runs. */
+const char* hfb200_pool_set_hash_suite(hfb200_pool* pool, int suite);
 /* Proves all jobs; returns NULL when every job succeeded, else the first failed job's error (every failed job keeps its own
  * message in jobs[i].error).  Failure handling (the reference's batch behaviour, /root/reference/data/watchdog.sh:58-83: a
  * failed input is set aside and the rest continue): a shape / argument error fails that job only; a CUDA error makes the
@@ -387,7 +426,7 @@ const char* hfb200_op_interpolate_ntt(hfb200_ctx* ctx, uint32_t* io, size_t coun
 const char* hfb200_op_expand_ntt(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t n_in, uint32_t expand_bits);
 /* The fused production path of commit_group: trace columns -> LDE evaluations (no coefficient round trip). */
 const char* hfb200_op_lde(hfb200_ctx* ctx, uint32_t* out, const uint32_t* in, size_t count, size_t n_in);
-/* Hal::hash_rows + Hal::hash_fold: full Merkle tree (heap layout, 2*rows digests) of a column-major matrix. */
+/* Hal::hash_rows + Hal::hash_fold: full Merkle tree (heap layout, 2*rows digests) of a column-major matrix, in the context's hash suite. */
 const char* hfb200_op_merkle(hfb200_ctx* ctx, const uint32_t* matrix, size_t rows, size_t cols, uint32_t* nodes_out);
 /* poseidon2_mix on `n` independent 24-word states. */
 const char* hfb200_op_poseidon2(hfb200_ctx* ctx, uint32_t* states, size_t n);
@@ -445,6 +484,12 @@ const char* hfb200_hal_hash_rows(hfb200_ctx* ctx, uint32_t* digests, const uint3
 /* Hal::hash_fold: io[output_size + i] = hash_pair(io[input_size + 2i], io[input_size + 2i + 1]) for i < output_size, digests
  * of 8 words, input_size = 2 * output_size: one level of the heap layout of hfb200_op_merkle (node 1 = root).  16-byte aligned. */
 const char* hfb200_hal_hash_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size);
+/* hfb200_hal_hash_rows / _hash_fold of the SHA-256 suite (upstream's Hal with HashSuite = Sha256HashSuite), whatever the
+ * context's own suite; same shapes, checks and stream rules.  sha_rows: digests[r] = SHA-256 compressions from the IV over row
+ * r's words as little-endian bytes, 16 words per block, the last block zero-filled, no length block; sha_fold: hash_pair =
+ * one compression of the 64 bytes of the two child digests.  Digest words are the byte-swapped state words. */
+const char* hfb200_hal_sha_rows(hfb200_ctx* ctx, uint32_t* digests, const uint32_t* matrix, size_t rows, size_t cols);
+const char* hfb200_hal_sha_fold(hfb200_ctx* ctx, uint32_t* io, size_t input_size, size_t output_size);
 /* Hal::batch_evaluate_any: out[j] = sum_{k < n} coeffs[which[j]][k] * xs[j]^k for j < count, coeffs u32[poly_count][n]
  * (natural order), which u32[count] (each < poly_count), xs and out Fp4[count].  count <= 262140. */
 const char* hfb200_hal_batch_evaluate_any(hfb200_ctx* ctx, const uint32_t* coeffs, size_t poly_count, size_t n, const uint32_t* which,
